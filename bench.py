@@ -23,6 +23,7 @@ N > 1    : ONE process (rank 0) drives all N devices through ONE library context
 (the reference is managed C# and there is no .NET runtime on the box; DESIGN.md "Oracle") — on all host threads.
 """
 import argparse
+import atexit
 import ctypes as C
 import json
 import math
@@ -40,6 +41,9 @@ UNIT = "GB/s"
 STREAM_BYTES = 65536
 FULL_STREAMS = 65536
 QUALITY = 8
+DUMP_BYTES = 64 * 10 ** 6      # --dump-outputs: size limit of all files together
+DUMP_STREAMS = 192             # --dump-outputs: decoded streams kept whole (192 x 64 KiB as float32 = 48 MiB)
+DUMP_SEED = 0xD0               # --dump-outputs: which streams, the same in every run and build
 
 
 def workload_config(streams, n_gpus=1):
@@ -67,6 +71,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100",
                                           "-i", str(self.index)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)   # the sampler loops until stopped: it must not outlive a run that fails before stop()
             self.thread = threading.Thread(target=self._pump, daemon=True)
             self.thread.start()
         except Exception:
@@ -316,6 +321,36 @@ def stream_mismatch(a, b, off, ln, chunk_bytes=1 << 30):
         del c
         s = e
     return out
+
+
+def dump_outputs(path, shards, n, size):
+    """--dump-outputs: what the timed decode returned in its last step, as .npy files that two builds can be compared by.
+    Per stream, over all devices' streams (device-major): status / out_len / consumed (float32 holds them exactly: 64 KiB
+    streams) and decoded_digest, the sum of (position + 1) x byte over the stream's decoded bytes (exact in float64), which
+    any change to one byte alters.  Besides, the decoded bytes of a seeded sample of whole streams (decoded_streams: their
+    indices)."""
+    import numpy as np
+    import torch
+
+    def digest(s):
+        rows = s["d_dst"][:n * size].view(n, size)
+        w = torch.arange(1, size + 1, dtype=torch.int64, device=s["dev"])
+        return torch.cat([(rows[i:i + 1024].to(torch.int64) * w).sum(1) for i in range(0, n, 1024)]).cpu()
+
+    per_stream = [torch.cat([s[k].cpu() for s in shards]).numpy().astype(np.float32) for k in ("st", "olen", "cons")]
+    per_stream.append(torch.cat([digest(s) for s in shards]).numpy().astype(np.float64))
+    total = len(shards) * n
+    room = DUMP_BYTES - 4096 - sum(a.nbytes for a in per_stream)   # (4096: the .npy headers)
+    rows = min(DUMP_STREAMS, total, room // (4 * size + 8))
+    assert rows > 0, f"--dump-outputs: {total} streams do not fit {DUMP_BYTES} bytes"
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(total, size=rows, replace=False))
+    decoded = torch.cat([s["d_dst"][:n * size].view(n, size)[torch.as_tensor(pick[pick // n == g] % n, device=s["dev"])].cpu()
+                         for g, s in enumerate(shards)])
+    os.makedirs(path, exist_ok=True)
+    for name, a in zip(("status", "out_len", "consumed", "decoded_digest"), per_stream):
+        np.save(os.path.join(path, name + ".npy"), a)
+    np.save(os.path.join(path, "decoded_streams.npy"), pick.astype(np.float64))
+    np.save(os.path.join(path, "decoded.npy"), decoded.numpy().astype(np.float32))
 
 
 def bench_decode_config(codec, name, fmt, raw, r_off, r_len, dev, ts, peak, steps, warmup, orders, drop_unrepresentable=False,
@@ -597,6 +632,8 @@ def run_ours(args):
     t_wall1 = time.time()
     launches = codec.kernel_launches - launches0
     clocks = sampler.stop(t_wall0, t_wall1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, shards, n, size)
     total_ms = max(ev[0][0].elapsed_time(ev[-1][1]) for ev in evs)              # max over devices
     kernel_ms = sum(a.elapsed_time(b) for a, b in evs[0]) / args.steps            # device 0: the roofline kernel
     ms_per_step = total_ms / args.steps
@@ -632,7 +669,7 @@ def run_ours(args):
     h_off, h_len = np.concatenate(h_off), np.concatenate(h_len)
     h_doff = np.arange(G * n, dtype=np.uint64) * np.uint64(size)
     h_cap = np.full(G * n, size, dtype=np.uint64)
-    e2e_steps = max(1, min(args.steps, 5))
+    e2e_steps = args.steps
     for _ in range(2):
         out_len, consumed, status = codec.decode_packed(fmt, h_src, h_off, h_len, h_dst, h_doff, h_cap, opts)
     assert (status == 0).all()
@@ -713,8 +750,11 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed passes over the C2 batch, both device resident (value) and end to end (e2e); the per-class "
+                         "breakdown and the configs C3 / C4 / C5 time fixed counts of their own")
+    ap.add_argument("--warmup", type=int, default=3,
+                    help="untimed decode passes before the timed steps (the GPU arm runs at least 3: its line's warmup says how many)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--streams", type=int, default=FULL_STREAMS, help="streams per GPU (default: the full C2 configuration)")
     ap.add_argument("--c3-streams", type=int, default=16384, help="streams of config C3 (all three formats together)")
@@ -723,7 +763,15 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="headline only (skip C3 / C4 / C5)")
     ap.add_argument("--quick", action="store_true", help="C5 only among the other configs")
     ap.add_argument("--dump-batch", default=None, help="write the reference arm's C2 sample (packed.bin, index.bin) for baseline/dotnet and exit")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one decoded to DIR/*.npy (float32 / float64, at most 64 MB): "
+                         "status, out_len, consumed and a digest of the decoded bytes of every stream, and the bytes of a fixed "
+                         "sample of streams")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl == "reference" or args.dump_batch):
+        ap.error("--dump-outputs writes the outputs of the GPU decode (--impl ours)")
     if args.impl == "reference" or args.dump_batch:
         return run_reference(args)
     return run_ours(args)

@@ -87,6 +87,12 @@ def test_reference_arm_ranks_other_than_zero_do_nothing():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "unused"]], ids=str)
+def test_bench_rejects_arguments_it_cannot_honour(args):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and out.stdout == "" and "error:" in out.stderr, out.stderr[-400:]
+
+
 def test_bench_stream_mismatch_flags_exactly_the_windows_that_differ():
     """bench.stream_mismatch (the per-stream verifier of the C3 / C4 bench lines and of tests/test_baseline_sizes_gpu.py):
     ragged adjacent windows, an empty one, chunked over several passes."""

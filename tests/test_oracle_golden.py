@@ -1,12 +1,15 @@
 """CPU tests: the oracle against every golden vector / known answer the reference holds for the hot path
 (SURVEY.md §8c, BASELINE.md §2).  These pin the checker before the GPU parity tests trust it."""
 import hashlib
+import os
 
 import numpy as np
 import pytest
 
 from auroralib.compression_b200 import _abi as A
 from tests.util import ALL_FORMATS, SIZED_FORMATS, end_position, fmt_id, synth
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_fixture_integrity(bmp, test_lz):
@@ -117,21 +120,14 @@ def test_data_recognition(oracle, fmt):
 
 
 def test_lz4_block_cross_check_with_system_liblz4(oracle, bmp):
-    """Second opinion for the LZ4 block format: the image's liblz4.so.1 (LZ4_decompress_safe / LZ4_compress_default)."""
-    import ctypes
-    try:
-        lz4 = ctypes.CDLL("liblz4.so.1")
-    except OSError:
-        pytest.skip("liblz4.so.1 not present")
+    """Second opinion for the LZ4 block format from liblz4 1.9.4, recorded so that the test needs no system library:
+    LZ4_decompress_safe decoded the oracle's block of the first 200 000 bytes of Test.bmp (SHA-256 below) to those bytes, and
+    tests/golden/liblz4_block_of_bmp_200000.lz4 is LZ4_compress_default's block of the same bytes."""
     raw = bmp[:200000]
     comp, st = oracle.encode(A.FMT_LZ4_BLOCK, raw, A.make_opts(quality=8))
-    dst = ctypes.create_string_buffer(len(raw))
-    n = lz4.LZ4_decompress_safe(comp, dst, len(comp), len(raw))
-    assert n == len(raw) and dst.raw == raw
-    bound = lz4.LZ4_compressBound(len(raw))
-    cbuf = ctypes.create_string_buffer(bound)
-    cn = lz4.LZ4_compress_default(raw, cbuf, len(raw), bound)
-    out, out_len, consumed, status = oracle.decode(A.FMT_LZ4_BLOCK, cbuf.raw[:cn], len(raw))
+    assert st == 0 and hashlib.sha256(comp).hexdigest() == "a3479a738b3689a7cc2e01ba541cce0a75d31f44d9180884aa0cd0f9d6fcd79c"
+    ref = open(os.path.join(ROOT, "tests", "golden", "liblz4_block_of_bmp_200000.lz4"), "rb").read()
+    out, out_len, consumed, status = oracle.decode(A.FMT_LZ4_BLOCK, ref, len(raw))
     assert status == 0 and out == raw
 
 
