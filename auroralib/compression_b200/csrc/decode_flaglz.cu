@@ -742,9 +742,20 @@ __device__ void resolver_role(uint8_t* ring, uint32_t qbase, uint32_t mail, uint
 // equally sized groups (random data: all literals; runs, tiles: all matches) are resolved by one ballot: every lane
 // looks at the flag byte its group would have if all groups before it had the size of the first one, and the walk starts
 // behind the leading lanes that agree.  Every lane then sizes its own 8 tokens, one packed warp scan gives output bases
-// and match-queue slots, literals are scattered lane-locally and the matches of all groups are queued for
-// resolve_matches().  All shared-memory traffic uses 32-bit shared addresses; the output ring is 8 KiB aligned, so the
-// wrapped address (pos & mask) | base is a single LOP3.
+// and match-queue slots, and the tokens are placed in two passes: a branch-free TOKEN pass in which every lane scatters
+// its literals and writes each match's position and token address into the match's own queue entry, and a MATCH pass in
+// which ONE queued match per lane (32 per round, at most 3 rounds) decodes its token in place into the
+// {pos, len | d << 17} that resolve_matches() reads.  All shared-memory traffic uses 32-bit shared addresses; the output
+// ring is 8 KiB aligned, so the wrapped address (pos & mask) | base is a single LOP3.
+// Before the split the match decode sat in a branch inside the per-slot loop; with ~10 % match tokens some lane of the
+// warp holds a match at nearly every slot, so the warp issued both sides at all 8 slots (148 SASS instructions for the
+// 8 slots of LZ10, now 50 for the token pass + 48 for the match pass).
+// Measured and rejected: the match pass as a loop over its rounds (C2 596 GB/s against 611; mixed entropy 779 against 831:
+// its run iterations queue 96 matches, and each round waited for its two dependent shared-memory loads before the next
+// one started; the unrolled pass issues the loads of all rounds first).  Because the token pass already knows each match's
+// queue entry, the match pass needs no lane -> (group, k-th match) mapping.  The mappings considered for it (an expand
+// through the group-start table, __fns over a warp-wide match mask) were not built: on top of the group search each needs
+// a segmented scan of the match lengths inside a group for the output position, which the token pass has in orel[].
 // ---------------------------------------------------------------------------------------------
 struct CutResult {
     uint32_t total, nq, nlan, consumed;
@@ -917,8 +928,9 @@ __device__ BodyResult decode_body_g32(InStream* in, Sink& sink, const uint32_t g
         const uint32_t myrel = mya - wa;
         const uint32_t m = mbits(lds_u8(mya));   // match bits in wire bit order
 
-        // ---- pass 1: sizes of my 8 tokens
-        uint32_t b1v[8], orel[8];
+        // ---- pass 1: sizes of my 8 tokens; tv[j] = shared address of token j << 8 | its first byte (shared addresses are
+        //      below 2^24, and the literal store takes the low byte)
+        uint32_t tv[8], orel[8];
         uint32_t gsize = 0;
         {
             uint32_t a = mya + 1;
@@ -926,7 +938,7 @@ __device__ BodyResult decode_body_g32(InStream* in, Sink& sink, const uint32_t g
             for (int j = 0; j < 8; j++) {
                 const bool ism = (K == K_LZ10) ? (m >> (7 - j)) & 1 : (m >> j) & 1;
                 const uint32_t b1 = lds_u8(a);
-                b1v[j] = b1;
+                tv[j] = (a << 8) | b1;
                 orel[j] = gsize;
                 uint32_t len;
                 if (K == K_LZ10) len = ism ? (b1 >> 4) + 3 : 1;
@@ -950,17 +962,39 @@ __device__ BodyResult decode_body_g32(InStream* in, Sink& sink, const uint32_t g
         const uint32_t cut = __shfl_sync(kFull, incl, (nl + 31) & 31);
         const uint32_t end_rel = nl == 32 ? chain_end : __shfl_sync(kFull, myrel, nl & 31);
         if (nl > 0 && (cut & 0xFFFFFu) <= remaining && cur + end_rel <= slen) {
-            // ---- fast path: every token of the first nl groups executes
-            uint32_t a = mya + 1, qa = qaddr + 8 * qexcl;
+            // ---- fast path: every token of the first nl groups executes.  Token pass: a literal stores its byte, a match
+            //      stores {pos, tv} into its queue entry; both stores are predicated, nothing branches per slot
             if (lane < nl) {
+                uint32_t qa = qaddr + 8 * qexcl;
 #pragma unroll
                 for (int j = 0; j < 8; j++) {
                     const bool ism = (K == K_LZ10) ? (m >> (7 - j)) & 1 : (m >> j) & 1;
                     const uint32_t pos = gbase + orel[j];
-                    if (!ism) {
-                        sts_u8((pos & kRingMask) | rb, b1v[j]);
-                    } else {
-                        const uint32_t b1 = b1v[j], b2 = lds_u8(a + 1);
+                    if (!ism) sts_u8((pos & kRingMask) | rb, tv[j]);
+                    if (ism) {
+                        sts_u64(qa, pos, tv[j]);
+                        qa += 8;
+                    }
+                }
+            }
+            total = cut & 0xFFFFFu;
+            nq = cut >> 20;
+            __syncwarp();
+            // ---- match pass: ONE queued match per lane decodes its token in place into {pos, len | dist << 17}
+            {
+                // the loads of all rounds are issued before their first use
+                constexpr int kRounds = (kIterMatches + 31) / 32;
+                uint32_t wv[kRounds], b2v[kRounds];
+#pragma unroll
+                for (int r = 0; r < kRounds; r++)
+                    if (lane + 32 * r < nq) wv[r] = lds_u32(qaddr + 8 * (lane + 32 * r) + 4);
+#pragma unroll
+                for (int r = 0; r < kRounds; r++)
+                    if (lane + 32 * r < nq) b2v[r] = lds_u8((wv[r] >> 8) + 1);
+#pragma unroll
+                for (int r = 0; r < kRounds; r++) {
+                    if (lane + 32 * r < nq) {
+                        const uint32_t e = qaddr + 8 * (lane + 32 * r), w = wv[r], b1 = w & 0xFFu, b2 = b2v[r];
                         uint32_t len, dist;
                         if (K == K_LZ10) {
                             len = (b1 >> 4) + 3;
@@ -970,18 +1004,14 @@ __device__ BodyResult decode_body_g32(InStream* in, Sink& sink, const uint32_t g
                             const uint32_t raw = ((b2 >> lz.length_bits) << 8) | b1;
                             const uint32_t ring_len = 1u << lz.windows_bits;
                             const uint32_t offset = (uint32_t(lz.max_distance) + raw - uint32_t(lz.windows_start)) & uint32_t(lz.max_distance - 1);
-                            const uint32_t rp = pos & (ring_len - 1);
+                            const uint32_t rp = lds_u32(e) & (ring_len - 1);
                             dist = rp >= offset ? rp - offset : rp - offset + ring_len;
                             if (dist == 0) dist = ring_len;
                         }
-                        sts_u64(qa, pos, len | (dist << 17));
-                        qa += 8;
+                        sts_u32(e + 4, len | (dist << 17));
                     }
-                    a += ism ? 2 : 1;
                 }
             }
-            total = cut & 0xFFFFFu;
-            nq = cut >> 20;
             nlan = nl;
             consumed = cur + end_rel;
         } else {
