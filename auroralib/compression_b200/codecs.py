@@ -448,12 +448,6 @@ class BLZ(_SizedCodec):
     """Nintendo/BLZ.cs: parsed and written backwards from the footer at the end of the stream (its own kernel, decode_blz.cu)."""
     FORMAT, Name = _abi.FMT_BLZ, "Nintendo BLZ"
 
-    def GetDecompressedSize(self, source):   # the footer sits at Length - 8: the whole stream is needed
-        _, data = _remaining(source)
-        size, st = default_codec().decoded_size_batch(self.FORMAT, [data], self._opts())
-        _raise_for(int(st[0]))
-        return int(size[0])
-
 
 class SMSR00(_SizedCodec):
     """Nintendo/SMSR00.cs: "SMSR00" header, MIO0 tokens with 16-bit big-endian mask words interleaved with the codes and the
@@ -479,16 +473,7 @@ class LZ60(LZ40):
     FORMAT, Name = _abi.FMT_LZ60, "Nintendo LZ60"
 
 
-class _WholeHeaderPeek:
-    # GetDecompressedSize looks past the first 16 bytes (LZ00: size at 48) or at the stream length (ECD)
-    def GetDecompressedSize(self, source):
-        _, data = _remaining(source)
-        size, st = default_codec().decoded_size_batch(self.FORMAT, [data], self._opts())
-        _raise_for(int(st[0]))
-        return int(size[0])
-
-
-class ECD(_WholeHeaderPeek, _SizedCodec):
+class ECD(_SizedCodec):
     """Extended/Specialized/ECD.cs: "ECD" + flag + plain size + compressed size + size (BE), PlainSize stored bytes + LZSS
     body with LzProperties(0x400, 0x42, 3, 0x3BE); quality 0, inputs of at most 16 bytes and incompressible inputs are stored"""
     FORMAT, Name = _abi.FMT_ECD, "ECD lzss"
@@ -509,7 +494,7 @@ class ECD(_WholeHeaderPeek, _SizedCodec):
         return size
 
 
-class LZ00(_WholeHeaderPeek, _SizedCodec):
+class LZ00(_SizedCodec):
     """Sega/LZ00.cs: 64-byte header (file length, name, size, key) + LZSS body (Lzss0Properties) under a per-byte LCG
     keystream; the header's name field is always the reference's default "Temp.dat" """
     FORMAT, Name = _abi.FMT_LZ00, "LZ00"

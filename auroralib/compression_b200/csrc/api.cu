@@ -827,75 +827,13 @@ int aurora_decoded_size_batch(aurora_ctx* ctx, int format, const aurora_codec_op
     if (!ctx) return AURORA_INVALID_ARGUMENT;
     if (n == 0) return AURORA_OK;
     if (!src_base || !src_off || !src_len || !out_size || !status) return AURORA_INVALID_ARGUMENT;
-    if (aurora::is_wrapper_format(format)) {   // header peeks of the wrapper formats (wrappers.cu)
-        for (size_t i = 0; i < n; i++) status[i] = aurora::wrapped_decoded_size(format, src_base + src_off[i], src_len[i], &out_size[i]);
-        return AURORA_OK;
-    }
-    const int bo = opts ? opts->byte_order : AURORA_ENDIAN_DEFAULT;
-    auto be32 = [](const uint8_t* p) { return (uint32_t(p[0]) << 24) | (uint32_t(p[1]) << 16) | (uint32_t(p[2]) << 8) | p[3]; };
-    auto le32 = [](const uint8_t* p) { return uint32_t(p[0]) | (uint32_t(p[1]) << 8) | (uint32_t(p[2]) << 16) | (uint32_t(p[3]) << 24); };
-    if (format == AURORA_FMT_BLZ) {   // BLZ.cs:35-43: the footer at Length - 8
-        for (size_t i = 0; i < n; i++) {
-            const uint64_t len = src_len[i];
-            const uint8_t* f = src_base + src_off[i] + (len >= 8 ? len - 8 : 0);
-            out_size[i] = 0;
-            if (len < 8) status[i] = AURORA_END_OF_STREAM;
-            else if (f[3] < 8) status[i] = AURORA_INVALID_DATA;   // "Invalid BLZ header."
-            else {
-                out_size[i] = uint32_t(le32(f + 4) + (uint32_t(f[0]) | (uint32_t(f[1]) << 8) | (uint32_t(f[2]) << 16)));
-                status[i] = AURORA_OK;
-            }
-        }
-        return AURORA_OK;
-    }
-    if (is_flaglz(format)) {
-        // GetDecompressedSize is a header peek (e.g. Yaz0.cs:50-55, LZ10.cs:47-57): a few bytes of host memory
+    // GetDecompressedSize is a header peek (e.g. Yaz0.cs:50-55, LZ10.cs:47-57): a few bytes of host memory
+    if (aurora::is_wrapper_format(format) || is_flaglz(format) || format == AURORA_FMT_BLZ) {
+        const int bo = opts ? opts->byte_order : AURORA_ENDIAN_DEFAULT;
         for (size_t i = 0; i < n; i++) {
             const uint8_t* p = src_base + src_off[i];
-            const uint64_t len = src_len[i];
-            int st = AURORA_OK;
-            uint64_t sz = 0;
-            if (format == AURORA_FMT_LZHUDSON) {   // LZHudson.cs:37-38
-                if (len < 4) st = AURORA_END_OF_STREAM;
-                else sz = be32(p);
-            } else if (format == AURORA_FMT_SMSR00) {   // SMSR00.cs:40-46
-                if (len < 6) st = AURORA_END_OF_STREAM;
-                else if (std::memcmp(p, "SMSR00", 6) != 0) st = AURORA_INVALID_IDENTIFIER;
-                else if (len < 12) st = AURORA_END_OF_STREAM;
-                else sz = be32(p + 8);
-            } else if (format == AURORA_FMT_LZ10 || format == AURORA_FMT_LZ11 || format == AURORA_FMT_LZ40 || format == AURORA_FMT_LZ60) {
-                const uint8_t id = format == AURORA_FMT_LZ10 ? 0x10 : format == AURORA_FMT_LZ11 ? 0x11 : format == AURORA_FMT_LZ40 ? 0x40 : 0x60;
-                if (len < 1) st = AURORA_END_OF_STREAM;
-                else if (p[0] != id) st = AURORA_INVALID_IDENTIFIER;
-                else if (len < 4) st = AURORA_END_OF_STREAM;
-                else {
-                    sz = uint32_t(p[1]) | (uint32_t(p[2]) << 8) | (uint32_t(p[3]) << 16);
-                    if (sz == 0) {
-                        if (len < 8) st = AURORA_END_OF_STREAM;
-                        else sz = le32(p + 4);
-                    }
-                }
-            } else {
-                const char* magic = format == AURORA_FMT_YAZ0 ? "Yaz0" : format == AURORA_FMT_YAZ1 ? "Yaz1" : format == AURORA_FMT_YAY0 ? "Yay0"
-                                    : format == AURORA_FMT_MIO0 ? "MIO0" : "LZSS";
-                if (len < 4) st = AURORA_END_OF_STREAM;
-                else if (std::memcmp(p, magic, 4) != 0) st = AURORA_INVALID_IDENTIFIER;
-                else if (len < 8) st = AURORA_END_OF_STREAM;
-                else if (format == AURORA_FMT_LZSS || format == AURORA_FMT_YAY0) sz = be32(p + 4);   // Yay0.cs:45-46 reads BE regardless
-                else if (format == AURORA_FMT_YAZ0 || format == AURORA_FMT_YAZ1) sz = bo == AURORA_ENDIAN_LITTLE ? le32(p + 4) : be32(p + 4);
-                else {   // MIO0.cs:42-48: detected order
-                    bool big = true;
-                    if (bo == AURORA_ENDIAN_LITTLE) big = false;
-                    else if (bo != AURORA_ENDIAN_BIG && len >= 16) {
-                        const uint32_t cb = be32(p + 8), lb = be32(p + 12), cl = le32(p + 8), ll = le32(p + 12);
-                        const bool pb = cb >= 0x10 && cb <= lb && lb <= len, pl = cl >= 0x10 && cl <= ll && ll <= len;
-                        big = pb || !pl;
-                    }
-                    sz = big ? be32(p + 4) : le32(p + 4);
-                }
-            }
-            out_size[i] = sz;
-            status[i] = st;
+            status[i] = aurora::is_wrapper_format(format) ? aurora::wrapped_decoded_size(format, p, src_len[i], &out_size[i])
+                                                          : aurora::core_decoded_size(format, bo, p, src_len[i], &out_size[i]);
         }
         return AURORA_OK;
     }
@@ -927,63 +865,7 @@ int aurora_is_match_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* 
     if (!ctx) return AURORA_INVALID_ARGUMENT;
     if (n == 0) return AURORA_OK;
     if (!src_base || !src_off || !src_len || !match) return AURORA_INVALID_ARGUMENT;
-    auto magic16 = [&](size_t i, const void* m, size_t k) {
-        return 0x10 < src_len[i] && src_len[i] >= k && std::memcmp(src_base + src_off[i], m, k) == 0;
-    };
-    static const uint8_t snappy_id[10] = {0xff, 0x06, 0x00, 0x00, 0x73, 0x4e, 0x61, 0x50, 0x70, 0x59};
-    if (aurora::is_wrapper_format(format)) {
-        // IsMatchStatic of the wrapper formats: identifier (+ a minimum length), then, for GCLZ / CXLZ / COMP, the
-        // LZ10 / LZ11 heuristic on the bytes behind it (GCLZ.cs:30-31, CXLZ.cs:31-32, COMP.cs:30-31, 3DS-LZ.cs:29-30,
-        // LZ77.cs:46-47, LZOn.cs:29-30, Level5LZSS.cs:29-30).  Level5.IsMatch needs zlib and the file name: not provided.
-        static const uint8_t lzon_id[8] = {'L', 'Z', 'O', 'n', 0x00, 0x2F, 0xF1, 0x71};
-        std::vector<size_t> idx;
-        std::vector<uint64_t> so, sl;
-        for (size_t i = 0; i < n; i++) {
-            const uint8_t* p = src_base + src_off[i];
-            const uint64_t len = src_len[i];
-            bool m = false;
-            switch (format) {
-                case AURORA_FMT_GCLZ: m = 0x8 < len && std::memcmp(p, "GCLZ", 4) == 0; break;
-                case AURORA_FMT_CXLZ: m = 0x8 < len && std::memcmp(p, "CXLZ", 4) == 0; break;
-                case AURORA_FMT_COMP: m = 0x8 < len && std::memcmp(p, "COMP", 4) == 0; break;
-                case AURORA_FMT_LZ_3DS: m = 0x10 < len && std::memcmp(p, "3DS-LZ\r\n", 8) == 0; break;
-                case AURORA_FMT_LZON: m = 0x10 < len && std::memcmp(p, lzon_id, 8) == 0; break;
-                case AURORA_FMT_LEVEL5_LZSS: m = 0x10 < len && std::memcmp(p, "SSZL", 4) == 0 && (p[4] | p[5] | p[6] | p[7]) == 0; break;
-                case AURORA_FMT_LZ77:
-                    m = 0x8 < len && std::memcmp(p, "LZ77", 4) == 0 &&
-                        (p[4] == 0x10 || p[4] == 0x11 || p[4] == 0x24 || p[4] == 0x28 || p[4] == 0x30 || p[4] == 0xF7);
-                    break;
-                // the LZSS-property family with an identifier (AKLZ.cs:31-32, LZ01.cs:33-34, FCMP.cs:31-32, IECP.cs:30-31, MDB4.cs:28-29)
-                case AURORA_FMT_AKLZ: m = 0x10 < len && std::memcmp(p, "AKLZ~?Qd=\xCC\xCC\xCD", 12) == 0; break;
-                case AURORA_FMT_SDPC: m = 0x10 < len && std::memcmp(p, "SDPC", 4) == 0 && (p[4] | p[5] | p[6] | p[7]) != 0; break;   // SDPC.cs:31-32
-                case AURORA_FMT_LZ01: m = 0x10 < len && std::memcmp(p, "LZ01", 4) == 0; break;
-                case AURORA_FMT_FCMP: m = 0x10 < len && std::memcmp(p, "FCMP", 4) == 0; break;
-                case AURORA_FMT_IECP: m = 0x10 < len && std::memcmp(p, "IECP", 4) == 0; break;
-                case AURORA_FMT_MDB4: m = 0x10 < len && std::memcmp(p, "MDB4", 4) == 0; break;
-                case AURORA_FMT_LZ00: m = 0x40 < len && std::memcmp(p, "LZ00", 4) == 0; break;   // LZ00.cs:37-38
-                case AURORA_FMT_ECD: {   // ECD.cs:37-38: identifier, the compressed size fits the stream, a non-zero decoded size
-                    auto be = [&](size_t at) { return (uint32_t(p[at]) << 24) | (uint32_t(p[at + 1]) << 16) | (uint32_t(p[at + 2]) << 8) | p[at + 3]; };
-                    m = 0x10 < len && std::memcmp(p, "ECD", 3) == 0 && uint64_t(be(8)) + 0x10 <= len && be(12) != 0;
-                    break;
-                }
-                default: return AURORA_NOT_SUPPORTED;   // Level5 (zlib, file name), LZSega / GCZ (no identifier)
-            }
-            match[i] = m ? 1 : 0;
-            if (m && (format == AURORA_FMT_GCLZ || format == AURORA_FMT_CXLZ || format == AURORA_FMT_COMP)) {
-                idx.push_back(i);
-                so.push_back(src_off[i] + 4);
-                sl.push_back(len - 4);
-            }
-        }
-        if (!idx.empty()) {
-            std::vector<uint8_t> mm(idx.size());
-            const int rc = aurora_is_match_batch(ctx, format == AURORA_FMT_COMP ? AURORA_FMT_LZ11 : AURORA_FMT_LZ10, opts, idx.size(),
-                                                 src_base, so.data(), sl.data(), mm.data());
-            if (rc != AURORA_OK) return rc;
-            for (size_t k = 0; k < idx.size(); k++) match[idx[k]] = mm[k];
-        }
-        return AURORA_OK;
-    }
+    if (aurora::is_wrapper_format(format)) return aurora::wrapped_is_match_batch(ctx, format, opts, n, src_base, src_off, src_len, match);
     if (format == AURORA_FMT_LZ10 || format == AURORA_FMT_LZ11 || format == AURORA_FMT_PRS) {
         // token-walk heuristics run on the device, one thread per candidate stream (csrc/ismatch.cu)
         if (n > 0xFFFFFFF0ull) return AURORA_INVALID_ARGUMENT;
@@ -1018,42 +900,14 @@ int aurora_is_match_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* 
         CU_TRY(ctx, cudaStreamSynchronize(st));
         return AURORA_OK;
     }
+    // the magic and footer rules (csrc/ismatch.cu) on the host: a peek of a few bytes per stream
     for (size_t i = 0; i < n; i++) {
-        const uint8_t* p = src_base + src_off[i];
-        bool m = false;
-        switch (format) {
-            case AURORA_FMT_YAZ0: m = magic16(i, "Yaz0", 4); break;
-            case AURORA_FMT_YAZ1: m = magic16(i, "Yaz1", 4); break;
-            case AURORA_FMT_LZHUDSON: m = 0x8 < src_len[i] && (p[0] | p[1] | p[2] | p[3]) != 0; break;   // LZHudson.cs:31-32, no file name
-            case AURORA_FMT_SMSR00: m = magic16(i, "SMSR00", 6); break;   // SMSR00.cs:36-37
-            case AURORA_FMT_BLZ: {   // BLZ.cs:31-32: the footer's compressed size is the whole stream, footer size >= 8
-                const uint64_t len = src_len[i];
-                m = len >= 8 && (uint64_t(p[len - 8]) | (uint64_t(p[len - 7]) << 8) | (uint64_t(p[len - 6]) << 16)) == len && p[len - 5] >= 8;
-                break;
-            }
-            case AURORA_FMT_LZ40:   // LZ40.cs:41-43, LZ60.cs:31-33: identifier and a non-zero size ("recognition is inaccurate!")
-            case AURORA_FMT_LZ60:
-                m = 0x8 < src_len[i] && p[0] == (format == AURORA_FMT_LZ40 ? 0x40 : 0x60) && ((p[1] | p[2] | p[3]) != 0 || (p[4] | p[5] | p[6] | p[7]) != 0);
-                break;
-            case AURORA_FMT_YAY0: m = magic16(i, "Yay0", 4); break;
-            case AURORA_FMT_MIO0: m = magic16(i, "MIO0", 4); break;
-            case AURORA_FMT_LZSS: m = magic16(i, "LZSS", 4); break;
-            case AURORA_FMT_LZ4_LEGACY: m = magic16(i, "\x02\x21\x4C\x18", 4); break;
-            case AURORA_FMT_SNAPPY: m = magic16(i, snappy_id, 10); break;
-            case AURORA_FMT_LZ4:
-                if (0x10 < src_len[i]) {
-                    const uint32_t v = uint32_t(p[0]) | (uint32_t(p[1]) << 8) | (uint32_t(p[2]) << 16) | (uint32_t(p[3]) << 24);
-                    m = v == 0x184C2102u || v == 0x184D2204u || (v >= 0x184D2A50u && v <= 0x184D2A5Fu);
-                }
-                break;
-            case AURORA_FMT_LZO:   // LZO.cs:31-39 without a file name
-                m = src_len[i] > 0 && (p[0] < 0x20);
-                break;
-            default:
-                ctx->set_error("aurora_is_match_batch: unknown format");
-                return AURORA_INVALID_ARGUMENT;
+        const int m = aurora::is_match_one(src_base + src_off[i], src_len[i], format);
+        if (m < 0) {
+            ctx->set_error("aurora_is_match_batch: unknown format");
+            return AURORA_INVALID_ARGUMENT;
         }
-        match[i] = m ? 1 : 0;
+        match[i] = uint8_t(m);
     }
     return AURORA_OK;
 }

@@ -197,12 +197,8 @@ void resolve(int format, size_t i, const uint8_t* p, uint64_t len, uint8_t* dst,
                 for (size_t k = 0; k < ends.size(); k++) {
                     const uint64_t avail = start <= len ? len - start : 0;
                     subs.push_back(Sub{i, AURORA_FMT_LZ10, std::min(start, len), avail, doff, kParseHeader, 0u});
-                    uint64_t csize = 0;
-                    const uint8_t* c = p + std::min(start, len);
-                    if (avail >= 4 && c[0] == 0x10) {
-                        csize = uint32_t(c[1]) | (uint32_t(c[2]) << 8) | (uint32_t(c[3]) << 16);
-                        if (csize == 0 && avail >= 8) csize = le32(c + 4);
-                    }
+                    uint64_t csize;   // 0 when the chunk's header does not parse
+                    core_decoded_size(AURORA_FMT_LZ10, AURORA_ENDIAN_DEFAULT, p + std::min(start, len), avail, &csize);
                     doff += csize;
                     start = pos + ends[k];
                 }
@@ -392,11 +388,11 @@ int wrapped_decoded_size(int format, const uint8_t* p, uint64_t len, uint64_t* o
     *out_size = 0;
     Plan pl;
     uint64_t at = 0;
-    uint8_t id = 0x10;
+    int core = AURORA_FMT_LZ10;
     switch (format) {
         case AURORA_FMT_GCLZ: if (!match_throw(pl, p, len, "GCLZ", 4)) return pl.status; at = 4; break;
         case AURORA_FMT_CXLZ: if (!match_throw(pl, p, len, "CXLZ", 4)) return pl.status; at = 4; break;
-        case AURORA_FMT_COMP: if (!match_throw(pl, p, len, "COMP", 4)) return pl.status; at = 4; id = 0x11; break;
+        case AURORA_FMT_COMP: if (!match_throw(pl, p, len, "COMP", 4)) return pl.status; at = 4; core = AURORA_FMT_LZ11; break;
         case AURORA_FMT_LZ_3DS: if (!match_throw(pl, p, len, "3DS-LZ\r\n", 8)) return pl.status; at = 8; break;
         case AURORA_FMT_LZ77: {
             if (!match_throw(pl, p, len, "LZ77", 4)) return pl.status;
@@ -444,16 +440,52 @@ int wrapped_decoded_size(int format, const uint8_t* p, uint64_t len, uint64_t* o
             return AURORA_OK;
         }
     }
-    // the prefixed LZ10 / LZ11 stream: type byte + u24 (LZ10.cs:47-57)
-    if (len < at + 1) return AURORA_END_OF_STREAM;
-    if (p[at] != id) return AURORA_INVALID_IDENTIFIER;
-    if (len < at + 4) return AURORA_END_OF_STREAM;
-    uint32_t v = uint32_t(p[at + 1]) | (uint32_t(p[at + 2]) << 8) | (uint32_t(p[at + 3]) << 16);
-    if (v == 0) {
-        if (len < at + 8) return AURORA_END_OF_STREAM;
-        v = le32(p + at + 4);
+    return core_decoded_size(core, AURORA_ENDIAN_DEFAULT, p + at, len - at, out_size);   // the LZ10 / LZ11 stream behind the identifier
+}
+
+// IsMatchStatic of the wrapper formats: identifier (+ a minimum length), then, for GCLZ / CXLZ / COMP, the LZ10 / LZ11
+// heuristic on the bytes behind it (GCLZ.cs:30-31, CXLZ.cs:31-32, COMP.cs:30-31, 3DS-LZ.cs:29-30, LZ77.cs:46-47, LZOn.cs:29-30,
+// Level5LZSS.cs:29-30; the LZSS family: AKLZ.cs:31-32, LZ01.cs:33-34, FCMP.cs:31-32, IECP.cs:30-31, MDB4.cs:28-29, LZ00.cs:37-38).
+// Level5.IsMatch needs zlib and the file name, LZSega / GCZ have no identifier: NOT_SUPPORTED.
+int wrapped_is_match_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* opts, size_t n, const uint8_t* src_base,
+                           const uint64_t* src_off, const uint64_t* src_len, uint8_t* match) {
+    const Family* f = family_of(format);
+    if (format == AURORA_FMT_LEVEL5 || (f && !f->magic_len)) return AURORA_NOT_SUPPORTED;
+    std::vector<size_t> idx;
+    std::vector<uint64_t> so, sl;
+    for (size_t i = 0; i < n; i++) {
+        const uint8_t* p = src_base + src_off[i];
+        const uint64_t len = src_len[i];
+        auto id = [&](uint64_t min_len, const void* magic, size_t k) { return min_len < len && std::memcmp(p, magic, k) == 0; };
+        bool m;
+        switch (format) {
+            case AURORA_FMT_GCLZ: m = id(0x8, "GCLZ", 4); break;
+            case AURORA_FMT_CXLZ: m = id(0x8, "CXLZ", 4); break;
+            case AURORA_FMT_COMP: m = id(0x8, "COMP", 4); break;
+            case AURORA_FMT_LZ_3DS: m = id(0x10, "3DS-LZ\r\n", 8); break;
+            case AURORA_FMT_LZON: m = id(0x10, kLzonMagic, 8); break;
+            case AURORA_FMT_LEVEL5_LZSS: m = id(0x10, "SSZL", 4) && (p[4] | p[5] | p[6] | p[7]) == 0; break;
+            case AURORA_FMT_LZ77: m = id(0x8, "LZ77", 4) && (p[4] == 0x10 || p[4] == 0x11 || p[4] == 0x24 || p[4] == 0x28 || p[4] == 0x30 || p[4] == 0xF7); break;
+            case AURORA_FMT_SDPC: m = id(0x10, "SDPC", 4) && (p[4] | p[5] | p[6] | p[7]) != 0; break;   // SDPC.cs:31-32
+            case AURORA_FMT_ECD:   // ECD.cs:37-38: identifier, the compressed size fits the stream, a non-zero decoded size
+                m = id(0x10, "ECD", 3) && uint64_t(be32(p + 8)) + 0x10 <= len && be32(p + 12) != 0;
+                break;
+            default: m = id(format == AURORA_FMT_LZ00 ? 0x40 : 0x10, f->magic, f->magic_len); break;
+        }
+        match[i] = m ? 1 : 0;
+        if (m && (format == AURORA_FMT_GCLZ || format == AURORA_FMT_CXLZ || format == AURORA_FMT_COMP)) {
+            idx.push_back(i);
+            so.push_back(src_off[i] + 4);
+            sl.push_back(len - 4);
+        }
     }
-    *out_size = v;
+    if (!idx.empty()) {
+        std::vector<uint8_t> mm(idx.size());
+        const int rc = aurora_is_match_batch(ctx, format == AURORA_FMT_COMP ? AURORA_FMT_LZ11 : AURORA_FMT_LZ10, opts, idx.size(),
+                                             src_base, so.data(), sl.data(), mm.data());
+        if (rc != AURORA_OK) return rc;
+        for (size_t k = 0; k < idx.size(); k++) match[idx[k]] = mm[k];
+    }
     return AURORA_OK;
 }
 

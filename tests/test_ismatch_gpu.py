@@ -7,26 +7,14 @@ import numpy as np
 import pytest
 
 from auroralib.compression_b200 import _abi as A
-from tests.util import ALL_FORMATS, SIZED_FORMATS, corrupt, fmt_id, synth
+from tests.util import MATCHABLE, SIZED_FORMATS, decoded_size_blobs, fmt_id, is_match_blobs, rom_like_image, synth
 
 pytestmark = pytest.mark.gpu
-
-MATCHABLE = [f for f in ALL_FORMATS if f not in (A.FMT_LZ4_BLOCK, A.FMT_SNAPPY_BLOCK)]
 
 
 @pytest.mark.parametrize("fmt", MATCHABLE, ids=fmt_id)
 def test_is_match_parity(codec, oracle, bmp, fmt):
-    rng = np.random.default_rng(500 + fmt)
-    blobs = []
-    for i in range(120):
-        raw = synth(rng, int(rng.integers(5, 6000)), i % 5)
-        for f in (fmt, ALL_FORMATS[i % len(ALL_FORMATS)]):
-            c, st = oracle.encode(f, raw, A.make_opts(quality=int(rng.choice([0, 8]))))
-            if st == 0:
-                blobs.append(c)
-                blobs.append(corrupt(rng, c, i % 5))
-        blobs.append(raw)
-    blobs += [b"", b"\x10", b"\x10\x00\x00\x00", bmp[:300], bytes(64), bytes([0x10, 5, 0, 0, 0, 1, 2, 3, 4, 5]), bytes([0x11] + [0] * 20)]
+    blobs = is_match_blobs(oracle, bmp, fmt)
     got = codec.is_match_batch(fmt, blobs)
     ref = np.array([oracle.is_match(fmt, b) for b in blobs])
     bad = np.nonzero(got != ref)[0]
@@ -36,13 +24,7 @@ def test_is_match_parity(codec, oracle, bmp, fmt):
 
 @pytest.mark.parametrize("fmt", SIZED_FORMATS, ids=fmt_id)
 def test_decoded_size_parity(codec, oracle, fmt):
-    rng = np.random.default_rng(600 + fmt)
-    blobs = []
-    for i in range(60):
-        raw = synth(rng, int(rng.integers(1, 3000)), i % 5)
-        for order in (A.ENDIAN_BIG, A.ENDIAN_LITTLE):
-            c, st = oracle.encode(fmt, raw, A.make_opts(quality=0, byte_order=order))
-            blobs += [c, corrupt(rng, c, 4), corrupt(rng, c, 1)]
+    blobs = decoded_size_blobs(oracle, fmt)
     for opts in (None, A.make_opts(byte_order=A.ENDIAN_LITTLE), A.make_opts(byte_order=A.ENDIAN_BIG)):
         size, status = codec.decoded_size_batch(fmt, blobs, opts)
         for b, s, st in zip(blobs, size, status):
@@ -107,14 +89,7 @@ def test_offset_scan_of_a_rom_like_image(codec, oracle, bmp):
     rng = np.random.default_rng(77)
     assets = [bmp[1000:9000], bytes(3000), synth(rng, 5000, 0), synth(rng, 2500, 2)]
     for fmt in (A.FMT_YAZ0, A.FMT_LZ10, A.FMT_LZ11, A.FMT_MIO0, A.FMT_LZ4, A.FMT_PRS):
-        image = bytearray(rng.integers(0, 256, size=700, dtype=np.uint8).tobytes())
-        starts = []
-        for a in assets:
-            c, st = oracle.encode(fmt, a, A.make_opts(quality=8))
-            assert st == 0
-            starts.append(len(image))
-            image += c + rng.integers(0, 256, size=int(rng.integers(10, 400)), dtype=np.uint8).tobytes()
-        image = bytes(image)
+        image, starts = rom_like_image(oracle, rng, fmt, assets)
         got = codec.scan_offsets(fmt, image)
         ref = np.array([oracle.is_match(fmt, image[i:]) for i in range(len(image))])
         assert (got == ref).all(), (fmt_id(fmt), int((got != ref).sum()))

@@ -5,7 +5,9 @@ real kernel file (everything above its "// ---- kernel" line) is compiled by g++
     sequential replay): every format and quality, the small-match table, matches beyond the data ring's lookahead, the
     three-section writers, CompatibilityMode, unaligned sources, too-small destinations;
   * decoders — csrc/decode_flaglz.cu (the headline kernel: a parser warp and a resolver warp per stream slot), decode_bytelz.cu,
-    decode_blz.cu: valid and corrupt streams, exact / short / larger destinations; status, out_len, consumed and bytes.
+    decode_blz.cu: valid and corrupt streams, exact / short / larger destinations; status, out_len, consumed and bytes;
+  * the IsMatch and GetDecompressedSize rules of csrc/ismatch.cu (plain per-stream functions, no lanes): every matchable format
+    on streams, corrupted streams, raw data and every offset of a ROM-like image.
 No GPU: this is the check of the kernels' lane-level logic that runs in the CPU suite, on more inputs than GPU time allows."""
 import ctypes as C
 import os
@@ -15,7 +17,7 @@ import numpy as np
 import pytest
 
 from auroralib.compression_b200 import _abi as A
-from tests.util import fmt_id, synth
+from tests.util import MATCHABLE, SIZED_FORMATS, decoded_size_blobs, fmt_id, is_match_blobs, rom_like_image, synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SIMT = os.path.join(ROOT, "tests", "simt")
@@ -438,3 +440,51 @@ def test_bytelz_size_scan_on_emulated_lanes(simt_bytelz_dec, oracle, bmp, fmt):
     # (the kernel reports the length with DST_TOO_SMALL against the zero capacity; api.cu's size path reads out_len)
     assert (status == A.DST_TOO_SMALL).all() and [int(x) for x in out_len] == [len(r) for r in raws]
     assert [int(x) for x in consumed] == [len(c) for c in comps]
+
+
+# ---- the IsMatch and GetDecompressedSize rules of csrc/ismatch.cu: the library runs them on the host for the magic formats and
+#      in the IsMatch / offset-scan kernels for every format, so one CPU build of them checks both
+@pytest.fixture(scope="session")
+def simt_rules():
+    lib = _build("ismatch", "ismatch_harness.cpp", "ISMATCH_DEVICE_INC")
+    lib.simt_is_match_one.restype = C.c_int
+    lib.simt_is_match_one.argtypes = [C.c_void_p, C.c_uint64, C.c_int]
+    lib.simt_core_decoded_size.restype = C.c_int
+    lib.simt_core_decoded_size.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+    return lib
+
+
+@pytest.mark.parametrize("fmt", MATCHABLE, ids=fmt_id)
+def test_is_match_rules_on_the_cpu(simt_rules, oracle, bmp, fmt):
+    blobs = is_match_blobs(oracle, bmp, fmt)
+    got = [simt_rules.simt_is_match_one(b, len(b), fmt) for b in blobs]
+    ref = [int(oracle.is_match(fmt, b)) for b in blobs]
+    bad = [i for i in range(len(blobs)) if got[i] != ref[i]]
+    assert not bad, f"{fmt_id(fmt)}: {len(bad)} of {len(blobs)} differ, first #{bad[0]} rule={got[bad[0]]} ref={ref[bad[0]]} blob={blobs[bad[0]][:24].hex()}"
+    assert sum(got) > 0
+    # every offset of a ROM-like image: the stream at offset i runs to the end of the image, as in the offset-scan kernel
+    rng = np.random.default_rng(77 + fmt)
+    image, _ = rom_like_image(oracle, rng, fmt, [bmp[1000:9000], bytes(3000), synth(rng, 5000, 0), synth(rng, 2500, 2)])
+    a = np.frombuffer(image, dtype=np.uint8)
+    got = [simt_rules.simt_is_match_one(a.ctypes.data + i, len(image) - i, fmt) for i in range(len(image))]
+    ref = [int(oracle.is_match(fmt, image[i:])) for i in range(len(image))]
+    bad = [i for i in range(len(image)) if got[i] != ref[i]]
+    assert not bad, f"{fmt_id(fmt)}: {len(bad)} of {len(image)} offsets differ, first {bad[0]}"
+
+
+def test_formats_without_an_is_match_rule(simt_rules):
+    blob = bytes(range(64))
+    for fmt in (A.FMT_LZ4_BLOCK, A.FMT_SNAPPY_BLOCK, A.FMT_GCLZ):
+        assert simt_rules.simt_is_match_one(blob, len(blob), fmt) == -1, fmt_id(fmt)
+
+
+@pytest.mark.parametrize("fmt", SIZED_FORMATS, ids=fmt_id)
+def test_decoded_size_rules_on_the_cpu(simt_rules, oracle, fmt):
+    blobs = decoded_size_blobs(oracle, fmt)
+    for order in (A.ENDIAN_DEFAULT, A.ENDIAN_LITTLE, A.ENDIAN_BIG):
+        opts = A.make_opts(byte_order=order)
+        for b in blobs:
+            size = C.c_uint64(77)
+            st = simt_rules.simt_core_decoded_size(fmt, order, b, len(b), C.byref(size))
+            rs, rst = oracle.decoded_size(fmt, b, opts)
+            assert (size.value, st) == (rs, rst) or (st != 0 and rst != 0), (fmt_id(fmt), order, b[:16].hex(), size.value, st, rs, rst)

@@ -5,6 +5,7 @@ from auroralib.compression_b200 import _abi as A
 
 ALL_FORMATS = [A.FMT_YAZ0, A.FMT_YAZ1, A.FMT_YAY0, A.FMT_MIO0, A.FMT_LZ10, A.FMT_LZ11, A.FMT_LZSS, A.FMT_LZ4,
                A.FMT_LZ4_LEGACY, A.FMT_LZ4_BLOCK, A.FMT_LZO, A.FMT_SNAPPY, A.FMT_SNAPPY_BLOCK, A.FMT_PRS, A.FMT_LZHUDSON, A.FMT_LZ40, A.FMT_LZ60, A.FMT_SMSR00, A.FMT_BLZ]
+MATCHABLE = [f for f in ALL_FORMATS if f not in (A.FMT_LZ4_BLOCK, A.FMT_SNAPPY_BLOCK)]   # the formats with an IsMatch rule
 SIZED_FORMATS = [A.FMT_YAZ0, A.FMT_YAZ1, A.FMT_YAY0, A.FMT_MIO0, A.FMT_LZ10, A.FMT_LZ11, A.FMT_LZSS, A.FMT_LZHUDSON, A.FMT_LZ40, A.FMT_LZ60, A.FMT_SMSR00, A.FMT_BLZ]
 
 
@@ -81,3 +82,43 @@ def corrupt(rng, blob, mode):
     if mode == 4:
         return bytes(b[:int(rng.integers(0, min(17, len(b) + 1)))])
     return bytes(b)
+
+
+def is_match_blobs(oracle, bmp, fmt):
+    """IsMatch inputs for one format: oracle streams of it and of the other formats, each also corrupted, the raw data, and
+    short / zero / header-only edge blobs."""
+    rng = np.random.default_rng(500 + fmt)
+    blobs = []
+    for i in range(120):
+        raw = synth(rng, int(rng.integers(5, 6000)), i % 5)
+        for f in (fmt, ALL_FORMATS[i % len(ALL_FORMATS)]):
+            c, st = oracle.encode(f, raw, A.make_opts(quality=int(rng.choice([0, 8]))))
+            if st == 0:
+                blobs.append(c)
+                blobs.append(corrupt(rng, c, i % 5))
+        blobs.append(raw)
+    return blobs + [b"", b"\x10", b"\x10\x00\x00\x00", bmp[:300], bytes(64), bytes([0x10, 5, 0, 0, 0, 1, 2, 3, 4, 5]), bytes([0x11] + [0] * 20)]
+
+
+def decoded_size_blobs(oracle, fmt):
+    """GetDecompressedSize inputs for one format: oracle streams in both byte orders, cut inside the header or with a byte flipped."""
+    rng = np.random.default_rng(600 + fmt)
+    blobs = []
+    for i in range(60):
+        raw = synth(rng, int(rng.integers(1, 3000)), i % 5)
+        for order in (A.ENDIAN_BIG, A.ENDIAN_LITTLE):
+            c, st = oracle.encode(fmt, raw, A.make_opts(quality=0, byte_order=order))
+            blobs += [c, corrupt(rng, c, 4), corrupt(rng, c, 1)]
+    return blobs
+
+
+def rom_like_image(oracle, rng, fmt, assets):
+    """The CLI's `-scan` input: `assets` compressed at quality 8 between runs of junk -> (image, start offset of each asset)."""
+    image = bytearray(rng.integers(0, 256, size=700, dtype=np.uint8).tobytes())
+    starts = []
+    for a in assets:
+        c, st = oracle.encode(fmt, a, A.make_opts(quality=8))
+        assert st == 0
+        starts.append(len(image))
+        image += c + rng.integers(0, 256, size=int(rng.integers(10, 400)), dtype=np.uint8).tobytes()
+    return bytes(image), starts
