@@ -15,7 +15,8 @@ EXPORTS = [
     "aurora_last_error_string", "aurora_status_string", "aurora_pinned_alloc", "aurora_pinned_free",
     "aurora_lz_props_window", "aurora_lz_props_bits", "aurora_codec_opts_init", "aurora_decoded_size_batch",
     "aurora_is_match_batch", "aurora_scan_offsets", "aurora_decode_batch", "aurora_encode_bound", "aurora_encode_batch",
-    "aurora_decode_batch_device", "aurora_encode_batch_device", "aurora_kernel_launch_count",
+    "aurora_decode_batch_device", "aurora_encode_batch_device", "aurora_decoded_size_batch_device", "aurora_is_match_batch_device",
+    "aurora_scan_offsets_device", "aurora_kernel_launch_count",
 ]
 
 _LIB = None
@@ -69,6 +70,12 @@ def load():
     L.aurora_decode_batch_device.argtypes = [vp, i32, i32, opts, sz, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.aurora_encode_batch_device.restype = i32
     L.aurora_encode_batch_device.argtypes = [vp, i32, i32, opts, sz, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.aurora_decoded_size_batch_device.restype = i32
+    L.aurora_decoded_size_batch_device.argtypes = [vp, i32, i32, opts, sz, vp, u64, vp, vp, i32, vp, vp, vp]
+    L.aurora_is_match_batch_device.restype = i32
+    L.aurora_is_match_batch_device.argtypes = [vp, i32, i32, opts, sz, vp, vp, vp, vp, vp]
+    L.aurora_scan_offsets_device.restype = i32
+    L.aurora_scan_offsets_device.argtypes = [vp, i32, i32, opts, vp, u64, vp, vp]
     L.aurora_kernel_launch_count.restype = u64
     L.aurora_kernel_launch_count.argtypes = [vp]
     _LIB = L

@@ -167,6 +167,64 @@ class BatchCodec:
             d_status.data_ptr(), stream)
         self._check(rc, "aurora_encode_batch_device")
 
+    def decoded_size_device(self, fmt, d_src, d_off, d_len, d_size, d_status, opts=None, size_scan=False, device=0, stream=None):
+        """GetDecompressedSize of device streams into d_size (int64) / d_status (int32): the answers of decoded_size_batch.
+        d_src must start 16-byte aligned.  Asynchronous on `stream` (a cudaStream_t handle; None = the library's stream)."""
+        opts = opts or _abi.make_opts()
+        rc = self._L.aurora_decoded_size_batch_device(
+            self._ctx, device, fmt, C.byref(opts), d_off.numel(), d_src.data_ptr(), d_src.numel(), d_off.data_ptr(),
+            d_len.data_ptr(), 1 if size_scan else 0, d_size.data_ptr(), d_status.data_ptr(), stream)
+        self._check(rc, "aurora_decoded_size_batch_device")
+
+    def is_match_device(self, fmt, d_src, d_off, d_len, d_match, opts=None, device=0, stream=None):
+        """IsMatch of device streams into d_match (uint8 or bool, one byte per stream).  Asynchronous on `stream`."""
+        opts = opts or _abi.make_opts()
+        rc = self._L.aurora_is_match_batch_device(self._ctx, device, fmt, C.byref(opts), d_off.numel(), d_src.data_ptr(),
+                                                  d_off.data_ptr(), d_len.data_ptr(), d_match.data_ptr(), stream)
+        self._check(rc, "aurora_is_match_batch_device")
+
+    def scan_offsets_device(self, fmt, d_image, d_match, opts=None, device=0, stream=None):
+        """IsMatch at every byte offset of a device image into d_match (d_image.numel() bytes).  Asynchronous on `stream`."""
+        opts = opts or _abi.make_opts()
+        rc = self._L.aurora_scan_offsets_device(self._ctx, device, fmt, C.byref(opts), d_image.data_ptr(), d_image.numel(),
+                                                d_match.data_ptr(), stream)
+        self._check(rc, "aurora_scan_offsets_device")
+
+    def decode_device_sized(self, fmt, d_src, d_off, d_len, opts=None, size_scan=True, max_size=1 << 30, device=0, stream=None):
+        """Decode device streams whose decoded sizes the caller does not know.
+        -> (d_dst, d_dst_off, d_cap, d_out_len, d_consumed, d_status), all on `stream` (None: torch's current stream).
+
+        The sizes come from decoded_size_device (with a size scan for the byte-LZ formats when size_scan is set).  A stream
+        gets the capacity its size names when that is OK and at most `max_size` bytes, else 0, so a forged header cannot
+        make this allocate gigabytes: such a stream reports the status of a fixed destination that is too small.  The
+        destination windows are packed at 16-byte aligned offsets.  The one host read is the total, to allocate d_dst."""
+        import torch
+        if d_src.data_ptr() % 16:
+            raise AuroraError("decode_device_sized: INVALID_ARGUMENT: d_src must start at a 16-byte aligned address "
+                              f"(data_ptr() % 16 == {d_src.data_ptr() % 16}; a sliced view may be misaligned)")
+        dev = d_src.device
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+        ts = torch.cuda.ExternalStream(stream, device=dev)
+        n = d_off.numel()
+        with torch.cuda.stream(ts):
+            d_size = torch.empty(n, dtype=torch.int64, device=dev)
+            d_sst = torch.empty(n, dtype=torch.int32, device=dev)
+            d_out_len = torch.empty(n, dtype=torch.int64, device=dev)
+            d_consumed = torch.empty(n, dtype=torch.int64, device=dev)
+            d_status = torch.empty(n, dtype=torch.int32, device=dev)
+            if n == 0:
+                return torch.zeros(16, dtype=torch.uint8, device=dev), d_size, torch.empty_like(d_size), d_out_len, d_consumed, d_status
+            self.decoded_size_device(fmt, d_src, d_off, d_len, d_size, d_sst, opts, size_scan, device, stream)
+            d_cap = torch.where((d_sst == _abi.OK) & (d_size <= max_size), d_size, torch.zeros_like(d_size))
+            padded = (d_cap + 15) & ~15
+            ends = torch.cumsum(padded, 0)
+            d_dst_off = ends - padded
+            total = int(ends[-1])
+            d_dst = torch.empty(max(total, 16), dtype=torch.uint8, device=dev)
+            self.decode_device(fmt, d_src, d_off, d_len, d_dst, d_dst_off, d_cap, d_out_len, d_consumed, d_status, opts, device, stream)
+        return d_dst, d_dst_off, d_cap, d_out_len, d_consumed, d_status
+
 
 _DEFAULT = None
 

@@ -84,6 +84,7 @@ struct DeviceCtx {
     cudaStream_t s_in = nullptr, s_out = nullptr;   // copy engines of the pipelined host path
     std::vector<cudaEvent_t> ev_in, ev_k;
     DevBuf src, dst, desc, ticket, scratch, order;
+    DevBuf size_scan;   // aurora_decoded_size_batch_device with a size scan: n zeroed offsets / capacities, then n consumed
     HostBuf hdesc;
     std::mutex mu;   // one batch at a time per device
 };
@@ -119,10 +120,14 @@ bool is_flaglz(int f) {
            f == AURORA_FMT_LZ10 || f == AURORA_FMT_LZ11 || f == AURORA_FMT_LZSS || f == AURORA_FMT_LZHUDSON ||
            f == AURORA_FMT_LZ40 || f == AURORA_FMT_LZ60 || f == AURORA_FMT_SMSR00;
 }
-bool is_bytelz(int f) {
-    return f == AURORA_FMT_LZ4 || f == AURORA_FMT_LZ4_BLOCK || f == AURORA_FMT_LZ4_LEGACY || f == AURORA_FMT_LZO ||
-           f == AURORA_FMT_SNAPPY || f == AURORA_FMT_SNAPPY_BLOCK || f == AURORA_FMT_PRS;
-}
+
+// The formats each query takes, one predicate per query for its host and its device entry point.  The host entry points
+// also take the wrapper formats (their headers are resolved on the host); the device entry points take exactly the formats
+// aurora_decode_batch_device decodes.
+bool size_query_format(int f) { return is_flaglz(f) || is_bytelz(f) || f == AURORA_FMT_BLZ; }
+// every IsMatch rule rejects an empty stream without reading it, so this asks only whether is_match_one has a rule
+bool is_match_query_format(int f) { return aurora::is_match_one(nullptr, 0, f) >= 0; }
+bool scan_query_format(int f) { return (is_flaglz(f) || is_bytelz(f)) && f != AURORA_FMT_LZ4_BLOCK && f != AURORA_FMT_SNAPPY_BLOCK; }
 
 int ceil_log2(long long x) {
     int b = 0;
@@ -739,6 +744,7 @@ void aurora_shutdown(aurora_ctx* ctx) {
         d->ticket.release();
         d->scratch.release();
         d->order.release();
+        d->size_scan.release();
         d->hdesc.release();
         for (cudaEvent_t e : d->ev_in) cudaEventDestroy(e);
         for (cudaEvent_t e : d->ev_k) cudaEventDestroy(e);
@@ -827,22 +833,16 @@ int aurora_decoded_size_batch(aurora_ctx* ctx, int format, const aurora_codec_op
     if (!ctx) return AURORA_INVALID_ARGUMENT;
     if (n == 0) return AURORA_OK;
     if (!src_base || !src_off || !src_len || !out_size || !status) return AURORA_INVALID_ARGUMENT;
-    // GetDecompressedSize is a header peek (e.g. Yaz0.cs:50-55, LZ10.cs:47-57): a few bytes of host memory
-    if (aurora::is_wrapper_format(format) || is_flaglz(format) || format == AURORA_FMT_BLZ) {
-        const int bo = opts ? opts->byte_order : AURORA_ENDIAN_DEFAULT;
-        for (size_t i = 0; i < n; i++) {
-            const uint8_t* p = src_base + src_off[i];
-            status[i] = aurora::is_wrapper_format(format) ? aurora::wrapped_decoded_size(format, p, src_len[i], &out_size[i])
-                                                          : aurora::core_decoded_size(format, bo, p, src_len[i], &out_size[i]);
-        }
+    if (aurora::is_wrapper_format(format)) {
+        for (size_t i = 0; i < n; i++) status[i] = aurora::wrapped_decoded_size(format, src_base + src_off[i], src_len[i], &out_size[i]);
         return AURORA_OK;
     }
-    if (!is_bytelz(format)) return AURORA_INVALID_ARGUMENT;
-    if (!size_scan) {
-        for (size_t i = 0; i < n; i++) {
-            out_size[i] = 0;
-            status[i] = AURORA_NOT_SUPPORTED;   // LZ4/LZO/Snappy/PRS do not implement IProvidesDecompressedSize
-        }
+    if (!size_query_format(format)) return AURORA_INVALID_ARGUMENT;
+    if (!size_scan || !is_bytelz(format)) {
+        // GetDecompressedSize is a header peek (e.g. Yaz0.cs:50-55, LZ10.cs:47-57): a few bytes of host memory.  The byte-LZ
+        // formats have no size header: NOT_SUPPORTED
+        const int bo = opts ? opts->byte_order : AURORA_ENDIAN_DEFAULT;
+        for (size_t i = 0; i < n; i++) status[i] = aurora::decoded_size_one(format, bo, src_base + src_off[i], src_len[i], &out_size[i]);
         return AURORA_OK;
     }
     // size-only pre-pass on the device: same parser, all stores dropped
@@ -854,8 +854,7 @@ int aurora_decoded_size_batch(aurora_ctx* ctx, int format, const aurora_codec_op
                             out_size, cons.data(), status, 1);
     });
     if (rc != AURORA_OK) return rc;
-    for (size_t i = 0; i < n; i++)
-        if (status[i] == AURORA_DST_TOO_SMALL) status[i] = AURORA_OK;
+    for (size_t i = 0; i < n; i++) status[i] = aurora::size_scan_status(status[i]);
     return AURORA_OK;
 }
 
@@ -866,6 +865,10 @@ int aurora_is_match_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* 
     if (n == 0) return AURORA_OK;
     if (!src_base || !src_off || !src_len || !match) return AURORA_INVALID_ARGUMENT;
     if (aurora::is_wrapper_format(format)) return aurora::wrapped_is_match_batch(ctx, format, opts, n, src_base, src_off, src_len, match);
+    if (!is_match_query_format(format)) {
+        ctx->set_error("aurora_is_match_batch: unknown format");
+        return AURORA_INVALID_ARGUMENT;
+    }
     if (format == AURORA_FMT_LZ10 || format == AURORA_FMT_LZ11 || format == AURORA_FMT_PRS) {
         // token-walk heuristics run on the device, one thread per candidate stream (csrc/ismatch.cu)
         if (n > 0xFFFFFFF0ull) return AURORA_INVALID_ARGUMENT;
@@ -901,14 +904,7 @@ int aurora_is_match_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* 
         return AURORA_OK;
     }
     // the magic and footer rules (csrc/ismatch.cu) on the host: a peek of a few bytes per stream
-    for (size_t i = 0; i < n; i++) {
-        const int m = aurora::is_match_one(src_base + src_off[i], src_len[i], format);
-        if (m < 0) {
-            ctx->set_error("aurora_is_match_batch: unknown format");
-            return AURORA_INVALID_ARGUMENT;
-        }
-        match[i] = uint8_t(m);
-    }
+    for (size_t i = 0; i < n; i++) match[i] = uint8_t(aurora::is_match_one(src_base + src_off[i], src_len[i], format));
     return AURORA_OK;
 }
 
@@ -916,9 +912,7 @@ int aurora_scan_offsets(aurora_ctx* ctx, int format, const aurora_codec_opts* op
     (void)opts;
     if (!ctx) return AURORA_INVALID_ARGUMENT;
     if (len == 0) return AURORA_OK;
-    if (!image || !match || !(is_flaglz(format) || is_bytelz(format)) || format == AURORA_FMT_LZ4_BLOCK || format == AURORA_FMT_SNAPPY_BLOCK ||
-        len > 0xFFFFFFFF00ull)
-        return AURORA_INVALID_ARGUMENT;
+    if (!image || !match || !scan_query_format(format) || len > 0xFFFFFFFF00ull) return AURORA_INVALID_ARGUMENT;
     DeviceCtx* d = ctx->devs[0];
     std::lock_guard<std::mutex> guard(d->mu);
     CU_TRY(ctx, cudaSetDevice(d->dev));
@@ -979,6 +973,100 @@ int aurora_decode_batch_device(aurora_ctx* ctx, int device, int format, const au
     P.ticket = static_cast<unsigned int*>(d->ticket.p);
     P.n = uint32_t(n);
     CU_TRY(ctx, launch_decode(P, d->sm_count, st));
+    ctx->launches++;
+    return AURORA_OK;
+}
+
+int aurora_decoded_size_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts, size_t n,
+                                     const uint8_t* d_src_base, uint64_t src_total, const uint64_t* d_src_off,
+                                     const uint64_t* d_src_len, int size_scan, uint64_t* d_out_size, int32_t* d_status, void* stream) {
+    if (!ctx || device < 0 || device >= int(ctx->devs.size())) return AURORA_INVALID_ARGUMENT;
+    if (n == 0) return AURORA_OK;
+    if (!d_src_base || !d_src_off || !d_src_len || !d_out_size || !d_status || n > 0xFFFFFFF0ull) return AURORA_INVALID_ARGUMENT;
+    if (!size_query_format(format)) {
+        ctx->set_error("aurora_decoded_size_batch_device: wrapper or unknown format (the wrapper formats: aurora_decoded_size_batch)");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    if ((reinterpret_cast<uintptr_t>(d_src_base) & 15) != 0) {
+        ctx->set_error("aurora_decoded_size_batch_device: d_src_base must be 16-byte aligned");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    DeviceCtx* d = ctx->devs[device];
+    std::lock_guard<std::mutex> guard(d->mu);
+    CU_TRY(ctx, cudaSetDevice(d->dev));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+    if (!size_scan || !is_bytelz(format)) {   // the header peek (NOT_SUPPORTED for the byte-LZ formats), one thread per stream
+        const int bo = opts ? opts->byte_order : AURORA_ENDIAN_DEFAULT;
+        CU_TRY(ctx, launch_decoded_size(d_src_base, d_src_off, d_src_len, d_out_size, d_status, uint32_t(n), format, bo, st));
+        ctx->launches++;
+        return AURORA_OK;
+    }
+    // size scan: the decode kernel in size_only mode on the caller's streams (the parser with every store dropped) against
+    // zero destination offsets and capacities, then DST_TOO_SMALL -> OK as in aurora_decoded_size_batch
+    DecodeParams P{};
+    fill_decode_params(P, format, opts);   // (its only per-batch override is for LZSS properties)
+    P.size_only = 1;
+    CU_TRY(ctx, d->size_scan.reserve(2 * n * sizeof(uint64_t)));
+    CU_TRY(ctx, d->ticket.reserve(256));
+    uint64_t* zero = static_cast<uint64_t*>(d->size_scan.p);
+    CU_TRY(ctx, cudaMemsetAsync(zero, 0, n * sizeof(uint64_t), st));
+    CU_TRY(ctx, cudaMemsetAsync(d->ticket.p, 0, 64, st));
+    P.src_base = d_src_base;
+    P.src_limit = align_up(src_total, 16);   // the allocation must be readable up to the next multiple of 16
+    P.src_off = d_src_off;
+    P.src_len = d_src_len;
+    P.dst_base = static_cast<uint8_t*>(d->size_scan.p);   // never written in size_only mode
+    P.dst_off = zero;
+    P.dst_cap = zero;
+    P.out_len = d_out_size;
+    P.consumed = zero + n;
+    P.status = d_status;
+    P.order = nullptr;
+    P.ticket = static_cast<unsigned int*>(d->ticket.p);
+    P.n = uint32_t(n);
+    CU_TRY(ctx, launch_decode(P, d->sm_count, st));
+    ctx->launches++;
+    CU_TRY(ctx, launch_size_scan_status(d_status, uint32_t(n), st));
+    ctx->launches++;
+    return AURORA_OK;
+}
+
+int aurora_is_match_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts, size_t n,
+                                 const uint8_t* d_src_base, const uint64_t* d_src_off, const uint64_t* d_src_len, uint8_t* d_match,
+                                 void* stream) {
+    (void)opts;
+    if (!ctx || device < 0 || device >= int(ctx->devs.size())) return AURORA_INVALID_ARGUMENT;
+    if (n == 0) return AURORA_OK;
+    if (!d_src_base || !d_src_off || !d_src_len || !d_match || n > 0xFFFFFFF0ull) return AURORA_INVALID_ARGUMENT;
+    if (!is_match_query_format(format)) {
+        ctx->set_error("aurora_is_match_batch_device: no IsMatch rule for this format on the device (the wrapper formats: "
+                       "aurora_is_match_batch)");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    DeviceCtx* d = ctx->devs[device];
+    std::lock_guard<std::mutex> guard(d->mu);
+    CU_TRY(ctx, cudaSetDevice(d->dev));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+    CU_TRY(ctx, launch_is_match(d_src_base, d_src_off, d_src_len, d_match, uint32_t(n), format, st));
+    ctx->launches++;
+    return AURORA_OK;
+}
+
+int aurora_scan_offsets_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts, const uint8_t* d_image,
+                               uint64_t len, uint8_t* d_match, void* stream) {
+    (void)opts;
+    if (!ctx || device < 0 || device >= int(ctx->devs.size())) return AURORA_INVALID_ARGUMENT;
+    if (len == 0) return AURORA_OK;
+    if (!d_image || !d_match || len > 0xFFFFFFFF00ull) return AURORA_INVALID_ARGUMENT;
+    if (!scan_query_format(format)) {
+        ctx->set_error("aurora_scan_offsets_device: this format has no offset scan (as in aurora_scan_offsets)");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    DeviceCtx* d = ctx->devs[device];
+    std::lock_guard<std::mutex> guard(d->mu);
+    CU_TRY(ctx, cudaSetDevice(d->dev));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+    CU_TRY(ctx, launch_scan(d_image, len, d_match, format, st));
     ctx->launches++;
     return AURORA_OK;
 }

@@ -26,7 +26,19 @@ int encode_core_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* opts
 __host__ __device__ int is_match_one(const uint8_t* p, uint64_t len, int format);
 // core_decoded_size: the header peek of BLZ and the flag-LZ formats.  A status; *size is 0 unless it is AURORA_OK.
 // AURORA_INVALID_ARGUMENT for a format without a size header.
-int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size);
+__host__ __device__ int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size);
+// decoded_size_one: GetDecompressedSize of one stream of a core format without a size scan — AURORA_NOT_SUPPORTED and size 0
+// for the byte-LZ formats, the header peek for the others.  Both aurora_decoded_size_batch and the device's
+// decoded_size_kernel call it.
+__host__ __device__ int decoded_size_one(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size);
+// size_scan_status: the status a size scan reports for a stream, from the status of its size-only decode (capacity 0).
+__host__ __device__ int size_scan_status(int status);
+
+// the byte-LZ formats: LZ4, LZ4 block, LZ4 legacy, LZO, Snappy, Snappy block, PRS (no size header; decode_bytelz.cu)
+__host__ __device__ inline bool is_bytelz(int f) {
+    return f == AURORA_FMT_LZ4 || f == AURORA_FMT_LZ4_BLOCK || f == AURORA_FMT_LZ4_LEGACY || f == AURORA_FMT_LZO ||
+           f == AURORA_FMT_SNAPPY || f == AURORA_FMT_SNAPPY_BLOCK || f == AURORA_FMT_PRS;
+}
 
 // wrapper formats (wrappers.cu)
 bool is_wrapper_format(int format);

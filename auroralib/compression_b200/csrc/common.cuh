@@ -84,6 +84,11 @@ cudaError_t launch_lcg_xor(uint8_t* base, const uint64_t* d_off, const uint64_t*
 cudaError_t launch_scan(const uint8_t* image, uint64_t len, uint8_t* match, int format, cudaStream_t st);
 cudaError_t launch_is_match(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint8_t* match, uint32_t n,
                             int format, cudaStream_t st);
+// GetDecompressedSize of every stream (decoded_size_one, one thread per stream), and the status fix-up of a size scan
+// (size_scan_status over the statuses of a size-only decode); ismatch.cu
+cudaError_t launch_decoded_size(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint64_t* size,
+                                int32_t* status, uint32_t n, int format, int byte_order, cudaStream_t st);
+cudaError_t launch_size_scan_status(int32_t* status, uint32_t n, cudaStream_t st);
 
 #ifdef __CUDACC__
 // ------------------------------------------------------------------------------------------------

@@ -6,8 +6,8 @@
 // per candidate stream, reading the blob straight from global memory (this is the data-parallel form of the CLI's
 // byte-by-byte `-scan` loop, Commands/ScanDecompressCommand.cs:23-39).  An exception inside the reference's walk (a read past
 // the end) makes IsMatch false here, like the oracle.
-#include <cstring>
-
+// core_decoded_size and decoded_size_one are __host__ __device__ too: aurora_decoded_size_batch runs them on the host,
+// aurora_decoded_size_batch_device in decoded_size_kernel, one thread per stream.
 #include "api_internal.hpp"
 #include "common.cuh"
 
@@ -172,7 +172,7 @@ __host__ __device__ int is_match_one(const uint8_t* p, uint64_t len, int format)
     return -1;
 }
 
-int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size) {
+__host__ __device__ int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size) {
     auto be32 = [](const uint8_t* q) { return (uint32_t(q[0]) << 24) | (uint32_t(q[1]) << 16) | (uint32_t(q[2]) << 8) | q[3]; };
     auto le32 = [](const uint8_t* q) { return uint32_t(q[0]) | (uint32_t(q[1]) << 8) | (uint32_t(q[2]) << 16) | (uint32_t(q[3]) << 24); };
     *size = 0;
@@ -190,7 +190,8 @@ int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len
             return AURORA_OK;
         case AURORA_FMT_SMSR00:   // SMSR00.cs:40-46
             if (len < 6) return AURORA_END_OF_STREAM;
-            if (std::memcmp(p, "SMSR00", 6) != 0) return AURORA_INVALID_IDENTIFIER;
+            for (int k = 0; k < 6; k++)
+                if (p[k] != uint8_t("SMSR00"[k])) return AURORA_INVALID_IDENTIFIER;
             if (len < 12) return AURORA_END_OF_STREAM;
             *size = be32(p + 8);
             return AURORA_OK;
@@ -211,7 +212,8 @@ int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len
             const char* magic = format == AURORA_FMT_YAZ0 ? "Yaz0" : format == AURORA_FMT_YAZ1 ? "Yaz1" : format == AURORA_FMT_YAY0 ? "Yay0"
                                 : format == AURORA_FMT_MIO0 ? "MIO0" : "LZSS";
             if (len < 4) return AURORA_END_OF_STREAM;
-            if (std::memcmp(p, magic, 4) != 0) return AURORA_INVALID_IDENTIFIER;
+            for (int k = 0; k < 4; k++)
+                if (p[k] != uint8_t(magic[k])) return AURORA_INVALID_IDENTIFIER;
             if (len < 8) return AURORA_END_OF_STREAM;
             bool big = true;   // LZSS, and Yay0.cs:45-46 reads BE regardless
             if (format == AURORA_FMT_YAZ0 || format == AURORA_FMT_YAZ1) {
@@ -231,6 +233,19 @@ int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len
     return AURORA_INVALID_ARGUMENT;
 }
 
+__host__ __device__ int decoded_size_one(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size) {
+    if (is_bytelz(format)) {   // LZ4 / LZO / Snappy / PRS do not implement IProvidesDecompressedSize
+        *size = 0;
+        return AURORA_NOT_SUPPORTED;
+    }
+    return core_decoded_size(format, byte_order, p, len, size);
+}
+
+__host__ __device__ int size_scan_status(int status) {
+    // the scan decodes against a zero capacity: a stream that parses to its end reports DST_TOO_SMALL
+    return status == AURORA_DST_TOO_SMALL ? AURORA_OK : status;
+}
+
 // ---- kernel
 namespace {
 
@@ -246,6 +261,20 @@ __global__ void scan_kernel(const uint8_t* image, uint64_t len, uint8_t* match, 
     const uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= len) return;
     match[i] = is_match_one(image + i, len - i, format) > 0;
+}
+
+__global__ void decoded_size_kernel(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint64_t* size,
+                                    int32_t* status, uint32_t n, int format, int byte_order) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint64_t s;
+    status[i] = decoded_size_one(format, byte_order, src_base + src_off[i], src_len[i], &s);
+    size[i] = s;
+}
+
+__global__ void size_scan_status_kernel(int32_t* status, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) status[i] = size_scan_status(status[i]);
 }
 
 // ---- largest-first stream order for batches with a wide size spread: counting sort by floor(log2(size)) ----
@@ -285,6 +314,17 @@ cudaError_t launch_scan(const uint8_t* image, uint64_t len, uint8_t* match, int 
 cudaError_t launch_is_match(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint8_t* match, uint32_t n,
                             int format, cudaStream_t st) {
     is_match_kernel<<<(n + 127) / 128, 128, 0, st>>>(src_base, src_off, src_len, match, n, format);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_decoded_size(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint64_t* size,
+                                int32_t* status, uint32_t n, int format, int byte_order, cudaStream_t st) {
+    decoded_size_kernel<<<(n + 127) / 128, 128, 0, st>>>(src_base, src_off, src_len, size, status, n, format, byte_order);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_size_scan_status(int32_t* status, uint32_t n, cudaStream_t st) {
+    size_scan_status_kernel<<<(n + 255) / 256, 256, 0, st>>>(status, n);
     return cudaGetLastError();
 }
 

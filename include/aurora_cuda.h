@@ -218,12 +218,15 @@ int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* op
 /*
  * ---- device-resident variants (single device, inputs already in HBM; used by bench `value`) ----
  * All pointers are device pointers on `device` (an index into the context's device list);
- * descriptor arrays are device arrays too.  src_off/dst_off must be multiples of 16.
+ * descriptor arrays are device arrays too.  Decode / encode: src_off/dst_off must be multiples of 16.
  * `stream` is a cudaStream_t passed as void* (NULL = the context's own stream for that device);
  * the call is asynchronous with respect to the host: synchronise the stream before reading results.
  * Calls on ONE device must be stream-ordered with each other and with the host-buffer entry points: a device's work
- * counter, size-order array and encoder scratch are per device, not per call, so two batches of the same device may not
- * run concurrently (use one stream per device, or order the streams with events); different devices are independent.
+ * counter, size-order array, encoder scratch and size-scan scratch (the zeroed destination offsets and the `consumed`
+ * array of aurora_decoded_size_batch_device with size_scan != 0) are per device, not per call, so two batches of the same
+ * device may not run concurrently (use one stream per device, or order the streams with events); different devices are
+ * independent.
+ * None of these calls synchronises with the host, reads a result on the host or copies the source to or from the host.
  */
 int aurora_decode_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts,
                                size_t n, const uint8_t* d_src_base, uint64_t src_total,
@@ -237,6 +240,36 @@ int aurora_encode_batch_device(aurora_ctx* ctx, int device, int format, const au
                                const uint64_t* d_src_off, const uint64_t* d_src_len,
                                uint8_t* d_dst_base, const uint64_t* d_dst_off, const uint64_t* d_dst_cap,
                                uint64_t* d_out_len, int32_t* d_status, void* stream);
+
+/*
+ * Device-resident GetDecompressedSize, IsMatch and offset scan: the same per-stream answers as aurora_decoded_size_batch,
+ * aurora_is_match_batch and aurora_scan_offsets for every input, for the formats aurora_decode_batch_device takes (the core
+ * formats and BLZ).  The wrapper formats, unknown ids and the formats the host entry point refuses return
+ * AURORA_INVALID_ARGUMENT with a last error naming the host entry point, and launch nothing.  n == 0 / len == 0: AURORA_OK,
+ * nothing launched.
+ *
+ * aurora_decoded_size_batch_device: d_out_size[i] / d_status[i] as aurora_decoded_size_batch with the same size_scan.  The
+ * flag-LZ formats and BLZ are a header peek (one kernel); the byte-LZ formats (LZ4, LZ4 legacy, LZ4 block, LZO, Snappy,
+ * Snappy block, PRS) report AURORA_NOT_SUPPORTED and size 0, unless size_scan != 0: then the decode kernel parses every
+ * stream in size-only mode (no stores) and a second kernel turns its DST_TOO_SMALL into AURORA_OK; a failing stream keeps
+ * its status and the length it reached.  d_src_base must be 16-byte aligned and, as for aurora_decode_batch_device, the
+ * allocation readable up to the next multiple of 16 of src_total (the size scan stages its input with the same bulk copies).
+ */
+int aurora_decoded_size_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts, size_t n,
+                                     const uint8_t* d_src_base, uint64_t src_total,
+                                     const uint64_t* d_src_off, const uint64_t* d_src_len,
+                                     int size_scan, uint64_t* d_out_size, int32_t* d_status, void* stream);
+
+/* IsMatch of n device streams (one kernel, one thread per stream): d_match[i] as aurora_is_match_batch.  Any alignment;
+ * only [d_src_off[i], d_src_off[i] + d_src_len[i]) is read.  LZ4 block and Snappy block have no IsMatch rule. */
+int aurora_is_match_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts, size_t n,
+                                 const uint8_t* d_src_base, const uint64_t* d_src_off, const uint64_t* d_src_len,
+                                 uint8_t* d_match, void* stream);
+
+/* IsMatch at every byte offset of a device image (one kernel): d_match[i] as aurora_scan_offsets.  Any alignment; len at
+ * most 0xFFFFFFFF00.  The formats aurora_scan_offsets takes: the core formats except LZ4 block, Snappy block and BLZ. */
+int aurora_scan_offsets_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts,
+                               const uint8_t* d_image, uint64_t len, uint8_t* d_match, void* stream);
 
 /* Number of kernels this library has launched since aurora_init (all devices). */
 uint64_t aurora_kernel_launch_count(const aurora_ctx* ctx);
