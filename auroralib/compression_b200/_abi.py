@@ -12,7 +12,8 @@ STATUS_NAMES = ["OK", "END_OF_STREAM", "INVALID_IDENTIFIER", "SIZE_MISMATCH", "D
 # aurora_format
 FMT_YAZ0, FMT_YAZ1, FMT_YAY0, FMT_MIO0, FMT_LZ10, FMT_LZ11, FMT_LZSS, FMT_LZ4, FMT_LZ4_BLOCK, \
     FMT_LZ4_LEGACY, FMT_LZO, FMT_SNAPPY, FMT_SNAPPY_BLOCK, FMT_PRS = range(1, 15)
-# wrapper formats (a header around one of the cores above; host entry points only)
+# wrapper formats (a header around one of the cores above; decode on host buffers and on the device, the other device
+# entry points do not take them)
 FMT_GCLZ, FMT_CXLZ, FMT_COMP, FMT_LZ_3DS, FMT_LZ77, FMT_LEVEL5, FMT_LZON, FMT_LEVEL5_LZSS = range(15, 23)
 FMT_AKLZ, FMT_LZ01, FMT_FCMP, FMT_IECP, FMT_MDB4, FMT_LZSEGA, FMT_GCZ = range(23, 30)   # header + LZSS headerless
 FMT_SDPC = 30   # "SDPC" + size + LZO headerless

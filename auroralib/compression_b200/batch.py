@@ -150,7 +150,10 @@ class BatchCodec:
     # ------------------------------------------------------------------ device-resident (torch CUDA tensors)
     def decode_device(self, fmt, d_src, d_off, d_len, d_dst, d_doff, d_cap, d_out_len, d_consumed, d_status,
                       opts=None, device=0, stream=None):
-        """All arguments are torch CUDA tensors (uint8 / int64 / int32).  Asynchronous on `stream`."""
+        """All arguments are torch CUDA tensors (uint8 / int64 / int32).  Asynchronous on `stream`.
+
+        Every format aurora_decode_batch takes, the wrapper formats included (same results as decode_batch); an LZ77 call
+        reads its chunk count back and so waits for `stream`.  d_src must start 16-byte aligned."""
         opts = opts or _abi.make_opts()
         rc = self._L.aurora_decode_batch_device(
             self._ctx, device, fmt, C.byref(opts), d_off.numel(), d_src.data_ptr(), d_src.numel(), d_off.data_ptr(),
@@ -197,7 +200,9 @@ class BatchCodec:
         The sizes come from decoded_size_device (with a size scan for the byte-LZ formats when size_scan is set).  A stream
         gets the capacity its size names when that is OK and at most `max_size` bytes, else 0, so a forged header cannot
         make this allocate gigabytes: such a stream reports the status of a fixed destination that is too small.  The
-        destination windows are packed at 16-byte aligned offsets.  The one host read is the total, to allocate d_dst."""
+        destination windows are packed at 16-byte aligned offsets.  The one host read is the total, to allocate d_dst.
+        The wrapper formats have no device-side size query, so this raises for them: pass capacities to decode_device
+        (for example from decoded_size_batch on the host)."""
         import torch
         if d_src.data_ptr() % 16:
             raise AuroraError("decode_device_sized: INVALID_ARGUMENT: d_src must start at a 16-byte aligned address "

@@ -19,6 +19,36 @@
 
 using namespace aurora;
 
+namespace aurora {
+
+// resolve the option block into kernel parameters; returns a per-batch status override (OK = run)
+int fill_decode_params(DecodeParams& p, int format, const aurora_codec_opts* o) {
+    p.format = format;
+    p.byte_order = o ? o->byte_order : AURORA_ENDIAN_DEFAULT;
+    if (p.byte_order != AURORA_ENDIAN_LITTLE && p.byte_order != AURORA_ENDIAN_BIG) p.byte_order = AURORA_ENDIAN_DEFAULT;
+    p.size_only = 0;
+    p.lz4_verify = o ? o->lz4_verify : 0;
+    aurora_lz_props lz;
+    if (o && o->lzss.windows_bits != 0) lz = o->lzss;
+    else aurora_lz_props_bits(&lz, 12, 4, 2);   // LZSS.DefaultProperties (LZSS.cs:33)
+    p.lzss = LzssParams{lz.windows_bits, lz.length_bits, lz.min_length, lz.max_distance, lz.windows_start,
+                        o ? o->lzss_initial_fill : 0};
+    if (format == AURORA_FMT_LZSS) {
+        if (lz.windows_bits < 1 || lz.windows_bits > 12 || lz.length_bits < 1 || lz.length_bits > 8 || lz.max_distance < 2 ||
+            lz.max_distance > 4096 || lz.min_length < 1 || lz.min_length > 255)
+            return AURORA_NOT_SUPPORTED;
+    }
+    return AURORA_OK;
+}
+
+cudaError_t launch_decode(const DecodeParams& p, int sm_count, cudaStream_t st) {
+    if (p.format == AURORA_FMT_BLZ) return launch_decode_blz(p, sm_count, st);
+    if (is_flaglz(p.format)) return launch_decode_flaglz(p, sm_count, st);
+    return launch_decode_bytelz(p, sm_count, st);
+}
+
+}  // namespace aurora
+
 namespace {
 
 // NVTX ranges of the host scheduler (SURVEY.md §5 "tracing"): one range per device shard and, inside it, one per pipeline
@@ -36,26 +66,6 @@ struct NvtxRange {
     NvtxRange& operator=(const NvtxRange&) = delete;
 };
 
-
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = n + n / 8 + 4096;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
 
 struct HostBuf {
     void* p = nullptr;
@@ -85,6 +95,7 @@ struct DeviceCtx {
     std::vector<cudaEvent_t> ev_in, ev_k;
     DevBuf src, dst, desc, ticket, scratch, order;
     DevBuf size_scan;   // aurora_decoded_size_batch_device with a size scan: n zeroed offsets / capacities, then n consumed
+    WrapScratch wrap;   // aurora_decode_batch_device of the wrapper formats
     HostBuf hdesc;
     std::mutex mu;   // one batch at a time per device
 };
@@ -115,15 +126,9 @@ thread_local std::string g_init_error;
         }                                                                                           \
     } while (0)
 
-bool is_flaglz(int f) {
-    return f == AURORA_FMT_YAZ0 || f == AURORA_FMT_YAZ1 || f == AURORA_FMT_YAY0 || f == AURORA_FMT_MIO0 ||
-           f == AURORA_FMT_LZ10 || f == AURORA_FMT_LZ11 || f == AURORA_FMT_LZSS || f == AURORA_FMT_LZHUDSON ||
-           f == AURORA_FMT_LZ40 || f == AURORA_FMT_LZ60 || f == AURORA_FMT_SMSR00;
-}
-
 // The formats each query takes, one predicate per query for its host and its device entry point.  The host entry points
-// also take the wrapper formats (their headers are resolved on the host); the device entry points take exactly the formats
-// aurora_decode_batch_device decodes.
+// also take the wrapper formats (their headers are resolved on the host); the device entry points take the core formats and
+// BLZ (aurora_decode_batch_device also decodes the wrapper formats, which bring their own capacities).
 bool size_query_format(int f) { return is_flaglz(f) || is_bytelz(f) || f == AURORA_FMT_BLZ; }
 // every IsMatch rule rejects an empty stream without reading it, so this asks only whether is_match_one has a rule
 bool is_match_query_format(int f) { return aurora::is_match_one(nullptr, 0, f) >= 0; }
@@ -133,26 +138,6 @@ int ceil_log2(long long x) {
     int b = 0;
     while ((1LL << b) < x) b++;
     return b;
-}
-
-// resolve the option block into kernel parameters; returns a per-batch status override (OK = run)
-int fill_decode_params(DecodeParams& p, int format, const aurora_codec_opts* o) {
-    p.format = format;
-    p.byte_order = o ? o->byte_order : AURORA_ENDIAN_DEFAULT;
-    if (p.byte_order != AURORA_ENDIAN_LITTLE && p.byte_order != AURORA_ENDIAN_BIG) p.byte_order = AURORA_ENDIAN_DEFAULT;
-    p.size_only = 0;
-    p.lz4_verify = o ? o->lz4_verify : 0;
-    aurora_lz_props lz;
-    if (o && o->lzss.windows_bits != 0) lz = o->lzss;
-    else aurora_lz_props_bits(&lz, 12, 4, 2);   // LZSS.DefaultProperties (LZSS.cs:33)
-    p.lzss = LzssParams{lz.windows_bits, lz.length_bits, lz.min_length, lz.max_distance, lz.windows_start,
-                        o ? o->lzss_initial_fill : 0};
-    if (format == AURORA_FMT_LZSS) {
-        if (lz.windows_bits < 1 || lz.windows_bits > 12 || lz.length_bits < 1 || lz.length_bits > 8 || lz.max_distance < 2 ||
-            lz.max_distance > 4096 || lz.min_length < 1 || lz.min_length > 255)
-            return AURORA_NOT_SUPPORTED;
-    }
-    return AURORA_OK;
 }
 
 cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
@@ -173,12 +158,6 @@ cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
     if (encode_lz_par_supported(p) && (want == 1 || (want == 0 && par_default))) return launch_encode_lz_par(p, warps / 48, st);
     if (is_flaglz(p.format) || p.format == AURORA_FMT_BLZ) return launch_encode_lz(p, warps, st);   // BLZ: LZ10's layout
     return launch_encode_bytelz(p, warps, st);
-}
-
-cudaError_t launch_decode(const DecodeParams& p, int sm_count, cudaStream_t st) {
-    if (p.format == AURORA_FMT_BLZ) return launch_decode_blz(p, sm_count, st);
-    if (is_flaglz(p.format)) return launch_decode_flaglz(p, sm_count, st);
-    return launch_decode_bytelz(p, sm_count, st);
 }
 
 struct Range {
@@ -745,6 +724,7 @@ void aurora_shutdown(aurora_ctx* ctx) {
         d->scratch.release();
         d->order.release();
         d->size_scan.release();
+        d->wrap.release();
         d->hdesc.release();
         for (cudaEvent_t e : d->ev_in) cudaEventDestroy(e);
         for (cudaEvent_t e : d->ev_k) cudaEventDestroy(e);
@@ -934,7 +914,8 @@ int aurora_decode_batch_device(aurora_ctx* ctx, int device, int format, const au
                                void* stream) {
     if (!ctx || device < 0 || device >= int(ctx->devs.size())) return AURORA_INVALID_ARGUMENT;
     if (n == 0) return AURORA_OK;
-    if (!(is_flaglz(format) || is_bytelz(format) || format == AURORA_FMT_BLZ) || n > 0xFFFFFFF0ull) return AURORA_INVALID_ARGUMENT;
+    const bool wrapper = aurora::is_wrapper_format(format);
+    if (!(is_flaglz(format) || is_bytelz(format) || format == AURORA_FMT_BLZ || wrapper) || n > 0xFFFFFFF0ull) return AURORA_INVALID_ARGUMENT;
     if ((reinterpret_cast<uintptr_t>(d_src_base) & 15) != 0) {
         ctx->set_error("aurora_decode_batch_device: d_src_base must be 16-byte aligned");
         return AURORA_INVALID_ARGUMENT;
@@ -942,6 +923,17 @@ int aurora_decode_batch_device(aurora_ctx* ctx, int device, int format, const au
     DeviceCtx* d = ctx->devs[device];
     std::lock_guard<std::mutex> guard(d->mu);
     CU_TRY(ctx, cudaSetDevice(d->dev));
+    if (wrapper) {   // the header pass, the core launches and the merge pass of wrappers.cu (opts.balance is not applied)
+        cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+        CU_TRY(ctx, d->ticket.reserve(256));
+        uint64_t launched = 0;
+        const cudaError_t e = aurora::wrapped_decode_batch_device(format, opts, n, d_src_base, src_total, d_src_off, d_src_len, d_dst_base,
+                                                                  d_dst_off, d_dst_cap, d_out_len, d_consumed, d_status, d->wrap,
+                                                                  static_cast<unsigned int*>(d->ticket.p), d->sm_count, st, &launched);
+        ctx->launches += launched;
+        CU_TRY(ctx, e);
+        return AURORA_OK;
+    }
     DecodeParams P{};
     if (fill_decode_params(P, format, opts) != AURORA_OK) {
         ctx->set_error("aurora_decode_batch_device: unsupported LZSS properties");

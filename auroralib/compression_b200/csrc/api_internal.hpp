@@ -24,15 +24,20 @@ int encode_core_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* opts
 // IsMatch and GetDecompressedSize rules of the core formats (ismatch.cu), the one copy of each.
 // is_match_one: 1 match, 0 no match, -1 no rule for this format.  It also runs in the IsMatch and offset-scan kernels.
 __host__ __device__ int is_match_one(const uint8_t* p, uint64_t len, int format);
-// core_decoded_size: the header peek of BLZ and the flag-LZ formats.  A status; *size is 0 unless it is AURORA_OK.
-// AURORA_INVALID_ARGUMENT for a format without a size header.
-__host__ __device__ int core_decoded_size(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size);
+// (core_decoded_size, the header peek of BLZ and the flag-LZ formats: size_peek.cuh)
 // decoded_size_one: GetDecompressedSize of one stream of a core format without a size scan — AURORA_NOT_SUPPORTED and size 0
 // for the byte-LZ formats, the header peek for the others.  Both aurora_decoded_size_batch and the device's
 // decoded_size_kernel call it.
 __host__ __device__ int decoded_size_one(int format, int byte_order, const uint8_t* p, uint64_t len, uint64_t* size);
 // size_scan_status: the status a size scan reports for a stream, from the status of its size-only decode (capacity 0).
 __host__ __device__ int size_scan_status(int status);
+
+// the flag-LZ formats (decode_flaglz.cu)
+inline bool is_flaglz(int f) {
+    return f == AURORA_FMT_YAZ0 || f == AURORA_FMT_YAZ1 || f == AURORA_FMT_YAY0 || f == AURORA_FMT_MIO0 ||
+           f == AURORA_FMT_LZ10 || f == AURORA_FMT_LZ11 || f == AURORA_FMT_LZSS || f == AURORA_FMT_LZHUDSON ||
+           f == AURORA_FMT_LZ40 || f == AURORA_FMT_LZ60 || f == AURORA_FMT_SMSR00;
+}
 
 // the byte-LZ formats: LZ4, LZ4 block, LZ4 legacy, LZO, Snappy, Snappy block, PRS (no size header; decode_bytelz.cu)
 __host__ __device__ inline bool is_bytelz(int f) {

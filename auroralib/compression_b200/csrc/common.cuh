@@ -64,6 +64,50 @@ struct EncodeParams {
     uint64_t scratch_per_warp;
 };
 
+#ifdef __CUDACC__   // (not in the CPU builds of the kernel sources under tests/simt)
+// a device allocation that grows (never shrinks) to the largest request; cudaFree of the old block synchronises the device
+struct DevBuf {
+    void* p = nullptr;
+    size_t cap = 0;
+    cudaError_t reserve(size_t n) {
+        if (n <= cap) return cudaSuccess;
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+        size_t want = n + n / 8 + 4096;
+        cudaError_t e = cudaMalloc(&p, want);
+        if (e == cudaSuccess) cap = want;
+        return e;
+    }
+    void release() {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+};
+
+// per-device scratch of aurora_decode_batch_device for the wrapper formats (wrappers.cu): per-stream plans and sub-streams
+// (+ LZ77's chunk counts and scan), the core launches' descriptors and results, LZ00's copy of the source
+struct WrapScratch {
+    DevBuf plans, slots, src;
+    void release() {
+        plans.release();
+        slots.release();
+        src.release();
+    }
+};
+// the wrapper pipeline on the caller's device arrays; counts its kernel launches into *launches
+cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opts, size_t n, const uint8_t* d_src_base, uint64_t src_total,
+                                        const uint64_t* d_src_off, const uint64_t* d_src_len, uint8_t* d_dst_base,
+                                        const uint64_t* d_dst_off, const uint64_t* d_dst_cap, uint64_t* d_out_len,
+                                        uint64_t* d_consumed, int32_t* d_status, WrapScratch& scr, unsigned int* ticket, int sm_count,
+                                        cudaStream_t st, uint64_t* launches);
+#endif
+
+// api.cu: the option block resolved into kernel parameters (returns a per-batch status override, OK = run), and the decode
+// kernel of p.format
+int fill_decode_params(DecodeParams& p, int format, const aurora_codec_opts* o);
+cudaError_t launch_decode(const DecodeParams& p, int sm_count, cudaStream_t st);
 // kernel launchers (one translation unit per kernel family); all return cudaGetLastError()
 cudaError_t launch_decode_flaglz(const DecodeParams& p, int sm_count, cudaStream_t st);
 cudaError_t launch_decode_bytelz(const DecodeParams& p, int sm_count, cudaStream_t st);

@@ -61,7 +61,8 @@ typedef enum aurora_format {
     AURORA_FMT_SNAPPY_BLOCK = 13, /* Snappy.DecompressHeaderless / CompressHeaderless        */
     AURORA_FMT_PRS          = 14, /* Sega/PRS.cs                                             */
     /* wrapper formats: a header around one of the cores above (SURVEY.md 8f item 2; paths under
-     * src/AuroraLib.Compression.Nintendo).  Host entry points only (the headers are resolved on the host). */
+     * src/AuroraLib.Compression.Nintendo).  aurora_decode_batch resolves the headers on the host,
+     * aurora_decode_batch_device on the device; the other device entry points do not take them. */
     AURORA_FMT_GCLZ         = 15, /* Nintendo/GCLZ.cs: "GCLZ" + LZ10                         */
     AURORA_FMT_CXLZ         = 16, /* Sega/CXLZ.cs: "CXLZ" + LZ10                             */
     AURORA_FMT_COMP         = 17, /* Sega/COMP.cs: "COMP" + LZ11                             */
@@ -226,7 +227,26 @@ int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* op
  * array of aurora_decoded_size_batch_device with size_scan != 0) are per device, not per call, so two batches of the same
  * device may not run concurrently (use one stream per device, or order the streams with events); different devices are
  * independent.
- * None of these calls synchronises with the host, reads a result on the host or copies the source to or from the host.
+ * The wrapper formats (15-32) add per-device scratch of their own: per-stream plans and sub-stream descriptors and results,
+ * LZ77's chunk counts, and LZ00's copy of the source.
+ * None of these calls synchronises with the host, reads a result on the host or copies the source to or from the host,
+ * with one exception: aurora_decode_batch_device of LZ77 (below).
+ *
+ * aurora_decode_batch_device of the wrapper formats: out_len, consumed, status and the decoded bytes in
+ * [dst_off[i], dst_off[i] + min(out_len[i], dst_cap[i])) are those aurora_decode_batch gives for the same streams, options
+ * and capacities; nothing outside the destination windows is written, and the caller's source is never modified (LZ00's
+ * keystream is lifted from a device-to-device copy of [0, src_total) in scratch).  Same argument rules as the core formats
+ * (16-byte aligned d_src_base, offsets multiples of 16); the sub-streams behind the headers start at any offset.  One
+ * thread per stream resolves the header, the core kernels run on the sub-streams, one thread per stream merges the
+ * results.  Kernel launches per call: 3 (header pass, core, merge) for GCLZ, CXLZ, COMP, 3DS-LZ, LZOn, SDPC, Level5LZSS and
+ * the LZSS-property family; 4 for Level5 and ECD (+ a warp-per-stream copy of stored payloads / ECD's plain prefix) and
+ * for LZ00 (+ the keystream pass); 9 for LZ77 (header pass, a two-kernel exclusive scan of the ChunkLZ10 chunk counts,
+ * chunk fill, LZ10 over stream and chunk slots, LZ11 over the stream slots, redo selection, a redo LZ10 launch that decodes
+ * a file's failing chunk once more so that its bytes win as in the reference's sequential loop, merge).  LZ77 READS ONE
+ * VALUE BACK: the batch's total chunk count (a chunk table may be as long as its stream, so only the device knows how many
+ * descriptors the chunks need); that call returns after the stream has run its header pass.  opts.balance is not applied
+ * to the wrapper formats.  aurora_decoded_size_batch_device / aurora_is_match_batch_device / aurora_scan_offsets_device do
+ * not take the wrapper formats: a wrapper caller passes its own capacities (e.g. from aurora_decoded_size_batch).
  */
 int aurora_decode_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts,
                                size_t n, const uint8_t* d_src_base, uint64_t src_total,
