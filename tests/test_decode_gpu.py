@@ -135,9 +135,10 @@ def test_lzss_properties(codec, oracle, props):
 
 @pytest.mark.parametrize("fmt", [A.FMT_LZ11, A.FMT_LZ40, A.FMT_LZ60], ids=fmt_id)
 def test_lz11_long_matches(codec, oracle, fmt):
-    """LZ11 matches of up to 65 808 bytes (LZ11.cs:106-112, 4-byte tokens; LZ40 / LZ60: up to 65 807, LZ40.cs:103-113, and
-    a period of 4096 is encoded as distance 0): long constant / periodic runs between literal-heavy stretches, valid,
-    truncated and with short destinations — the group-per-lane core's long-group path."""
+    """Long constant / periodic runs between literal-heavy stretches, encoded by the reference encoder: valid, truncated and
+    with short destinations — the group-per-lane core's long-group path.  The encoder's LzProperties(0x1000, 0x4000, 3) cap a
+    match at 16 384 bytes, so these streams never carry a 4-byte token longer than that; tests/test_token_streams_gpu.py
+    writes the full range (up to 65 808 bytes for LZ11, 65 807 for LZ40 / LZ60, LZ11.cs:106-112, LZ40.cs:103-113)."""
     rng = np.random.default_rng(4111 + fmt)
     raws = []
     for i in range(48):

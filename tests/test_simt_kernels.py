@@ -287,7 +287,8 @@ def simt_bytelz_dec():
     return f
 
 
-def simt_decode_bytelz(entry, fmt, comps, caps, byte_order=A.ENDIAN_DEFAULT, lz4_verify=0, flag_lz=False, lzss=None, size_only=0):
+def simt_decode_bytelz(entry, fmt, comps, caps, byte_order=A.ENDIAN_DEFAULT, lz4_verify=0, flag_lz=False, lzss=None, size_only=0,
+                       initial_fill=0):
     """One emulated warp (byte-LZ kernel) or parser / resolver warp pair (flag_lz: the flag-LZ kernel) decodes `comps`."""
     n = len(comps)
     off, pos = [], 7
@@ -312,7 +313,7 @@ def simt_decode_bytelz(entry, fmt, comps, caps, byte_order=A.ENDIAN_DEFAULT, lz4
     p = lambda a: a.ctypes.data_as(C.c_void_p)
     if flag_lz:
         lz = lzss if lzss is not None else A.lz_props_bits(12, 4, 2)   # LZSS.DefaultProperties (api.cu fill_decode_params)
-        head = (C.c_int(fmt), C.c_int(byte_order), C.c_int(0), (C.c_int * 6)(lz.windows_bits, lz.length_bits, lz.min_length, lz.max_distance, lz.windows_start, 0))
+        head = (C.c_int(fmt), C.c_int(byte_order), C.c_int(0), (C.c_int * 6)(lz.windows_bits, lz.length_bits, lz.min_length, lz.max_distance, lz.windows_start, initial_fill))
     else:
         head = (C.c_int(fmt), C.c_int(byte_order), C.c_int(lz4_verify), C.c_int(size_only))
     rc = entry(*head, p(src), C.c_uint64(limit), p(src_off), p(src_len), p(dst), p(dst_off), p(dst_cap), p(out_len), p(consumed), p(status),
