@@ -1096,11 +1096,16 @@ int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* op
     const int rc = aurora::encode_core_batch(ctx, format, opts, n, src_base, src_off, src_len, dst_base, dst_off, dst_cap, out_len, status);
     if (rc == AURORA_OK && format == AURORA_FMT_BLZ) {
         // BLZ.Compress (BLZ.cs:78-92): behind the codes 0xFF padding to a multiple of 16, then the footer — u24 LE total size,
-        // u8 footer-and-padding size, i32 LE (decoded size - total size)
+        // u8 footer-and-padding size, i32 LE (decoded size - total size).  A stream that does not fit reports the whole size
+        // too, as every other format does, so that a caller can retry with exactly that capacity.
         for (size_t i = 0; i < n; i++) {
-            if (status[i] != AURORA_OK) continue;
+            if (status[i] != AURORA_OK && status[i] != AURORA_DST_TOO_SMALL) continue;
             const uint64_t total0 = out_len[i] + 8, padding = (16 - total0 % 16) % 16, total = total0 + padding;
-            if (total > dst_cap[i]) { status[i] = AURORA_DST_TOO_SMALL; continue; }
+            if (status[i] != AURORA_OK || total > dst_cap[i]) {
+                status[i] = AURORA_DST_TOO_SMALL;
+                out_len[i] = total;
+                continue;
+            }
             uint8_t* d = dst_base + dst_off[i] + out_len[i];
             std::memset(d, 0xFF, size_t(padding));
             d += padding;

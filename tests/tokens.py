@@ -30,17 +30,19 @@ CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
 
 def _constants(name):
     """`#define AURORA_X n` and `constexpr int kX = <expr>;` of a kernel file, evaluated in order (expressions that name
-    template parameters are skipped)."""
+    template parameters are skipped).  `constexpr int kA = 1, kB = kA - 1;` declares both."""
     src = re.sub(r"//[^\n]*", "", open(os.path.join(CSRC, name)).read())
     env = {}
-    for m in re.finditer(r"#define (AURORA_\w+) (\d+)\b|constexpr int (k\w+) = ([^;]+);", src):
+    for m in re.finditer(r"#define (AURORA_\w+) (\d+)\b|constexpr int (k\w+ = [^;]+);", src):
         if m.group(1):
             env.setdefault(m.group(1), int(m.group(2)))
             continue
-        try:
-            env.setdefault(m.group(3), int(eval(m.group(4), {"__builtins__": {}}, dict(env))))
-        except Exception:
-            pass
+        for decl in re.split(r",\s*(?=k\w+ = )", m.group(3)):
+            name, expr = decl.split(" = ", 1)
+            try:
+                env.setdefault(name, int(eval(expr, {"__builtins__": {}}, dict(env))))
+            except Exception:
+                pass
     return env
 
 
