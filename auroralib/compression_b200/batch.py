@@ -163,6 +163,11 @@ class BatchCodec:
 
     def encode_device(self, fmt, d_src, d_off, d_len, d_dst, d_doff, d_cap, d_out_len, d_status, opts=None, device=0,
                       stream=None):
+        """All arguments are torch CUDA tensors (uint8 / int64 / int32).  Asynchronous on `stream`.
+
+        Every format encode_batch takes except BLZ, the wrapper formats included (same statuses, lengths and bytes as
+        encode_batch / encode_packed with the same capacities); LZ77 with lz77_type 0xF7 (ChunkLZ10) reads its chunk count
+        back and so waits for `stream`.  The source is never modified."""
         opts = opts or _abi.make_opts()
         rc = self._L.aurora_encode_batch_device(
             self._ctx, device, fmt, C.byref(opts), d_off.numel(), d_src.data_ptr(), d_src.numel(), d_off.data_ptr(),

@@ -128,7 +128,8 @@ thread_local std::string g_init_error;
 
 // The formats each query takes, one predicate per query for its host and its device entry point.  The host entry points
 // also take the wrapper formats (their headers are resolved on the host); the device entry points take the core formats and
-// BLZ (aurora_decode_batch_device also decodes the wrapper formats, which bring their own capacities).
+// BLZ (aurora_decode_batch_device and aurora_encode_batch_device also take the wrapper formats, whose callers bring their own
+// capacities).
 bool size_query_format(int f) { return is_flaglz(f) || is_bytelz(f) || f == AURORA_FMT_BLZ; }
 // every IsMatch rule rejects an empty stream without reading it, so this asks only whether is_match_one has a rule
 bool is_match_query_format(int f) { return aurora::is_match_one(nullptr, 0, f) >= 0; }
@@ -139,6 +140,10 @@ int ceil_log2(long long x) {
     while ((1LL << b) < x) b++;
     return b;
 }
+
+}  // namespace
+
+namespace aurora {
 
 cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
     // Flag-byte formats (LZ10 / BLZ, LZ11 / LZ40 / LZ60, Yaz0 / Yaz1, LZSS, MIO0, Yay0, LZHudson, SMSR00): the window search with one lane per
@@ -159,6 +164,10 @@ cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
     if (is_flaglz(p.format) || p.format == AURORA_FMT_BLZ) return launch_encode_lz(p, warps, st);   // BLZ: LZ10's layout
     return launch_encode_bytelz(p, warps, st);
 }
+
+}  // namespace aurora
+
+namespace {
 
 struct Range {
     size_t begin, end;
@@ -506,6 +515,10 @@ int isqrt2q(int q) {
     return r;
 }
 
+}  // namespace
+
+namespace aurora {
+
 int fill_encode_params(EncodeParams& p, int format, const aurora_codec_opts* o) {
     int q = (o && o->quality >= 0) ? o->quality : 8;   // default(CompressionSettings) == Balanced
     if (q > 15) return AURORA_INVALID_ARGUMENT;
@@ -572,6 +585,10 @@ int fill_encode_params(EncodeParams& p, int format, const aurora_codec_opts* o) 
     p.lzss = LzssParams{lz.windows_bits, lz.length_bits, lz.min_length, lz.max_distance, lz.windows_start, 0};
     return AURORA_OK;
 }
+
+}  // namespace aurora
+
+namespace {
 
 int encode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_opts* opts, size_t b, size_t e,
                  const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint8_t* dst_base,
@@ -1069,17 +1086,7 @@ extern "C" {
 
 uint64_t aurora_encode_bound(int format, uint64_t raw_len) {
     if (aurora::is_wrapper_format(format)) return aurora::wrapped_encode_bound(format, raw_len, nullptr);
-    // worst case of every token writer on the hot path: all literals + flag bits + headers / chunk framing
-    switch (format) {
-        case AURORA_FMT_LZ4:
-        case AURORA_FMT_LZ4_LEGACY:
-        case AURORA_FMT_LZ4_BLOCK: return raw_len + raw_len / 255 + 64 + 8 * (raw_len / 0x400000 + 1);
-        case AURORA_FMT_SNAPPY:
-        case AURORA_FMT_SNAPPY_BLOCK: return raw_len + raw_len / 60 + 32 + 16 * (raw_len / 0x10000 + 1);
-        // LZO: a far 3-byte match costs 3 bytes and splits the literal run around it (4 literals + 1 match = 7 bytes in, 8 out)
-        case AURORA_FMT_LZO: return raw_len + raw_len / 6 + 64;
-        default: return raw_len + raw_len / 8 + 64;
-    }
+    return aurora::core_encode_bound(format, raw_len);
 }
 
 int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* opts, size_t n, const uint8_t* src_base,
@@ -1166,6 +1173,22 @@ int aurora_encode_batch_device(aurora_ctx* ctx, int device, int format, const au
     DeviceCtx* d = ctx->devs[device];
     std::lock_guard<std::mutex> guard(d->mu);
     CU_TRY(ctx, cudaSetDevice(d->dev));
+    if (aurora::is_wrapper_format(format)) {   // the plan pass, one core encoder launch and the finish pass of wrappers.cu
+        cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+        CU_TRY(ctx, d->ticket.reserve(256));
+        uint64_t launched = 0;
+        cudaError_t e = cudaSuccess;
+        const int rc = aurora::wrapped_encode_batch_device(format, opts, n, d_src_base, src_total, d_src_off, d_src_len, d_dst_base,
+                                                           d_dst_off, d_dst_cap, d_out_len, d_status, d->wrap, d->scratch,
+                                                           static_cast<unsigned int*>(d->ticket.p), d->sm_count, st, &launched, &e);
+        ctx->launches += launched;
+        CU_TRY(ctx, e);
+        if (rc != AURORA_OK) {
+            ctx->set_error("aurora_encode_batch_device: invalid settings");
+            return rc;
+        }
+        return AURORA_OK;
+    }
     EncodeParams P{};
     const int rc = format == AURORA_FMT_BLZ ? AURORA_NOT_SUPPORTED   // needs the reversal passes and the host-written footer
                                              : fill_encode_params(P, format, opts);

@@ -64,6 +64,21 @@ struct EncodeParams {
     uint64_t scratch_per_warp;
 };
 
+// aurora_encode_bound of the core formats: the worst case of every token writer on the hot path, all literals + flag bits +
+// headers / chunk framing (also the chunk slots of a ChunkLZ10 encode, wrappers.cu)
+__host__ __device__ inline uint64_t core_encode_bound(int format, uint64_t raw_len) {
+    switch (format) {
+        case AURORA_FMT_LZ4:
+        case AURORA_FMT_LZ4_LEGACY:
+        case AURORA_FMT_LZ4_BLOCK: return raw_len + raw_len / 255 + 64 + 8 * (raw_len / 0x400000 + 1);
+        case AURORA_FMT_SNAPPY:
+        case AURORA_FMT_SNAPPY_BLOCK: return raw_len + raw_len / 60 + 32 + 16 * (raw_len / 0x10000 + 1);
+        // LZO: a far 3-byte match costs 3 bytes and splits the literal run around it (4 literals + 1 match = 7 bytes in, 8 out)
+        case AURORA_FMT_LZO: return raw_len + raw_len / 6 + 64;
+        default: return raw_len + raw_len / 8 + 64;
+    }
+}
+
 #ifdef __CUDACC__   // (not in the CPU builds of the kernel sources under tests/simt)
 // a device allocation that grows (never shrinks) to the largest request; cudaFree of the old block synchronises the device
 struct DevBuf {
@@ -86,8 +101,9 @@ struct DevBuf {
     }
 };
 
-// per-device scratch of aurora_decode_batch_device for the wrapper formats (wrappers.cu): per-stream plans and sub-streams
-// (+ LZ77's chunk counts and scan), the core launches' descriptors and results, LZ00's copy of the source
+// per-device scratch of aurora_decode_batch_device / aurora_encode_batch_device for the wrapper formats (wrappers.cu):
+// per-stream plans and sub-streams (+ LZ77's chunk counts and scan), the core launches' descriptors and results, LZ00's copy
+// of the source (decode)
 struct WrapScratch {
     DevBuf plans, slots, src;
     void release() {
@@ -102,12 +118,23 @@ cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opt
                                         const uint64_t* d_dst_off, const uint64_t* d_dst_cap, uint64_t* d_out_len,
                                         uint64_t* d_consumed, int32_t* d_status, WrapScratch& scr, unsigned int* ticket, int sm_count,
                                         cudaStream_t st, uint64_t* launches);
+// the wrapper encode pipeline on the caller's device arrays (enc_scratch: the core encoder's per-warp tables); returns
+// AURORA_OK, AURORA_INVALID_ARGUMENT (settings) or AURORA_CUDA_ERROR with *err set; counts its kernel launches into *launches
+int wrapped_encode_batch_device(int format, const aurora_codec_opts* opts, size_t n, const uint8_t* d_src_base, uint64_t src_total,
+                                const uint64_t* d_src_off, const uint64_t* d_src_len, uint8_t* d_dst_base, const uint64_t* d_dst_off,
+                                const uint64_t* d_dst_cap, uint64_t* d_out_len, int32_t* d_status, WrapScratch& scr,
+                                DevBuf& enc_scratch, unsigned int* ticket, int sm_count, cudaStream_t st, uint64_t* launches,
+                                cudaError_t* err);
 #endif
 
 // api.cu: the option block resolved into kernel parameters (returns a per-batch status override, OK = run), and the decode
 // kernel of p.format
 int fill_decode_params(DecodeParams& p, int format, const aurora_codec_opts* o);
 cudaError_t launch_decode(const DecodeParams& p, int sm_count, cudaStream_t st);
+// the same for the encoders: CompressionSettings + LzProperties -> finder parameters (AURORA_OK, or the batch's argument
+// error), and the encode kernel of p.format (the lane-per-position finder or the sequential replay)
+int fill_encode_params(EncodeParams& p, int format, const aurora_codec_opts* o);
+cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st);
 // kernel launchers (one translation unit per kernel family); all return cudaGetLastError()
 cudaError_t launch_decode_flaglz(const DecodeParams& p, int sm_count, cudaStream_t st);
 cudaError_t launch_decode_bytelz(const DecodeParams& p, int sm_count, cudaStream_t st);

@@ -3,7 +3,9 @@
 // on the device exactly like a direct call.  The header rule (wrap_resolve, wrap_chunk), the merge of the core results
 // (wrap_merge) and the ChunkLZ10 redo selection (wrap_redo_chunk) are written once, above the "// ---- kernel" line, and are
 // __host__ __device__: aurora_decode_batch resolves the headers on the host, aurora_decode_batch_device in
-// wrap_resolve_kernel, one thread per stream.
+// wrap_resolve_kernel, one thread per stream.  The encode rules (wrap_encode_plan: a stream's core pieces; wrap_encode_finish:
+// its status, header and the copies / moves around the core output) sit there too: aurora_encode_batch applies them on the
+// host, aurora_encode_batch_device in wrap_enc_plan_kernel and wrap_enc_finish_kernel.
 //
 // Reference semantics restated (paths under /root/reference/src/AuroraLib.Compression.Nintendo):
 //   Nintendo/GCLZ.cs:39-53, Sega/CXLZ.cs:41-55, Nintendo/3DS-LZ.cs:37-50   magic + LZ10.Decompress / Compress
@@ -42,7 +44,7 @@ __host__ __device__ inline const char* lzon_magic() { return "LZOn\0\x2F\xF1\x71
 
 constexpr uint64_t kParseHeader = ~0ull;   // raw size "none": the core parses its own header
 
-// LZSS-property family: identifier, header bytes that are READ (a short stream is END_OF_STREAM), bytes skipped by a seek
+// LZSS-property family: identifier (nullptr: none), header bytes that are READ (a short stream is END_OF_STREAM), bytes skipped by a seek
 // after them, where the decoded size sits, and which LzProperties the body uses.  A switch rather than a table: device code
 // cannot read a host array.
 struct Family {
@@ -58,8 +60,8 @@ __host__ __device__ inline bool family_of(int format, Family& f) {
         case AURORA_FMT_FCMP: f = Family{format, "FCMP", 4, 12, 0, 4, false, true}; return true;
         case AURORA_FMT_IECP: f = Family{format, "IECP", 4, 8, 0, 4, false, true}; return true;
         case AURORA_FMT_MDB4: f = Family{format, "MDB4", 4, 16, 16, 8, false, false}; return true;
-        case AURORA_FMT_LZSEGA: f = Family{format, "", 0, 8, 0, 4, false, false}; return true;
-        case AURORA_FMT_GCZ: f = Family{format, "", 0, 4, 0, 0, false, true}; return true;
+        case AURORA_FMT_LZSEGA: f = Family{format, nullptr, 0, 8, 0, 4, false, false}; return true;
+        case AURORA_FMT_GCZ: f = Family{format, nullptr, 0, 4, 0, 0, false, true}; return true;
         // LZ00.cs:56-63: magic, length, 8 skipped (a seek), 32-byte name, size, key are READ up to byte 56; 8 more are skipped
         case AURORA_FMT_LZ00: f = Family{format, "LZ00", 4, 56, 8, 48, false, true}; return true;
     }
@@ -302,6 +304,334 @@ __host__ __device__ inline int64_t wrap_redo_chunk(const WrapPlan& pl, const int
     return -1;
 }
 
+// ---- encode rules: the core encoder writes at an offset the wrapper header leaves free, then the header is written (or the
+// core's own header is rewritten in place).  aurora_encode_batch applies them on the host, aurora_encode_batch_device in
+// wrap_enc_plan_kernel (one thread per stream) and wrap_enc_finish_kernel (one warp per stream).
+
+__host__ __device__ inline void put_le32(uint8_t* p, uint32_t v) { p[0] = uint8_t(v); p[1] = uint8_t(v >> 8); p[2] = uint8_t(v >> 16); p[3] = uint8_t(v >> 24); }
+__host__ __device__ inline void put_be32(uint8_t* p, uint32_t v) { p[3] = uint8_t(v); p[2] = uint8_t(v >> 8); p[1] = uint8_t(v >> 16); p[0] = uint8_t(v >> 24); }
+__host__ __device__ inline void put_bytes(uint8_t* p, const char* s, uint64_t k) {
+    for (uint64_t j = 0; j < k; j++) p[j] = uint8_t(s[j]);
+}
+// identifiers as little-endian words, folded at compile time (a string literal in device code would be one more global object)
+__host__ __device__ constexpr uint32_t le_word(const char* s) {
+    return uint32_t(uint8_t(s[0])) | (uint32_t(uint8_t(s[1])) << 8) | (uint32_t(uint8_t(s[2])) << 16) | (uint32_t(uint8_t(s[3])) << 24);
+}
+constexpr uint32_t kIdGCLZ = le_word("GCLZ"), kIdCXLZ = le_word("CXLZ"), kIdCOMP = le_word("COMP"), kId3DS0 = le_word("3DS-"),
+                   kId3DS1 = le_word("LZ\r\n"), kIdLZ77 = le_word("LZ77"), kIdSDPC = le_word("SDPC"), kIdSSZL = le_word("SSZL"),
+                   kIdECD = le_word("ECD\0"), kIdTemp0 = le_word("Temp"), kIdTemp1 = le_word(".dat");
+
+// the options of a wrapped encode, resolved once per batch
+struct WrapEnc {
+    int format;
+    int status;            // OK, or the status of every stream: NOT_SUPPORTED for an LZ77 / Level5 sub-type without an encoder
+    int core;              // AURORA_FMT_LZ10 / LZ11 / LZSS / LZO
+    uint64_t head;         // bytes in front of the core's output
+    uint32_t lz77_type, level5_type, lz00_key;
+    uint64_t chunk;        // LZ77.ChunkSize
+    uint64_t ecd_plain;    // ECD.PlainSize
+    bool quality0;         // quality 0: Level5 and ECD store
+};
+
+// false: not a wrapper format.  The extension fields of the option block count only when the caller's block has them.
+inline bool wrap_encode_opts(int format, const aurora_codec_opts& o, WrapEnc& e) {
+    const bool has_ext = o.struct_size >= sizeof(aurora_codec_opts);
+    e.format = format;
+    e.status = AURORA_OK;
+    e.core = AURORA_FMT_LZ10;
+    e.head = 4;
+    e.lz77_type = (has_ext && o.lz77_type) ? o.lz77_type : 0x10;
+    e.chunk = (has_ext && o.lz77_chunk_size) ? o.lz77_chunk_size : 0x1000;
+    e.level5_type = (o.quality == 0) ? 0 : ((has_ext && o.level5_type) ? o.level5_type : 1);
+    e.lz00_key = has_ext ? o.lz00_key : 0;
+    e.ecd_plain = (has_ext && o.ecd_plain_size) ? o.ecd_plain_size : 4;   // ECD.PlainSize
+    e.quality0 = o.quality == 0;
+    switch (format) {
+        case AURORA_FMT_GCLZ: case AURORA_FMT_CXLZ: break;
+        case AURORA_FMT_COMP: e.core = AURORA_FMT_LZ11; break;
+        case AURORA_FMT_LZ_3DS: e.head = 8; break;
+        case AURORA_FMT_LZ77:
+            if (e.lz77_type == 0x11) e.core = AURORA_FMT_LZ11;
+            else if (e.lz77_type != 0x10 && e.lz77_type != 0xF7) e.status = AURORA_NOT_SUPPORTED;
+            break;
+        case AURORA_FMT_LEVEL5:
+            if (e.level5_type > 1) e.status = AURORA_NOT_SUPPORTED;
+            e.head = 0;   // the LZ10 header is rewritten in place
+            break;
+        case AURORA_FMT_LZON: e.core = AURORA_FMT_LZO; e.head = 16; break;
+        case AURORA_FMT_SDPC: e.core = AURORA_FMT_LZO; e.head = 8; break;
+        case AURORA_FMT_LEVEL5_LZSS: e.core = AURORA_FMT_LZSS; e.head = 0; break;   // the 16-byte LZSS header is rewritten in place
+        case AURORA_FMT_ECD:
+            // header (16) + plain bytes, then the body: the LZSS core's own 16-byte header lands on [plain, plain + 16)
+            e.core = AURORA_FMT_LZSS;
+            e.head = e.ecd_plain;
+            break;
+        default: {
+            Family f{};
+            if (!family_of(format, f)) return false;
+            // The LZSS core writes its own 16-byte header in front of the body.  It is placed so that the body starts right
+            // behind the family's header (header >= 16 bytes), or the body is moved down afterwards (header < 16 bytes).
+            e.core = AURORA_FMT_LZSS;
+            const uint64_t hlen = f.read_len + f.skip_len;
+            e.head = hlen >= 16 ? hlen - 16 : 0;
+            break;
+        }
+    }
+    return true;
+}
+
+// The plan of one stream of `len` raw bytes with a destination of `cap` bytes: its up-front status (a stream that is not OK
+// runs no core piece and reports out_len 0), whether it is stored, and how many core pieces it has (wrap_encode_piece)
+struct WrapEncPlan {
+    int status;
+    bool stored;    // Level5 OnlySave / ECD stored: no core piece, the finish rule copies the source
+    bool chunked;   // ChunkLZ10 with more than one chunk: the u16 end-offset table at 8, the chunks behind it
+    uint64_t len, cap;
+    uint64_t pieces;   // 0, 1, or the chunk count
+};
+// one core piece: source bytes [soff, soff + slen) of the stream, encoded to [doff, doff + dcap) of its destination window
+struct WrapEncPiece {
+    uint64_t soff, slen, doff, dcap;
+};
+
+// ChunkLZ10: every chunk is encoded into its own worst-case slot and compacted afterwards
+__host__ __device__ inline uint64_t wrap_chunk_slot(const WrapEnc& e) { return core_encode_bound(AURORA_FMT_LZ10, e.chunk); }
+
+__host__ __device__ inline WrapEncPlan wrap_encode_plan(const WrapEnc& e, uint64_t len, uint64_t cap) {
+    WrapEncPlan pl{e.status, false, false, len, cap, 0};
+    if (e.status != AURORA_OK) return pl;
+    if (e.format == AURORA_FMT_LEVEL5 && e.level5_type == 0) {
+        pl.stored = true;
+        if (cap < 4 + len) pl.status = AURORA_DST_TOO_SMALL;
+        return pl;
+    }
+    if (e.format == AURORA_FMT_ECD) {
+        if (e.quality0 || len <= 0x10) {   // ECD.cs:91
+            pl.stored = true;
+            if (cap < 16 + len) pl.status = AURORA_DST_TOO_SMALL;
+            return pl;
+        }
+        if (e.ecd_plain > len) {   // source.Slice(0, plainSize)
+            pl.status = AURORA_INVALID_ARGUMENT;
+            return pl;
+        }
+    }
+    if (e.format == AURORA_FMT_LZ77 && e.lz77_type == 0xF7 && e.chunk < len) {
+        const uint64_t segs = (len + e.chunk - 1) / e.chunk;
+        if (8 + 2 * segs + segs * wrap_chunk_slot(e) > cap) {
+            pl.status = AURORA_DST_TOO_SMALL;
+            return pl;
+        }
+        pl.chunked = true;
+        pl.pieces = segs;
+        return pl;
+    }
+    if (cap < e.head) {
+        pl.status = AURORA_DST_TOO_SMALL;
+        return pl;
+    }
+    pl.pieces = 1;
+    return pl;
+}
+
+// piece k < pl.pieces
+__host__ __device__ inline WrapEncPiece wrap_encode_piece(const WrapEnc& e, const WrapEncPlan& pl, uint64_t k) {
+    if (pl.chunked) {
+        const uint64_t per = wrap_chunk_slot(e), at = k * e.chunk;
+        return WrapEncPiece{at, umin(e.chunk, pl.len - at), 8 + 2 * pl.pieces + k * per, per};
+    }
+    const uint64_t skip = e.format == AURORA_FMT_ECD ? e.ecd_plain : 0;   // ECD's plain prefix is stored, not encoded
+    return WrapEncPiece{skip, pl.len - skip, e.head, pl.cap - e.head};
+}
+
+// The finish rule: the stream's status and out_len from its plan and its pieces' results (r_out / r_st[k], k < pl.pieces),
+// and what is left to write, in this order: a copy from the source, a downward move inside the window, the ChunkLZ10
+// compaction (wrap_encode_chunk_move), then the header bytes (wrap_encode_header).
+struct WrapEncFin {
+    int status;
+    uint64_t out_len;
+    bool stored;                             // the stored form (Level5 OnlySave; ECD stored, also as ECD's fall-back)
+    uint64_t clen;                           // the core's output length
+    uint64_t head_len;                       // header bytes at the start of the window
+    uint64_t copy_dst, copy_src, copy_len;   // source bytes [copy_src, copy_src + copy_len) to window offset copy_dst
+    uint64_t move_dst, move_src, move_len;   // move_dst < move_src: the ranges may overlap
+    uint64_t chunks;                         // ChunkLZ10: chunks 0 .. chunks-1 are compacted, in ascending order
+};
+
+__host__ __device__ inline WrapEncFin wrap_encode_finish(const WrapEnc& e, const WrapEncPlan& pl, const uint64_t* r_out, const int32_t* r_st) {
+    WrapEncFin f{pl.status, 0, false, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (pl.status != AURORA_OK) return f;
+    const uint64_t len = pl.len;
+    auto store = [&](uint64_t h) {
+        if (pl.cap < h + len) {
+            f.status = AURORA_DST_TOO_SMALL;
+            return;
+        }
+        f.stored = true;
+        f.head_len = f.copy_dst = h;
+        f.copy_len = len;
+        f.out_len = h + len;
+    };
+    if (pl.stored) {
+        store(e.format == AURORA_FMT_LEVEL5 ? 4 : 16);
+        return f;
+    }
+    if (pl.chunked) {
+        // the header is written whatever the chunks give; the first failing chunk ends the compaction
+        f.head_len = 8;
+        uint64_t end = 0;
+        for (uint64_t k = 0; k < pl.pieces; k++) {
+            if (r_st[k] != AURORA_OK) {
+                f.status = r_st[k];
+                break;
+            }
+            f.chunks = k + 1;
+            end += r_out[k];
+            if (end > 0xFFFF) {   // "chunks too large to process"
+                f.status = AURORA_INVALID_ARGUMENT;
+                break;
+            }
+        }
+        if (f.status == AURORA_OK) f.out_len = 8 + 2 * pl.pieces + end;
+        return f;
+    }
+    const uint64_t clen = r_out[0];
+    const int cst = r_st[0];
+    f.clen = clen;
+    if (e.format == AURORA_FMT_ECD) {   // ECD.cs:88-121
+        // compressed size = plain bytes + body; not smaller than the input (or no room for it): stored instead
+        if (cst == AURORA_DST_TOO_SMALL || (cst == AURORA_OK && e.ecd_plain + (clen - 16) >= len)) {
+            store(16);
+            return f;
+        }
+        if (cst != AURORA_OK) {
+            f.status = cst;
+            return f;
+        }
+        f.copy_dst = 16;   // over the LZSS core's header
+        f.copy_len = e.ecd_plain;
+        f.head_len = 16;
+        f.out_len = e.ecd_plain + clen;
+        return f;
+    }
+    if (cst != AURORA_OK) {
+        f.status = cst;
+        return f;
+    }
+    f.head_len = e.head;
+    f.out_len = e.head + clen;
+    if (e.format == AURORA_FMT_LEVEL5) {
+        // LZ10.Compress wrote 0x10 + u24 (or, above 0xFFFFFF bytes, 0x10 00 00 00 + u32): CompressHeaderless is the same bytes
+        // without it
+        const uint64_t h = len > 0xFFFFFF ? 8 : 4;
+        if (h == 8) {
+            f.move_dst = 4;
+            f.move_src = 8;
+            f.move_len = clen - 8;
+        }
+        f.head_len = 4;
+        f.out_len = clen - h + 4;
+    } else if (e.format == AURORA_FMT_LEVEL5_LZSS) {
+        f.head_len = 16;
+    } else {
+        Family fam{};
+        if (family_of(e.format, fam)) {
+            const uint64_t hlen = fam.read_len + fam.skip_len;   // the body (CompressHeaderless) goes right behind the header
+            if (hlen < 16) {
+                f.move_dst = hlen;
+                f.move_src = 16;
+                f.move_len = clen - 16;
+            }
+            f.head_len = hlen;
+            f.out_len = hlen + clen - 16;
+        }
+    }
+    return f;
+}
+
+// ChunkLZ10 compaction step k (k < f.chunks, in ascending order): chunk k moves from its slot to behind the chunks in front of
+// it (`end` bytes, updated).  Its destination may overlap earlier chunks' slots, never a later one's: a slot holds at most
+// wrap_chunk_slot bytes.  The chunk's u16 end offset goes to 8 + 2k (wrap_encode_table).
+struct WrapMove {
+    uint64_t dst, src, len;
+};
+__host__ __device__ inline WrapMove wrap_encode_chunk_move(const WrapEnc& e, const WrapEncPlan& pl, uint64_t k, uint64_t ol, uint64_t& end) {
+    const WrapMove m{8 + 2 * pl.pieces + end, wrap_encode_piece(e, pl, k).doff, ol};
+    end += ol;
+    return m;
+}
+__host__ __device__ inline void wrap_encode_table(uint8_t* d, uint64_t k, uint64_t end) {
+    if (end > 0xFFFF) return;
+    d[8 + 2 * k] = uint8_t(end);
+    d[8 + 2 * k + 1] = uint8_t(end >> 8);
+}
+
+// the f.head_len header bytes at d
+__host__ __device__ inline void wrap_encode_header(const WrapEnc& e, const WrapEncPlan& pl, const WrapEncFin& f, uint8_t* d) {
+    if (!f.head_len) return;
+    const uint32_t len = uint32_t(pl.len);
+    const uint64_t clen = f.clen;
+    switch (e.format) {
+        case AURORA_FMT_GCLZ: put_le32(d, kIdGCLZ); break;
+        case AURORA_FMT_CXLZ: put_le32(d, kIdCXLZ); break;
+        case AURORA_FMT_COMP: put_le32(d, kIdCOMP); break;
+        case AURORA_FMT_LZ_3DS:
+            put_le32(d, kId3DS0);
+            put_le32(d + 4, kId3DS1);
+            break;
+        case AURORA_FMT_LZ77:
+            put_le32(d, kIdLZ77);
+            if (pl.chunked) put_le32(d + 4, 0xF7u | (len << 8));
+            break;
+        case AURORA_FMT_SDPC:
+            put_le32(d, kIdSDPC);
+            put_le32(d + 4, len);
+            break;
+        case AURORA_FMT_LZON:
+            put_bytes(d, lzon_magic(), 8);
+            put_be32(d + 8, len);
+            put_be32(d + 12, uint32_t(clen));
+            break;
+        case AURORA_FMT_LEVEL5: put_le32(d, f.stored ? len << 3 : 1u | (len << 3)); break;
+        case AURORA_FMT_LEVEL5_LZSS:
+            put_le32(d, kIdSSZL);
+            put_le32(d + 4, 0);
+            put_le32(d + 8, uint32_t(clen - 16));
+            put_le32(d + 12, len);
+            break;
+        case AURORA_FMT_ECD:
+            put_le32(d, f.stored ? kIdECD : kIdECD | (1u << 24));   // identifier + flag
+            put_be32(d + 4, f.stored ? 0u : uint32_t(e.ecd_plain));
+            put_be32(d + 8, f.stored ? len : uint32_t(e.ecd_plain + clen - 16));
+            put_be32(d + 12, len);
+            break;
+        default: {
+            Family fam{};
+            family_of(e.format, fam);
+            const uint32_t blen = uint32_t(clen - 16);   // body bytes (CompressHeaderless)
+            for (uint64_t j = 0; j < f.head_len; j++) d[j] = 0;
+            put_bytes(d, fam.magic, fam.magic_len);
+            switch (e.format) {
+                case AURORA_FMT_AKLZ: put_be32(d + 12, len); break;
+                case AURORA_FMT_LZ01: put_le32(d + 4, 16 + blen); put_le32(d + 8, len); break;   // LZ01.cs:80-81: the whole file
+                case AURORA_FMT_FCMP: put_le32(d + 4, len); put_le32(d + 8, 305397760u); break;
+                case AURORA_FMT_IECP: put_le32(d + 4, len); break;
+                case AURORA_FMT_MDB4: put_le32(d + 4, len + 1); put_le32(d + 8, len); put_le32(d + 12, 32 + blen - 0x10); break;   // MDB4.cs:78
+                case AURORA_FMT_LZSEGA: put_le32(d, blen); put_le32(d + 4, len); break;
+                case AURORA_FMT_GCZ: put_le32(d, len); break;
+                case AURORA_FMT_LZ00:   // LZ00.cs:86-110
+                    put_le32(d + 4, 64 + blen);
+                    put_le32(d + 16, kIdTemp0);   // LZ00.Name default "Temp.dat", zero padded to 32 bytes
+                    put_le32(d + 20, kIdTemp1);
+                    put_le32(d + 48, len);
+                    put_le32(d + 52, e.lz00_key);
+                    break;
+            }
+            break;
+        }
+    }
+}
+
 // ---- kernel
 namespace {
 
@@ -489,6 +819,102 @@ WrapSlots take_slots(Carve& c, uint64_t m) {
     S.status = c.take<int32_t>(m);
     S.key = c.take<uint32_t>(m);
     return S;
+}
+
+// ---- encode
+
+// encoder slot j: piece k of a stream at (src_off, dst_off), or (use false) an empty slot — length 0, capacity 0, nothing written
+__device__ void put_enc_slot(const WrapSlots& S, uint64_t j, const WrapEnc& e, const WrapEncPlan& pl, uint64_t k, bool use, uint64_t src_off,
+                             uint64_t dst_off) {
+    const WrapEncPiece pc = use ? wrap_encode_piece(e, pl, k) : WrapEncPiece{0, 0, 0, 0};
+    S.src_off[j] = src_off + pc.soff;
+    S.src_len[j] = pc.slen;
+    S.dst_off[j] = dst_off + pc.doff;
+    S.dst_cap[j] = pc.dcap;
+    if (S.key) S.key[j] = e.lz00_key;
+}
+
+// one thread per stream: the plan and the stream slot (its one piece, else empty); ChunkLZ10 batches write the chunk counts
+// instead (entry n stays 0, so the scan's entry n is the total) and leave the slots to wrap_enc_chunk_fill_kernel
+__global__ void wrap_enc_plan_kernel(WrapEnc e, const uint64_t* src_off, const uint64_t* src_len, const uint64_t* dst_off, const uint64_t* dst_cap,
+                                     uint32_t n, WrapEncPlan* plans, uint64_t* chunks, WrapSlots A) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const WrapEncPlan pl = wrap_encode_plan(e, src_len[i], dst_cap[i]);
+    plans[i] = pl;
+    if (chunks) {
+        chunks[i] = pl.chunked ? pl.pieces : 0;
+        if (i == 0) chunks[n] = 0;
+    }
+    if (A.src_off) put_enc_slot(A, i, e, pl, 0, pl.pieces == 1 && !pl.chunked, src_off[i], dst_off[i]);
+}
+
+// ChunkLZ10: stream slot i, then the chunk slots of stream i behind the n stream slots, at n + base[i]
+__global__ void wrap_enc_chunk_fill_kernel(WrapEnc e, const uint64_t* src_off, const uint64_t* dst_off, uint32_t n, const WrapEncPlan* plans,
+                                           const uint64_t* base, WrapSlots A) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const WrapEncPlan pl = plans[i];
+    const uint64_t so = src_off[i], dof = dst_off[i];
+    put_enc_slot(A, i, e, pl, 0, pl.pieces == 1 && !pl.chunked, so, dof);
+    if (pl.chunked)
+        for (uint64_t k = 0; k < pl.pieces; k++) put_enc_slot(A, n + base[i] + k, e, pl, k, true, so, dof);
+}
+
+// in-place downward move (d < s, the ranges may overlap), in pieces of 32 x kMoveBytes bytes: every lane loads its bytes of a
+// piece before any lane stores them, and the pieces go in ascending order, so no store lands on a byte a later load reads
+constexpr int kMoveBytes = 16;
+__device__ void warp_move_down(uint8_t* d, const uint8_t* s, uint64_t len, uint32_t lane) {
+    for (uint64_t at = 0; at < len; at += 32 * kMoveBytes) {
+        uint8_t v[kMoveBytes];
+#pragma unroll
+        for (int j = 0; j < kMoveBytes; j++) {
+            const uint64_t p = at + j * 32 + lane;
+            if (p < len) v[j] = s[p];
+        }
+        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < kMoveBytes; j++) {
+            const uint64_t p = at + j * 32 + lane;
+            if (p < len) d[p] = v[j];
+        }
+        __syncwarp();
+    }
+}
+
+// one warp per stream: the finish rule over the pieces' results — the stored copy or ECD's plain prefix, the downward move, the
+// ChunkLZ10 compaction with its end-offset table, then the header bytes and the caller's out_len / status
+__global__ void wrap_enc_finish_kernel(WrapEnc e, const uint8_t* src, const uint64_t* src_off, uint8_t* dst, const uint64_t* dst_off,
+                                       uint32_t n, const WrapEncPlan* plans, const uint64_t* base, WrapSlots A, uint64_t* out_len,
+                                       int32_t* status) {
+    const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (w >= n) return;
+    const WrapEncPlan pl = plans[w];
+    const uint64_t j = pl.chunked ? n + base[w] : w;
+    const WrapEncFin f = wrap_encode_finish(e, pl, A.out_len + j, A.status + j);
+    uint8_t* d = dst + dst_off[w];
+    if (f.copy_len) {   // (16-byte accesses when source and destination share their address modulo 16, else 8, 4 or 1 byte)
+        uint8_t* cd = d + f.copy_dst;
+        const uint8_t* cs = src + src_off[w] + f.copy_src;
+        const uintptr_t mis = reinterpret_cast<uintptr_t>(cd) ^ reinterpret_cast<uintptr_t>(cs);
+        if ((mis & 15) == 0) warp_copy<uint4>(cd, cs, f.copy_len, lane);
+        else if ((mis & 7) == 0) warp_copy<uint2>(cd, cs, f.copy_len, lane);
+        else if ((mis & 3) == 0) warp_copy<uint32_t>(cd, cs, f.copy_len, lane);
+        else warp_copy<uint8_t>(cd, cs, f.copy_len, lane);
+    }
+    if (f.move_len) warp_move_down(d + f.move_dst, d + f.move_src, f.move_len, lane);
+    uint64_t end = 0;
+    for (uint64_t k = 0; k < f.chunks; k++) {
+        const WrapMove mv = wrap_encode_chunk_move(e, pl, k, A.out_len[j + k], end);
+        if (mv.dst != mv.src) warp_move_down(d + mv.dst, d + mv.src, mv.len, lane);
+        if (lane == 0) wrap_encode_table(d, k, end);
+    }
+    __syncwarp();
+    if (lane == 0) {
+        wrap_encode_header(e, pl, f, d);
+        out_len[w] = f.out_len;
+        status[w] = f.status;
+    }
 }
 
 #define WRAP_TRY(expr)                                   \
@@ -724,10 +1150,98 @@ cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opt
     return cudaSuccess;
 }
 
-namespace {
-inline void put_le32(uint8_t* p, uint32_t v) { p[0] = uint8_t(v); p[1] = uint8_t(v >> 8); p[2] = uint8_t(v >> 16); p[3] = uint8_t(v >> 24); }
-inline void put_be32(uint8_t* p, uint32_t v) { p[3] = uint8_t(v); p[2] = uint8_t(v >> 8); p[1] = uint8_t(v >> 16); p[0] = uint8_t(v >> 24); }
-}  // namespace
+int wrapped_encode_batch_device(int format, const aurora_codec_opts* opts, size_t n, const uint8_t* d_src_base, uint64_t src_total,
+                                const uint64_t* d_src_off, const uint64_t* d_src_len, uint8_t* d_dst_base, const uint64_t* d_dst_off,
+                                const uint64_t* d_dst_cap, uint64_t* d_out_len, int32_t* d_status, WrapScratch& scr,
+                                DevBuf& enc_scratch, unsigned int* ticket, int sm_count, cudaStream_t st, uint64_t* launches,
+                                cudaError_t* err) {
+    const aurora_codec_opts o = wrap_core_opts(format, opts);
+    WrapEnc e;
+    if (!wrap_encode_opts(format, o, e)) return AURORA_INVALID_ARGUMENT;
+    EncodeParams P{};
+    const int rc = fill_encode_params(P, e.core, &o);   // (the LzProperties of every wrapper format are valid)
+    if (rc != AURORA_OK) return rc;
+    auto cuda = [&](cudaError_t c) {
+        *err = c;
+        return c == cudaSuccess ? AURORA_OK : AURORA_CUDA_ERROR;
+    };
+#define WRAP_ENC_TRY(expr)                                     \
+    do {                                                       \
+        if (cuda(expr) != AURORA_OK) return AURORA_CUDA_ERROR; \
+    } while (0)
+    const bool chunked = format == AURORA_FMT_LZ77 && e.lz77_type == 0xF7;
+    const uint32_t N = uint32_t(n);
+    const unsigned grid = (N + 127) / 128;
+
+    // per-stream scratch: plans, ChunkLZ10's chunk counts and their exclusive scan, the scan's temporary storage
+    size_t scan_bytes = 0;
+    if (chunked)
+        WRAP_ENC_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, static_cast<uint64_t*>(nullptr), static_cast<uint64_t*>(nullptr), n + 1, st));
+    WRAP_ENC_TRY(scr.plans.reserve(((n * sizeof(WrapEncPlan) + 15) & ~15ull) + 2 * (((n + 1) * 8 + 15) & ~15ull) + scan_bytes));
+    Carve cp{static_cast<uint8_t*>(scr.plans.p)};
+    WrapEncPlan* plans = cp.take<WrapEncPlan>(n);
+    uint64_t* counts = cp.take<uint64_t>(n + 1);
+    uint64_t* base = cp.take<uint64_t>(n + 1);
+    void* scan_tmp = cp.p;
+
+    WrapSlots A{};
+    uint64_t m = n;
+    if (!chunked) {   // one slot per stream: the plan pass writes them
+        WRAP_ENC_TRY(scr.slots.reserve(slot_bytes(n)));
+        Carve cs{static_cast<uint8_t*>(scr.slots.p)};
+        A = take_slots(cs, n);
+        if (format != AURORA_FMT_LZ00) A.key = nullptr;
+    }
+    wrap_enc_plan_kernel<<<grid, 128, 0, st>>>(e, d_src_off, d_src_len, d_dst_off, d_dst_cap, N, plans, chunked ? counts : nullptr, A);
+    WRAP_ENC_TRY(cudaGetLastError());
+    ++*launches;
+    if (chunked) {
+        // the chunk slots follow the n stream slots; their number sizes the descriptors, and only the device knows the lengths
+        WRAP_ENC_TRY(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, counts, base, n + 1, st));
+        *launches += 2;   // (DeviceScan: an initialisation and a scan kernel)
+        uint64_t total = 0;
+        WRAP_ENC_TRY(cudaMemcpyAsync(&total, base + n, sizeof(total), cudaMemcpyDeviceToHost, st));
+        WRAP_ENC_TRY(cudaStreamSynchronize(st));
+        m = n + total;
+        if (m > 0xFFFFFFF0ull) return cuda(cudaErrorInvalidValue);   // a core launch counts its streams in 32 bits
+        WRAP_ENC_TRY(scr.slots.reserve(slot_bytes(m)));
+        Carve cs{static_cast<uint8_t*>(scr.slots.p)};
+        A = take_slots(cs, m);
+        A.key = nullptr;
+        wrap_enc_chunk_fill_kernel<<<grid, 128, 0, st>>>(e, d_src_off, d_dst_off, N, plans, base, A);
+        WRAP_ENC_TRY(cudaGetLastError());
+        ++*launches;
+    }
+
+    // the core encoder over every slot, as aurora_encode_batch_device runs it
+    const int warps = encode_resident_warps(sm_count);
+    P.scratch_per_warp = encode_scratch_per_warp(e.core, P.hash_bits, P.chain_bits, 0);   // (no section staging: not MIO0 / Yay0)
+    WRAP_ENC_TRY(enc_scratch.reserve(size_t(warps) * P.scratch_per_warp));
+    WRAP_ENC_TRY(cudaMemsetAsync(ticket, 0, 64, st));
+    P.scratch = static_cast<uint8_t*>(enc_scratch.p);
+    P.src_base = d_src_base;
+    P.src_limit = src_total;
+    P.src_off = A.src_off;
+    P.src_len = A.src_len;
+    P.dst_base = d_dst_base;
+    P.dst_off = A.dst_off;
+    P.dst_cap = A.dst_cap;
+    P.out_len = A.out_len;
+    P.status = A.status;
+    P.ticket = ticket;
+    P.n = uint32_t(m);
+    WRAP_ENC_TRY(launch_encode(P, warps, st));
+    ++*launches;
+    if (format == AURORA_FMT_LZ00) {   // the body the encoder just wrote goes under the keystream (bytes [16, out_len) of every piece)
+        WRAP_ENC_TRY(launch_lcg_xor(d_dst_base, A.dst_off, A.out_len, A.dst_cap, A.key, 16, N, st));
+        ++*launches;
+    }
+    wrap_enc_finish_kernel<<<(N + 3) / 4, 128, 0, st>>>(e, d_src_base, d_src_off, d_dst_base, d_dst_off, N, plans, base, A, d_out_len, d_status);
+    WRAP_ENC_TRY(cudaGetLastError());
+    ++*launches;
+#undef WRAP_ENC_TRY
+    return AURORA_OK;
+}
 
 // GetDecompressedSize of the wrapper formats: a header peek
 int wrapped_decoded_size(int format, const uint8_t* p, uint64_t len, uint64_t* out_size) {
@@ -859,234 +1373,57 @@ uint64_t wrapped_encode_bound(int format, uint64_t raw_len, const aurora_codec_o
     }
 }
 
-// Compress of the wrapper formats: the core encoder writes at the offset the wrapper header leaves free, the header
-// bytes are written (or the core's own header is rewritten in place) on the host afterwards.
+// Compress of the wrapper formats: the encode rules above, with the core pieces of every stream in one core batch and the
+// finish rule's copies, moves and header bytes applied on the host.
 int wrapped_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* opts, size_t n, const uint8_t* src_base,
                          const uint64_t* src_off, const uint64_t* src_len, uint8_t* dst_base, const uint64_t* dst_off,
                          const uint64_t* dst_cap, uint64_t* out_len, int32_t* status) {
-    aurora_codec_opts o;
-    if (opts) o = *opts;
-    else aurora_codec_opts_init(&o);
-    const bool has_ext = o.struct_size >= sizeof(aurora_codec_opts);
-    const uint32_t lz77_type = (has_ext && o.lz77_type) ? o.lz77_type : 0x10;
-    const uint64_t chunk = (has_ext && o.lz77_chunk_size) ? o.lz77_chunk_size : 0x1000;
-    const uint32_t level5_type = (o.quality == 0) ? 0 : ((has_ext && o.level5_type) ? o.level5_type : 1);
-
-    const uint64_t ecd_plain = (has_ext && o.ecd_plain_size) ? o.ecd_plain_size : 4;   // ECD.PlainSize
-    auto ecd_stored = [&](uint64_t len) { return o.quality == 0 || len <= 0x10; };    // ECD.cs:91
-    const uint32_t lz00_key = has_ext ? o.lz00_key : 0;
-
-    int core = AURORA_FMT_LZ10;
-    uint64_t head = 4;   // bytes in front of the core's output
-    switch (format) {
-        case AURORA_FMT_GCLZ: case AURORA_FMT_CXLZ: break;
-        case AURORA_FMT_COMP: core = AURORA_FMT_LZ11; break;
-        case AURORA_FMT_LZ_3DS: head = 8; break;
-        case AURORA_FMT_LZ77:
-            if (lz77_type == 0x11) core = AURORA_FMT_LZ11;
-            else if (lz77_type != 0x10 && lz77_type != 0xF7) {
-                for (size_t i = 0; i < n; i++) { status[i] = AURORA_NOT_SUPPORTED; out_len[i] = 0; }
-                return AURORA_OK;
-            }
-            break;
-        case AURORA_FMT_LEVEL5:
-            if (level5_type > 1) {
-                for (size_t i = 0; i < n; i++) { status[i] = AURORA_NOT_SUPPORTED; out_len[i] = 0; }
-                return AURORA_OK;
-            }
-            head = 0;   // the LZ10 header is rewritten in place
-            break;
-        case AURORA_FMT_LZON: core = AURORA_FMT_LZO; head = 16; break;
-        case AURORA_FMT_SDPC: core = AURORA_FMT_LZO; head = 8; break;
-        case AURORA_FMT_LEVEL5_LZSS:
-            core = AURORA_FMT_LZSS;
-            head = 0;   // the 16-byte LZSS header is rewritten in place
-            aurora_lz_props_window(&o.lzss, 0x1000, 0xF + 3, 3, 0xFEE, 1);
-            break;
-        case AURORA_FMT_ECD:
-            // header (16) + plain bytes, then the body: the LZSS core's own 16-byte header lands on [plain, plain + 16)
-            core = AURORA_FMT_LZSS;
-            head = ecd_plain;
-            aurora_lz_props_window(&o.lzss, 0x400, 0x42, 3, 0x3BE, 1);
-            break;
-        default: {
-            Family f{};
-            if (!family_of(format, f)) return AURORA_INVALID_ARGUMENT;
-            // The LZSS core writes its own 16-byte header in front of the body.  It is placed so that the body starts right
-            // behind the family's header (header >= 16 bytes), or the body is moved down afterwards (header < 16 bytes).
-            core = AURORA_FMT_LZSS;
-            const uint64_t hlen = f.read_len + f.skip_len;
-            head = hlen >= 16 ? hlen - 16 : 0;
-            family_props(f, &o.lzss);
-            break;
-        }
+    const aurora_codec_opts o = wrap_core_opts(format, opts);
+    WrapEnc e;
+    if (!wrap_encode_opts(format, o, e)) return AURORA_INVALID_ARGUMENT;
+    if (e.status != AURORA_OK) {
+        for (size_t i = 0; i < n; i++) { status[i] = e.status; out_len[i] = 0; }
+        return AURORA_OK;
     }
-
-    // sub-buffers: one per stream, or one per chunk for LZ77 ChunkLZ10 with more than one chunk
-    struct Piece { size_t stream; uint64_t soff, slen, doff; };
-    std::vector<Piece> pieces;
-    std::vector<uint64_t> table_at(n, 0);   // chunked: offset of the u16 table inside the stream's slot
+    std::vector<WrapEncPlan> plans(n);
+    std::vector<size_t> first(n);   // the stream's first piece
+    std::vector<uint64_t> so, sl, dof, dc;
     for (size_t i = 0; i < n; i++) {
-        status[i] = AURORA_OK;
-        out_len[i] = 0;
-        const uint64_t len = src_len[i];
-        if (format == AURORA_FMT_LEVEL5 && level5_type == 0) continue;   // stored on the host below
-        if (format == AURORA_FMT_ECD) {
-            if (ecd_stored(len)) continue;                                   // stored on the host below
-            if (ecd_plain > len) { status[i] = AURORA_INVALID_ARGUMENT; continue; }   // source.Slice(0, plainSize)
-            if (dst_cap[i] < head) { status[i] = AURORA_DST_TOO_SMALL; continue; }
-            pieces.push_back(Piece{i, ecd_plain, len - ecd_plain, head});
-            continue;
-        }
-        if (format == AURORA_FMT_LZ77 && lz77_type == 0xF7 && chunk < len) {
-            const uint64_t segs = (len + chunk - 1) / chunk;
-            const uint64_t body = 8 + 2 * segs;
-            const uint64_t per = aurora_encode_bound(AURORA_FMT_LZ10, chunk);
-            if (body + segs * per > dst_cap[i]) { status[i] = AURORA_DST_TOO_SMALL; continue; }
-            table_at[i] = 8;
-            for (uint64_t k = 0; k < segs; k++)   // encode every chunk into its own worst-case slot, compact afterwards
-                pieces.push_back(Piece{i, k * chunk, std::min(chunk, len - k * chunk), body + k * per});
-        } else {
-            if (dst_cap[i] < head) { status[i] = AURORA_DST_TOO_SMALL; continue; }
-            pieces.push_back(Piece{i, 0, len, head});
+        plans[i] = wrap_encode_plan(e, src_len[i], dst_cap[i]);
+        first[i] = so.size();
+        for (uint64_t k = 0; k < plans[i].pieces; k++) {
+            const WrapEncPiece pc = wrap_encode_piece(e, plans[i], k);
+            so.push_back(src_off[i] + pc.soff);
+            sl.push_back(pc.slen);
+            dof.push_back(dst_off[i] + pc.doff);
+            dc.push_back(pc.dcap);
         }
     }
-    const size_t m = pieces.size();
-    std::vector<uint64_t> so(m), sl(m), dof(m), dc(m), ol(m);
-    std::vector<int32_t> st(m);
-    for (size_t j = 0; j < m; j++) {
-        const Piece& pc = pieces[j];
-        so[j] = src_off[pc.stream] + pc.soff;
-        sl[j] = pc.slen;
-        dof[j] = dst_off[pc.stream] + pc.doff;
-        dc[j] = table_at[pc.stream] ? aurora_encode_bound(AURORA_FMT_LZ10, chunk) : dst_cap[pc.stream] - pc.doff;
-    }
+    const size_t m = so.size();
+    std::vector<uint64_t> ol(m + 1, 0);
+    std::vector<int32_t> st(m + 1, AURORA_OK);
     if (m) {
         std::vector<uint32_t> keys;
-        if (format == AURORA_FMT_LZ00) keys.assign(m, lz00_key);   // the body goes under the keystream on the device
-        const int rc = encode_core_batch(ctx, core, &o, m, src_base, so.data(), sl.data(), dst_base, dof.data(), dc.data(), ol.data(),
+        if (format == AURORA_FMT_LZ00) keys.assign(m, e.lz00_key);   // the body goes under the keystream on the device
+        const int rc = encode_core_batch(ctx, e.core, &o, m, src_base, so.data(), sl.data(), dst_base, dof.data(), dc.data(), ol.data(),
                                          st.data(), keys.empty() ? nullptr : keys.data(), 16);
         if (rc != AURORA_OK) return rc;
     }
-
-    // headers
-    size_t j = 0;
     for (size_t i = 0; i < n; i++) {
+        const WrapEncPlan& pl = plans[i];
+        const WrapEncFin f = wrap_encode_finish(e, pl, ol.data() + first[i], st.data() + first[i]);
         uint8_t* d = dst_base + dst_off[i];
-        const uint64_t len = src_len[i];
-        if (format == AURORA_FMT_LEVEL5 && level5_type == 0) {
-            if (dst_cap[i] < 4 + len) { status[i] = AURORA_DST_TOO_SMALL; continue; }
-            put_le32(d, uint32_t(len) << 3);
-            std::memcpy(d + 4, src_base + src_off[i], size_t(len));
-            out_len[i] = 4 + len;
-            continue;
+        if (f.copy_len) std::memcpy(d + f.copy_dst, src_base + src_off[i] + f.copy_src, size_t(f.copy_len));
+        if (f.move_len) std::memmove(d + f.move_dst, d + f.move_src, size_t(f.move_len));
+        uint64_t end = 0;
+        for (uint64_t k = 0; k < f.chunks; k++) {
+            const WrapMove mv = wrap_encode_chunk_move(e, pl, k, ol[first[i] + k], end);
+            std::memmove(d + mv.dst, d + mv.src, size_t(mv.len));
+            wrap_encode_table(d, k, end);
         }
-        if (format == AURORA_FMT_ECD) {   // ECD.cs:88-121
-            auto store = [&]() {
-                if (dst_cap[i] < 16 + len) { status[i] = AURORA_DST_TOO_SMALL; return; }
-                std::memcpy(d, "ECD", 4);   // identifier + flag 0
-                put_be32(d + 4, 0);
-                put_be32(d + 8, uint32_t(len));
-                put_be32(d + 12, uint32_t(len));
-                std::memcpy(d + 16, src_base + src_off[i], size_t(len));
-                status[i] = AURORA_OK;
-                out_len[i] = 16 + len;
-            };
-            if (ecd_stored(len)) { store(); continue; }
-            if (status[i] != AURORA_OK) continue;
-            const uint64_t clen = ol[j];
-            const int cst = st[j];
-            j++;
-            // compressed size = plain bytes + body; not smaller than the input (or no room for it): stored instead
-            if (cst == AURORA_DST_TOO_SMALL || (cst == AURORA_OK && ecd_plain + (clen - 16) >= len)) { store(); continue; }
-            if (cst != AURORA_OK) { status[i] = cst; continue; }
-            std::memmove(d + 16, src_base + src_off[i], size_t(ecd_plain));   // overwrites the LZSS core's header
-            std::memcpy(d, "ECD\x01", 4);
-            put_be32(d + 4, uint32_t(ecd_plain));
-            put_be32(d + 8, uint32_t(ecd_plain + clen - 16));
-            put_be32(d + 12, uint32_t(len));
-            out_len[i] = 16 + ecd_plain + clen - 16;
-            continue;
-        }
-        if (status[i] != AURORA_OK) continue;
-        if (table_at[i]) {
-            const uint64_t segs = (len + chunk - 1) / chunk;
-            const uint64_t body = 8 + 2 * segs;
-            std::memcpy(d, "LZ77", 4);
-            put_le32(d + 4, 0xF7u | (uint32_t(len) << 8));
-            uint64_t end = 0;
-            for (uint64_t k = 0; k < segs; k++, j++) {
-                if (st[j] != AURORA_OK && status[i] == AURORA_OK) status[i] = st[j];
-                if (status[i] != AURORA_OK) continue;
-                std::memmove(d + body + end, d + pieces[j].doff, size_t(ol[j]));
-                end += ol[j];
-                if (end > 0xFFFF) { status[i] = AURORA_INVALID_ARGUMENT; continue; }   // "chunks too large to process"
-                d[8 + 2 * k] = uint8_t(end);
-                d[8 + 2 * k + 1] = uint8_t(end >> 8);
-            }
-            if (status[i] == AURORA_OK) out_len[i] = body + end;
-            continue;
-        }
-        const uint64_t clen = ol[j];
-        const int cst = st[j];
-        j++;
-        if (cst != AURORA_OK) { status[i] = cst; continue; }
-        switch (format) {
-            case AURORA_FMT_GCLZ: std::memcpy(d, "GCLZ", 4); break;
-            case AURORA_FMT_CXLZ: std::memcpy(d, "CXLZ", 4); break;
-            case AURORA_FMT_COMP: std::memcpy(d, "COMP", 4); break;
-            case AURORA_FMT_LZ77: std::memcpy(d, "LZ77", 4); break;
-            case AURORA_FMT_LZ_3DS: std::memcpy(d, "3DS-LZ\r\n", 8); break;
-            case AURORA_FMT_SDPC:
-                std::memcpy(d, "SDPC", 4);
-                put_le32(d + 4, uint32_t(len));
-                break;
-            case AURORA_FMT_LZON:
-                std::memcpy(d, lzon_magic(), 8);
-                put_be32(d + 8, uint32_t(len));
-                put_be32(d + 12, uint32_t(clen));
-                break;
-            case AURORA_FMT_LEVEL5: {
-                // LZ10.Compress wrote 0x10 + u24 (or 0x10 00 00 00 + u32): CompressHeaderless is the same bytes without it
-                const uint64_t h = (d[1] | d[2] | d[3]) == 0 ? 8 : 4;
-                if (h == 8) std::memmove(d + 4, d + 8, size_t(clen - 8));
-                put_le32(d, 1u | (uint32_t(len) << 3));
-                out_len[i] = clen - h + 4;
-                continue;
-            }
-            case AURORA_FMT_LEVEL5_LZSS:
-                std::memcpy(d, "SSZL", 4);
-                put_le32(d + 4, 0);
-                put_le32(d + 8, uint32_t(clen - 16));
-                put_le32(d + 12, uint32_t(len));
-                break;
-            default: {
-                Family f{};
-                family_of(format, f);
-                const uint64_t hlen = f.read_len + f.skip_len, blen = clen - 16;   // body bytes (CompressHeaderless)
-                if (hlen < 16) std::memmove(d + hlen, d + 16, size_t(blen));
-                std::memset(d, 0, size_t(hlen));
-                if (f.magic_len) std::memcpy(d, f.magic, f.magic_len);
-                switch (format) {
-                    case AURORA_FMT_AKLZ: put_be32(d + 12, uint32_t(len)); break;
-                    case AURORA_FMT_LZ01: put_le32(d + 4, uint32_t(16 + blen)); put_le32(d + 8, uint32_t(len)); break;   // LZ01.cs:80-81: the whole file
-                    case AURORA_FMT_FCMP: put_le32(d + 4, uint32_t(len)); put_le32(d + 8, 305397760u); break;
-                    case AURORA_FMT_IECP: put_le32(d + 4, uint32_t(len)); break;
-                    case AURORA_FMT_MDB4: put_le32(d + 4, uint32_t(len) + 1); put_le32(d + 8, uint32_t(len)); put_le32(d + 12, uint32_t(32 + blen - 0x10)); break;   // MDB4.cs:78
-                    case AURORA_FMT_LZSEGA: put_le32(d, uint32_t(blen)); put_le32(d + 4, uint32_t(len)); break;
-                    case AURORA_FMT_GCZ: put_le32(d, uint32_t(len)); break;
-                    case AURORA_FMT_LZ00:   // LZ00.cs:86-110
-                        put_le32(d + 4, uint32_t(64 + blen));
-                        std::memcpy(d + 16, "Temp.dat", 8);   // LZ00.Name default, zero padded to 32 bytes
-                        put_le32(d + 48, uint32_t(len));
-                        put_le32(d + 52, lz00_key);
-                        break;
-                }
-                out_len[i] = hlen + blen;
-                continue;
-            }
-        }
-        out_len[i] = head + clen;
+        wrap_encode_header(e, pl, f, d);
+        out_len[i] = f.out_len;
+        status[i] = f.status;
     }
     return AURORA_OK;
 }

@@ -227,10 +227,12 @@ int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* op
  * array of aurora_decoded_size_batch_device with size_scan != 0) are per device, not per call, so two batches of the same
  * device may not run concurrently (use one stream per device, or order the streams with events); different devices are
  * independent.
- * The wrapper formats (15-32) add per-device scratch of their own: per-stream plans and sub-stream descriptors and results,
- * LZ77's chunk counts, and LZ00's copy of the source.
+ * The wrapper formats (15-32) add per-device scratch of their own, shared by decode and encode: per-stream plans and
+ * sub-stream (encode: core piece) descriptors and results, LZ77's chunk counts and their scan, and LZ00's copy of the source
+ * (decode).  A wrapped encode also uses the device's encoder scratch.
  * None of these calls synchronises with the host, reads a result on the host or copies the source to or from the host,
- * with one exception: aurora_decode_batch_device of LZ77 (below).
+ * with two exceptions: aurora_decode_batch_device of LZ77 and aurora_encode_batch_device of LZ77 with opts.lz77_type 0xF7
+ * (below).
  *
  * aurora_decode_batch_device of the wrapper formats: out_len, consumed, status and the decoded bytes in
  * [dst_off[i], dst_off[i] + min(out_len[i], dst_cap[i])) are those aurora_decode_batch gives for the same streams, options
@@ -255,6 +257,22 @@ int aurora_decode_batch_device(aurora_ctx* ctx, int device, int format, const au
                                uint64_t* d_out_len, uint64_t* d_consumed, int32_t* d_status,
                                void* stream);
 
+/*
+ * aurora_encode_batch_device: the core formats and the wrapper formats (15-32); BLZ answers AURORA_NOT_SUPPORTED (its reversal
+ * passes and footer run only in aurora_encode_batch).  For the wrapper formats, out_len, status and the bytes
+ * [dst_off[i], dst_off[i] + out_len[i]) of OK streams are those aurora_encode_batch gives for the same sources, options and
+ * capacities, including its answers for a core piece without room (DST_TOO_SMALL, out_len 0), ChunkLZ10 end offsets past
+ * 0xFFFF (INVALID_ARGUMENT), an lz77_type / level5_type without an encoder (NOT_SUPPORTED on every stream) and ECD's
+ * ecd_plain_size above the source length (INVALID_ARGUMENT).  Nothing outside the destination windows is written and the
+ * source is never modified (LZ00's keystream goes over the encoded output).  Same argument rules as the core formats.  One
+ * thread per stream plans its core pieces (one piece, or one per ChunkLZ10 chunk in a worst-case slot), the unchanged core
+ * encoder runs once over all pieces, and one warp per stream writes the header, the stored payloads and ECD's plain prefix,
+ * moves bodies down in place (Level5 above 0xFFFFFF bytes, FCMP / IECP / LZSega / GCZ) and compacts the ChunkLZ10 chunks
+ * behind their end-offset table.  Kernel launches per call: 3 (plan, core, finish); 4 for LZ00 (+ the keystream pass); 6 for
+ * LZ77 with opts.lz77_type 0xF7 (plan, a two-kernel exclusive scan of the chunk counts, chunk fill, core, finish).  ChunkLZ10
+ * READS ONE VALUE BACK, the batch's total chunk count, which sizes the piece descriptors: that call returns after the stream
+ * has run its plan pass.  opts.balance is not applied to the wrapper formats.
+ */
 int aurora_encode_batch_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts,
                                size_t n, const uint8_t* d_src_base, uint64_t src_total,
                                const uint64_t* d_src_off, const uint64_t* d_src_len,
