@@ -96,10 +96,10 @@ class BatchCodec:
         outs = [dst[int(doff[i]):int(doff[i]) + min(int(out_len[i]), int(caps[i]))].tobytes() for i in range(len(blobs))]
         return outs, out_len, consumed, status
 
-    def decoded_size_batch(self, fmt, blobs, opts=None, size_scan=False):
+    def decoded_size_packed(self, fmt, base, off, ln, opts=None, size_scan=False):
+        """GetDecompressedSize of the streams base[off[i]:off[i] + ln[i]] -> (size u64, status i32)"""
         opts = opts or _abi.make_opts()
-        base, off, ln = pack(blobs)
-        n = len(blobs)
+        n = len(off)
         out = np.zeros(n, dtype=np.uint64)
         status = np.zeros(n, dtype=np.int32)
         rc = self._L.aurora_decoded_size_batch(self._ctx, fmt, C.byref(opts), n, _ptr(base), _ptr(off), _ptr(ln),
@@ -107,14 +107,22 @@ class BatchCodec:
         self._check(rc, "aurora_decoded_size_batch")
         return out, status
 
-    def is_match_batch(self, fmt, blobs, opts=None):
-        opts = opts or _abi.make_opts()
+    def decoded_size_batch(self, fmt, blobs, opts=None, size_scan=False):
         base, off, ln = pack(blobs)
-        n = len(blobs)
+        return self.decoded_size_packed(fmt, base, off, ln, opts, size_scan)
+
+    def is_match_packed(self, fmt, base, off, ln, opts=None):
+        """IsMatch of the streams base[off[i]:off[i] + ln[i]] -> bool array"""
+        opts = opts or _abi.make_opts()
+        n = len(off)
         m = np.zeros(n, dtype=np.uint8)
         rc = self._L.aurora_is_match_batch(self._ctx, fmt, C.byref(opts), n, _ptr(base), _ptr(off), _ptr(ln), _ptr(m))
         self._check(rc, "aurora_is_match_batch")
         return m.astype(bool)
+
+    def is_match_batch(self, fmt, blobs, opts=None):
+        base, off, ln = pack(blobs)
+        return self.is_match_packed(fmt, base, off, ln, opts)
 
     def scan_offsets(self, fmt, image, opts=None):
         """IsMatch at every byte offset of `image` -> bool array (the data-parallel `-scan`)."""
@@ -153,7 +161,8 @@ class BatchCodec:
         """All arguments are torch CUDA tensors (uint8 / int64 / int32).  Asynchronous on `stream`.
 
         Every format aurora_decode_batch takes, the wrapper formats included (same results as decode_batch); an LZ77 call
-        reads its chunk count back and so waits for `stream`.  d_src must start 16-byte aligned."""
+        reads its chunk count back and an LZ00 call the total size of its keystream-free bodies, so both wait for `stream`.
+        Source windows may repeat and overlap.  d_src must start 16-byte aligned."""
         opts = opts or _abi.make_opts()
         rc = self._L.aurora_decode_batch_device(
             self._ctx, device, fmt, C.byref(opts), d_off.numel(), d_src.data_ptr(), d_src.numel(), d_off.data_ptr(),

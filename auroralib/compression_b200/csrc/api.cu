@@ -215,7 +215,9 @@ struct Layout {
     std::vector<uint64_t> dev_off;
 };
 
-Layout plan_layout(const uint64_t* off, const uint64_t* len, size_t b, size_t e) {
+// packed: re-lay the windows out even when the span copy would be compact enough.  A shard whose kernels rewrite the device
+// copy of its source in place (LZ00's keystream, BLZ's reversal) needs one copy per stream when windows share bytes.
+Layout plan_layout(const uint64_t* off, const uint64_t* len, size_t b, size_t e, bool packed = false) {
     Layout L;
     uint64_t lo = ~0ull, hi = 0, sum = 0;
     for (size_t i = b; i < e; i++) {
@@ -226,7 +228,7 @@ Layout plan_layout(const uint64_t* off, const uint64_t* len, size_t b, size_t e)
     if (b == e) { lo = hi = 0; }
     lo &= ~15ull;
     L.dev_off.resize(e - b);
-    if (hi - lo <= sum + sum / 4 + (1u << 20) + 64 * (e - b)) {
+    if (!packed && hi - lo <= sum + sum / 4 + (1u << 20) + 64 * (e - b)) {
         L.span = true;
         L.lo = lo;
         L.bytes = align_up(hi - lo, 16);
@@ -243,6 +245,21 @@ Layout plan_layout(const uint64_t* off, const uint64_t* len, size_t b, size_t e)
     return L;
 }
 
+// whether two of the non-empty windows [off[i], off[i] + len[i]) of streams [b, e) share a byte (sorted by offset, each window
+// against the furthest end before it)
+bool windows_overlap(const uint64_t* off, const uint64_t* len, size_t b, size_t e) {
+    std::vector<size_t> idx;
+    idx.reserve(e - b);
+    for (size_t i = b; i < e; i++)
+        if (len[i]) idx.push_back(i);
+    std::sort(idx.begin(), idx.end(), [&](size_t x, size_t y) { return off[x] < off[y]; });
+    uint64_t end = 0;
+    for (size_t k = 0; k < idx.size(); k++) {
+        if (k > 0 && off[idx[k]] < end) return true;
+        end = std::max(end, off[idx[k]] + len[idx[k]]);
+    }
+    return false;
+}
 
 // Device -> host copy of the destination windows [off[i], off[i] + ext(i)) of streams [i0, i1) in span mode.  Windows that
 // follow each other in ascending order with a gap of at most `gap_tol` bytes (the alignment padding of a packed batch)
@@ -293,7 +310,8 @@ int decode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
     }
     P.size_only = size_only;
     P.headerless = raw_size != nullptr;
-    const Layout S = plan_layout(src_off, src_len, b, e);
+    // (LZ00 lifts its keystream off the device copy of the source in place: windows that share bytes get one copy each)
+    const Layout S = plan_layout(src_off, src_len, b, e, xor_key && windows_overlap(src_off, src_len, b, e));
     Layout D;
     if (!size_only) D = plan_layout(dst_off, dst_cap, b, e);
     else D.dev_off.assign(n, 0);
@@ -420,7 +438,7 @@ int decode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
                 Q.order = ord;
             }
             if (xor_key) {   // LZ00: lift the keystream off this piece's bodies (device copy, in place)
-                CU_TRY(ctx, launch_lcg_xor(dsrc, Q.src_off, Q.src_len, nullptr, dkey + i0, 0, Q.n, st));
+                CU_TRY(ctx, launch_lcg_xor(dsrc, Q.src_off, dsrc, Q.src_off, Q.src_len, nullptr, dkey + i0, 0, Q.n, st));
                 ctx->launches++;
             }
             CU_TRY(ctx, launch_decode(Q, d->sm_count, st));
@@ -460,7 +478,7 @@ int decode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
             P.order = hist + 64;
         }
         if (xor_key) {   // LZ00: lift the keystream off the bodies (device copy, in place)
-            CU_TRY(ctx, launch_lcg_xor(dsrc, P.src_off, P.src_len, nullptr, dkey, 0, P.n, st));
+            CU_TRY(ctx, launch_lcg_xor(dsrc, P.src_off, dsrc, P.src_off, P.src_len, nullptr, dkey, 0, P.n, st));
             ctx->launches++;
         }
         CU_TRY(ctx, launch_decode(P, d->sm_count, st));
@@ -601,7 +619,8 @@ int encode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
     CU_TRY(ctx, cudaSetDevice(d->dev));
     EncodeParams P{};
     if (fill_encode_params(P, format, opts) != AURORA_OK) return AURORA_INVALID_ARGUMENT;
-    const Layout S = plan_layout(src_off, src_len, b, e);
+    // (BLZ reverses the device copy of the source in place: windows that share bytes get one copy each)
+    const Layout S = plan_layout(src_off, src_len, b, e, format == AURORA_FMT_BLZ && windows_overlap(src_off, src_len, b, e));
     const Layout D = plan_layout(dst_off, dst_cap, b, e);
     uint64_t max_len = 0;
     for (size_t i = b; i < e; i++) max_len = std::max(max_len, src_len[i]);
@@ -662,7 +681,7 @@ int encode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
         uint32_t* dkey = reinterpret_cast<uint32_t*>(dv + 5 * n) + n;
         std::memcpy(hkey, xor_key + b, n * sizeof(uint32_t));
         CU_TRY(ctx, cudaMemcpyAsync(dkey, hkey, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-        CU_TRY(ctx, launch_lcg_xor(ddst, P.dst_off, P.out_len, P.dst_cap, dkey, xor_skip, P.n, st));
+        CU_TRY(ctx, launch_lcg_xor(ddst, P.dst_off, ddst, P.dst_off, P.out_len, P.dst_cap, dkey, xor_skip, P.n, st));
         ctx->launches++;
     }
     CU_TRY(ctx, cudaMemcpyAsync(h + 4 * n, dv + 4 * n, n * sizeof(uint64_t) + n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));

@@ -10,7 +10,8 @@ namespace aurora {
 // core batches (api.cu): the bodies of aurora_decode_batch / aurora_encode_batch for the 14 core formats.
 // raw_size: nullptr, or per-stream decoded sizes of headerless LZ10 / LZ11 / LZSS bodies (DecompressHeaderless).
 // xor_key: nullptr, or per-stream LZ00 keys: the keystream pass (keystream.cu) runs on the device copy of every source
-// stream before it is decoded, resp. over bytes [xor_skip, out_len) of every encoded stream.
+// stream before it is decoded (one copy per stream when windows overlap), resp. over bytes [xor_skip, out_len) of every
+// encoded stream.
 // exact: write only the bytes every stream produced to the host (several sub-batches share one destination).
 int decode_core_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* opts, size_t n, const uint8_t* src_base,
                       const uint64_t* src_off, const uint64_t* src_len, uint8_t* dst_base, const uint64_t* dst_off,

@@ -102,8 +102,8 @@ struct DevBuf {
 };
 
 // per-device scratch of aurora_decode_batch_device / aurora_encode_batch_device for the wrapper formats (wrappers.cu):
-// per-stream plans and sub-streams (+ LZ77's chunk counts and scan), the core launches' descriptors and results, LZ00's copy
-// of the source (decode)
+// per-stream plans and sub-streams (+ LZ77's chunk counts and scan), the core launches' descriptors and results, LZ00's
+// keystream-free bodies (decode: one 16-byte aligned slot per stream)
 struct WrapScratch {
     DevBuf plans, slots, src;
     void release() {
@@ -149,9 +149,10 @@ cudaError_t launch_encode_lz_par(const EncodeParams& p, int sm_count, cudaStream
 size_t encode_scratch_per_warp(int format, int hash_bits, int chain_bits, uint64_t max_src_len);
 int encode_resident_warps(int sm_count);
 cudaError_t launch_size_order(const uint64_t* d_size, uint32_t n, uint32_t* d_hist64, uint32_t* d_order, cudaStream_t st);
-// LZ00's per-byte LCG keystream over bytes [off[i] + skip, off[i] + min(len[i], cap[i])) of every stream (keystream.cu); cap may be null
-cudaError_t launch_lcg_xor(uint8_t* base, const uint64_t* d_off, const uint64_t* d_len, const uint64_t* d_cap, const uint32_t* d_key,
-                           uint32_t skip, uint32_t n, cudaStream_t st);
+// LZ00's per-byte LCG keystream over bytes [skip, min(len[i], cap[i])) of every stream, read at in + in_off[i] and written at
+// out + out_off[i] (keystream.cu; in place: the same pointer and offsets twice); cap may be null
+cudaError_t launch_lcg_xor(const uint8_t* in, const uint64_t* d_in_off, uint8_t* out, const uint64_t* d_out_off, const uint64_t* d_len,
+                           const uint64_t* d_cap, const uint32_t* d_key, uint32_t skip, uint32_t n, cudaStream_t st);
 cudaError_t launch_scan(const uint8_t* image, uint64_t len, uint8_t* match, int format, cudaStream_t st);
 cudaError_t launch_is_match(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint8_t* match, uint32_t n,
                             int format, cudaStream_t st);

@@ -4,8 +4,9 @@
 // steps the key once per byte (GenerateNextKey :125-131: the shift / subtract ladder multiplies by 1103515245, then adds
 // 12345 — an affine map K' = A*K + C mod 2^32).  An affine map composes in closed form, so byte i's key
 // K_(i+1) = A^(i+1)*K0 + C*(A^i + ... + 1) is reachable by square-and-multiply from any position: every thread jumps to
-// its first byte and then strides with the 256-step map.  Decode runs this pass over the device copy of the LZSS body
-// before the LZSS kernel reads it; encode runs it over the body the LZSS encoder just wrote.
+// its first byte and then strides with the 256-step map.  Decode lifts the keystream off the LZSS body before the LZSS kernel
+// reads it (the host entry point in place on its own device copy, the device entry point out of place from the caller's
+// bytes into per-stream scratch slots); encode runs it in place over the body the LZSS encoder just wrote.
 #include "common.cuh"
 
 namespace aurora {
@@ -28,9 +29,11 @@ __device__ __forceinline__ Affine affine_pow(Affine f, uint64_t k) {
 
 constexpr int kThreads = 256;
 
-// bytes [off[i] + skip, off[i] + min(len[i], cap[i])) of stream i, key[i]; blockIdx.y cuts every stream into gridDim.y segments
-__global__ void __launch_bounds__(kThreads) lcg_xor_kernel(uint8_t* base, const uint64_t* off, const uint64_t* len, const uint64_t* cap,
-                                                           const uint32_t* key, uint32_t skip, uint32_t n) {
+// bytes [skip, min(len[i], cap[i])) of stream i under key[i], read at in + in_off[i] and written at out + out_off[i] (the same
+// bytes when in == out and in_off == out_off); blockIdx.y cuts every stream into gridDim.y segments
+__global__ void __launch_bounds__(kThreads) lcg_xor_kernel(const uint8_t* in, const uint64_t* in_off, uint8_t* out, const uint64_t* out_off,
+                                                           const uint64_t* len, const uint64_t* cap, const uint32_t* key, uint32_t skip,
+                                                           uint32_t n) {
     const Affine step{1103515245u, 12345u};
     const Affine stride = affine_pow(step, kThreads);
     for (uint32_t s = blockIdx.x; s < n; s += gridDim.x) {
@@ -41,12 +44,13 @@ __global__ void __launch_bounds__(kThreads) lcg_xor_kernel(uint8_t* base, const 
         const uint64_t lo = seg * blockIdx.y, hi = lo + seg < total ? lo + seg : total;
         uint64_t i = lo + threadIdx.x;
         if (i >= hi) continue;
-        uint8_t* p = base + off[s] + skip;
+        const uint8_t* p = in + in_off[s] + skip;
+        uint8_t* q = out + out_off[s] + skip;
         const Affine jump = affine_pow(step, i + 1);   // Transform steps the key BEFORE it uses it
         uint32_t k = jump.a * key[s] + jump.c;
         for (; i < hi; i += kThreads) {
             const uint32_t t = (k >> 16) & 0x7FFFu;
-            p[i] = uint8_t(p[i] ^ (((t << 8) - t) >> 15));
+            q[i] = uint8_t(p[i] ^ (((t << 8) - t) >> 15));
             k = stride.a * k + stride.c;
         }
     }
@@ -54,11 +58,11 @@ __global__ void __launch_bounds__(kThreads) lcg_xor_kernel(uint8_t* base, const 
 
 }  // namespace
 
-cudaError_t launch_lcg_xor(uint8_t* base, const uint64_t* d_off, const uint64_t* d_len, const uint64_t* d_cap, const uint32_t* d_key,
-                           uint32_t skip, uint32_t n, cudaStream_t st) {
+cudaError_t launch_lcg_xor(const uint8_t* in, const uint64_t* d_in_off, uint8_t* out, const uint64_t* d_out_off, const uint64_t* d_len,
+                           const uint64_t* d_cap, const uint32_t* d_key, uint32_t skip, uint32_t n, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
     const dim3 grid(n < 4736u ? n : 4736u, n >= 1184u ? 1u : n >= 148u ? 8u : 32u);
-    lcg_xor_kernel<<<grid, kThreads, 0, st>>>(base, d_off, d_len, d_cap, d_key, skip, n);
+    lcg_xor_kernel<<<grid, kThreads, 0, st>>>(in, d_in_off, out, d_out_off, d_len, d_cap, d_key, skip, n);
     return cudaGetLastError();
 }
 

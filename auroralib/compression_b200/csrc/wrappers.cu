@@ -797,6 +797,15 @@ __global__ void wrap_merge_kernel(int format, uint32_t n, const WrapPlan* plans,
     status[i] = st;
 }
 
+// LZ00 decode: the size of every body's 16-byte aligned slot in the keystream-free copy, for the scan (entry n is 0, so the
+// scan's entry n is the total)
+__global__ void wrap_slot_bytes_kernel(const uint64_t* len, uint32_t n, uint64_t* bytes) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    bytes[i] = (len[i] + 15) & ~uint64_t(15);
+    if (i == 0) bytes[n] = 0;
+}
+
 // carve 16-byte aligned arrays out of one scratch block
 struct Carve {
     uint8_t* p;
@@ -1048,9 +1057,13 @@ cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opt
     const uint32_t N = uint32_t(n);
     const unsigned grid = (N + 127) / 128;
 
-    // per-stream scratch: plans, sub-streams, LZ77's chunk counts and their exclusive scan, the scan's temporary storage
+    const bool lz00 = format == AURORA_FMT_LZ00;
+
+    // per-stream scratch: plans, sub-streams, LZ77's chunk counts (LZ00: its body slots' sizes) and their exclusive scan, the
+    // scan's temporary storage
     size_t scan_bytes = 0;
-    if (lz77) WRAP_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, static_cast<uint64_t*>(nullptr), static_cast<uint64_t*>(nullptr), n + 1, st));
+    if (lz77 || lz00)
+        WRAP_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, static_cast<uint64_t*>(nullptr), static_cast<uint64_t*>(nullptr), n + 1, st));
     const uint64_t per_stream = ((n * sizeof(WrapPlan) + 15) & ~15ull) + ((n * sizeof(WrapSub) + 15) & ~15ull) + 2 * (((n + 1) * 8 + 15) & ~15ull) + scan_bytes;
     WRAP_TRY(scr.plans.reserve(per_stream));
     Carve cp{static_cast<uint8_t*>(scr.plans.p)};
@@ -1101,13 +1114,27 @@ cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opt
     }
 
     const uint8_t* src = d_src_base;
-    if (format == AURORA_FMT_LZ00) {
-        // the keystream is lifted from a device copy of the source: the caller's bytes stay as they are
-        WRAP_TRY(scr.src.reserve(src_total + 16));
-        WRAP_TRY(cudaMemcpyAsync(scr.src.p, d_src_base, src_total, cudaMemcpyDeviceToDevice, st));
-        WRAP_TRY(launch_lcg_xor(static_cast<uint8_t*>(scr.src.p), A.src_off, A.src_len, nullptr, A.key, 0, N, st));
+    uint64_t src_limit = (src_total + 15) & ~15ull;
+    WrapSlots K = A;   // the core launch's slots (LZ00: its bodies are read from their slots in scratch)
+    if (lz00) {
+        // The keystream is lifted out of place, from the caller's bytes into one 16-byte aligned slot per body: the caller's
+        // source stays as it is, and bodies that share source bytes (a file listed twice, windows that overlap) each get
+        // their own keystream-free copy.  The slots follow each other in stream order (base[i], the exclusive scan of the
+        // aligned body lengths); their total sizes the scratch, and only the device knows the body lengths.
+        wrap_slot_bytes_kernel<<<grid, 128, 0, st>>>(A.src_len, N, counts);
+        WRAP_TRY(cudaGetLastError());
+        ++*launches;
+        WRAP_TRY(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, counts, base, n + 1, st));
+        *launches += 2;   // (DeviceScan: an initialisation and a scan kernel)
+        uint64_t total = 0;
+        WRAP_TRY(cudaMemcpyAsync(&total, base + n, sizeof(total), cudaMemcpyDeviceToHost, st));
+        WRAP_TRY(cudaStreamSynchronize(st));
+        WRAP_TRY(scr.src.reserve(total + 16));
+        WRAP_TRY(launch_lcg_xor(d_src_base, A.src_off, static_cast<uint8_t*>(scr.src.p), base, A.src_len, nullptr, A.key, 0, N, st));
         ++*launches;
         src = static_cast<const uint8_t*>(scr.src.p);
+        src_limit = total;
+        K.src_off = base;
     }
 
     WRAP_TRY(cudaMemsetAsync(ticket, 0, 64, st));
@@ -1116,7 +1143,7 @@ cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opt
         fill_decode_params(P, core, &o);   // (the LzProperties of every wrapper format are valid: no override)
         P.headerless = headerless;
         P.src_base = src;
-        P.src_limit = (src_total + 15) & ~15ull;
+        P.src_limit = src_limit;
         P.src_off = S.src_off;
         P.src_len = S.src_len;
         P.dst_base = d_dst_base;
@@ -1131,7 +1158,7 @@ cudaError_t wrapped_decode_batch_device(int format, const aurora_codec_opts* opt
         ++*launches;
         return launch_decode(P, sm_count, st);
     };
-    WRAP_TRY(run(cores.core, cores.headerless, A, m, ticket));
+    WRAP_TRY(run(cores.core, cores.headerless, K, m, ticket));
     if (lz77) {
         WRAP_TRY(run(AURORA_FMT_LZ11, false, B, n, ticket + 1));
         wrap_redo_select_kernel<<<grid, 128, 0, st>>>(N, plans, base, A, R);
@@ -1233,7 +1260,7 @@ int wrapped_encode_batch_device(int format, const aurora_codec_opts* opts, size_
     WRAP_ENC_TRY(launch_encode(P, warps, st));
     ++*launches;
     if (format == AURORA_FMT_LZ00) {   // the body the encoder just wrote goes under the keystream (bytes [16, out_len) of every piece)
-        WRAP_ENC_TRY(launch_lcg_xor(d_dst_base, A.dst_off, A.out_len, A.dst_cap, A.key, 16, N, st));
+        WRAP_ENC_TRY(launch_lcg_xor(d_dst_base, A.dst_off, d_dst_base, A.dst_off, A.out_len, A.dst_cap, A.key, 16, N, st));
         ++*launches;
     }
     wrap_enc_finish_kernel<<<(N + 3) / 4, 128, 0, st>>>(e, d_src_base, d_src_off, d_dst_base, d_dst_off, N, plans, base, A, d_out_len, d_status);

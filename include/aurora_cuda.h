@@ -172,6 +172,9 @@ void aurora_codec_opts_init(aurora_codec_opts* opts);
  * ---- batch entry points over HOST buffers (the call the C# shim makes) ----
  * Stream i occupies src_base[src_off[i] .. src_off[i]+src_len[i]).  Decoded bytes go to
  * dst_base[dst_off[i] .. dst_off[i]+dst_cap[i]).  All per-stream arrays have n entries.
+ * Source windows may repeat and overlap (one file listed twice, several prefixes of one buffer, every scan hit of an image
+ * read to its end): each stream's results are those it gets alone, and the source is never modified.  Destination windows
+ * must not overlap.  This holds for every entry point below, the device-resident ones included.
  * Streams are sharded over the context's devices by size; no stream aborts the batch: errors
  * are reported in status[i].  Returns AURORA_OK, AURORA_INVALID_ARGUMENT or AURORA_CUDA_ERROR.
  * What the library writes into dst_base: the destination windows and nothing else, with ONE exception — windows that follow
@@ -228,25 +231,29 @@ int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* op
  * device may not run concurrently (use one stream per device, or order the streams with events); different devices are
  * independent.
  * The wrapper formats (15-32) add per-device scratch of their own, shared by decode and encode: per-stream plans and
- * sub-stream (encode: core piece) descriptors and results, LZ77's chunk counts and their scan, and LZ00's copy of the source
- * (decode).  A wrapped encode also uses the device's encoder scratch.
+ * sub-stream (encode: core piece) descriptors and results, LZ77's chunk counts and their scan, and LZ00's keystream-free
+ * bodies with their slot sizes and scan (decode).  A wrapped encode also uses the device's encoder scratch.
  * None of these calls synchronises with the host, reads a result on the host or copies the source to or from the host,
- * with two exceptions: aurora_decode_batch_device of LZ77 and aurora_encode_batch_device of LZ77 with opts.lz77_type 0xF7
- * (below).
+ * with three exceptions: aurora_decode_batch_device of LZ77 and of LZ00, and aurora_encode_batch_device of LZ77 with
+ * opts.lz77_type 0xF7 (below).
  *
  * aurora_decode_batch_device of the wrapper formats: out_len, consumed, status and the decoded bytes in
  * [dst_off[i], dst_off[i] + min(out_len[i], dst_cap[i])) are those aurora_decode_batch gives for the same streams, options
  * and capacities; nothing outside the destination windows is written, and the caller's source is never modified (LZ00's
- * keystream is lifted from a device-to-device copy of [0, src_total) in scratch).  Same argument rules as the core formats
+ * keystream is lifted out of place, from the caller's bytes into one 16-byte aligned scratch slot per body, so bodies that
+ * share source bytes are each decoded as if alone).  Same argument rules as the core formats
  * (16-byte aligned d_src_base, offsets multiples of 16); the sub-streams behind the headers start at any offset.  One
  * thread per stream resolves the header, the core kernels run on the sub-streams, one thread per stream merges the
  * results.  Kernel launches per call: 3 (header pass, core, merge) for GCLZ, CXLZ, COMP, 3DS-LZ, LZOn, SDPC, Level5LZSS and
- * the LZSS-property family; 4 for Level5 and ECD (+ a warp-per-stream copy of stored payloads / ECD's plain prefix) and
- * for LZ00 (+ the keystream pass); 9 for LZ77 (header pass, a two-kernel exclusive scan of the ChunkLZ10 chunk counts,
- * chunk fill, LZ10 over stream and chunk slots, LZ11 over the stream slots, redo selection, a redo LZ10 launch that decodes
- * a file's failing chunk once more so that its bytes win as in the reference's sequential loop, merge).  LZ77 READS ONE
- * VALUE BACK: the batch's total chunk count (a chunk table may be as long as its stream, so only the device knows how many
- * descriptors the chunks need); that call returns after the stream has run its header pass.  opts.balance is not applied
+ * the LZSS-property family; 4 for Level5 and ECD (+ a warp-per-stream copy of stored payloads / ECD's plain prefix); 7 for
+ * LZ00 (header pass, the body slots' sizes, a two-kernel exclusive scan of them, the keystream pass into the slots, core,
+ * merge); 9 for LZ77 (header pass, a two-kernel exclusive scan of the ChunkLZ10 chunk counts, chunk fill, LZ10 over stream
+ * and chunk slots, LZ11 over the stream slots, redo selection, a redo LZ10 launch that decodes a file's failing chunk once
+ * more so that its bytes win as in the reference's sequential loop, merge).  LZ77 READS ONE VALUE BACK: the batch's total
+ * chunk count (a chunk table may be as long as its stream, so only the device knows how many descriptors the chunks need);
+ * LZ00 READS ONE VALUE BACK too: the total size of the body slots (bodies may repeat or overlap in the source, so their
+ * summed length is not bounded by src_total).  Either call returns after the stream has run its header pass and scan.
+ * opts.balance is not applied
  * to the wrapper formats.  aurora_decoded_size_batch_device / aurora_is_match_batch_device / aurora_scan_offsets_device do
  * not take the wrapper formats: a wrapper caller passes its own capacities (e.g. from aurora_decoded_size_batch).
  */

@@ -15,8 +15,10 @@ pytestmark = pytest.mark.gpu
 WRAPPERS = A.WRAPPER_FORMATS
 SENTINEL = 0xA5
 # kernels per call (include/aurora_cuda.h): resolve + core + merge; + the store pass for the formats with stored bytes;
-# + the keystream pass for LZ00; LZ77: resolve, scan (2), chunk fill, LZ10, LZ11, redo selection, redo LZ10, merge
-LAUNCHES = {f: 3 for f in WRAPPERS} | {A.FMT_LEVEL5: 4, A.FMT_ECD: 4, A.FMT_LZ00: 4, A.FMT_LZ77: 9}
+# LZ00: resolve, slot sizes, scan (2), keystream, core, merge; LZ77: resolve, scan (2), chunk fill, LZ10, LZ11, redo
+# selection, redo LZ10, merge
+LAUNCHES = {f: 3 for f in WRAPPERS} | {A.FMT_LEVEL5: 4, A.FMT_ECD: 4, A.FMT_LZ00: 7, A.FMT_LZ77: 9}
+READS_BACK = (A.FMT_LZ77, A.FMT_LZ00)   # the calls that read one value back (LZ77: its chunk count; LZ00: its slot total)
 
 
 def _device_inputs(comps, caps, dev, fill=SENTINEL):
@@ -160,7 +162,9 @@ def test_lz00_keys_leave_the_source_unchanged(codec, oracle):
         assert all(h_dst[int(X["doff"][i]):int(X["doff"][i]) + len(r)].tobytes() == r for i, r in enumerate(raws))
 
 
-def test_calls_are_asynchronous_and_stream_ordered(codec, oracle):
+def test_calls_are_stream_ordered_and_wait_only_to_read_back(codec, oracle):
+    """every wrapper call launches what the header promises on the caller's stream; only LZ77 and LZ00, which read one
+    value back, wait for that stream"""
     import torch
     dev = torch.device("cuda", 0)
     s = torch.cuda.Stream(device=dev)
@@ -184,7 +188,7 @@ def test_calls_are_asynchronous_and_stream_ordered(codec, oracle):
             before = codec.kernel_launches
             _device_call(codec, fmt, X, opts, stream=s.cuda_stream)
             assert codec.kernel_launches - before == LAUNCHES[fmt], fmt_id(fmt)
-            if fmt != A.FMT_LZ77:   # (LZ77 reads its chunk count back: it waits for the stream)
+            if fmt not in READS_BACK:   # (they wait for the stream)
                 assert not s.query(), f"{fmt_id(fmt)}: decode_device waited for the stream"
         s.synchronize()
         _check_against_host(codec, fmt, X, opts, "async")

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 from auroralib.compression_b200 import _abi as A
-from tests.util import corrupt, fmt_id, synth
+from tests.util import corrupt, fmt_id, literal_lzss0_body, lz00_file, lz00_stream, lz00_stream_fast, synth
 
 WRAPPERS = A.WRAPPER_FORMATS
 NO_IDENTIFIER = (A.FMT_LEVEL5, A.FMT_LZSEGA, A.FMT_GCZ)   # no magic: IsMatch is a heuristic on zlib / lengths / the file name
@@ -72,18 +72,7 @@ def test_oracle_wrapper_layouts(oracle, bmp):
     noise = bytes(np.random.default_rng(5).integers(0, 256, 3000, dtype=np.uint8))
     assert oracle.encode(A.FMT_ECD, noise, q8)[0] == b"ECD\x00" + be(0) + be(3000) + be(3000) + noise
     assert oracle.encode(A.FMT_ECD, raw[:16], q8)[0] == b"ECD\x00" + be(0) + be(16) + be(16) + raw[:16]   # Length > 0x10 compresses
-    # LZ00.cs:83-139: 64-byte header, then the Lzss0 body XORed byte by byte; the key steps BEFORE every byte through the
-    # shift / subtract ladder of GenerateNextKey, restated here literally
-    def lz00_stream(key, count):
-        out, M = bytearray(), 0xFFFFFFFF
-        for _ in range(count):
-            x = ((((((((key << 1) + key) << 5) - key) << 5) + key) << 7) - key) & M
-            x = ((x << 6) - x) & M
-            x = ((x << 4) - x) & M
-            key = ((x << 2) - x + 12345) & M
-            t = (key >> 16) & 0x7FFF
-            out.append((((t << 8) - t) >> 15) & 0xFF)
-        return bytes(out)
+    # LZ00.cs:83-139: 64-byte header, then the Lzss0 body XORed byte by byte with lz00_stream (the reference's ladder, literally)
     key = 0x5EEDC0DE
     z = enc(A.FMT_LZ00, lz00_key=key)
     assert z[:64] == b"LZ00" + le(64 + len(b0)) + bytes(8) + b"Temp.dat" + bytes(24) + le(n) + le(key) + bytes(8)
@@ -130,6 +119,26 @@ def test_oracle_wrapper_roundtrip_and_errors(oracle, bmp, fmt):
     assert dst[0] == A.END_OF_STREAM and cons[0] == 3
     _, _, _, dst = oracle.decode_batch(fmt, [c], [2999])
     assert dst[0] == A.DST_TOO_SMALL
+
+
+def test_lz00_keystream_restatements_agree():
+    """lz00_stream_fast (block-wise affine jumps) gives lz00_stream's bytes (the reference's ladder) for every key and length"""
+    rng = np.random.default_rng(32)
+    for key in [0, 1, 0xFFFFFFFF, 0x5EEDC0DE] + [int(k) for k in rng.integers(0, 1 << 32, size=4)]:
+        for count in (0, 1, 255, 256, 257, 511, 513, 3000):
+            assert lz00_stream_fast(key, count) == lz00_stream(key, count), (hex(key), count)
+
+
+def test_oracle_decodes_hand_built_lz00_files(oracle):
+    """the literal-only LZ00 files the keystream tests build: every body length except 1 mod 9, decoded by the oracle"""
+    rng = np.random.default_rng(33)
+    for n in (0, 1, 7, 8, 9, 100, 2047, 8191):
+        raw = rng.integers(0, 256, size=n, dtype=np.uint8).tobytes()
+        body = literal_lzss0_body(raw)
+        assert len(body) == n + (n + 7) // 8
+        z = lz00_file(body, n, 0xC0FFEE + n)
+        outs, olen, cons, st = oracle.decode_batch(A.FMT_LZ00, [z], [n])
+        assert st[0] == A.OK and outs[0] == raw and cons[0] == len(z)
 
 
 def test_oracle_unsupported_subtypes(oracle):

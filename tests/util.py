@@ -122,3 +122,55 @@ def rom_like_image(oracle, rng, fmt, assets):
         starts.append(len(image))
         image += c + rng.integers(0, 256, size=int(rng.integers(10, 400)), dtype=np.uint8).tobytes()
     return bytes(image), starts
+
+
+def lz00_stream(key, count):
+    """LZ00's keystream (LZ00.cs:112-139): the key steps BEFORE every byte through the shift / subtract ladder of
+    GenerateNextKey, restated here literally; byte i of the body is XORed with the i-th value."""
+    out, M = bytearray(), 0xFFFFFFFF
+    for _ in range(count):
+        x = ((((((((key << 1) + key) << 5) - key) << 5) + key) << 7) - key) & M
+        x = ((x << 6) - x) & M
+        x = ((x << 4) - x) & M
+        key = ((x << 2) - x + 12345) & M
+        t = (key >> 16) & 0x7FFF
+        out.append((((t << 8) - t) >> 15) & 0xFF)
+    return bytes(out)
+
+
+def lz00_stream_fast(key, count):
+    """lz00_stream for long bodies: the ladder is the affine map K' = 1103515245 K + 12345 (mod 2**32), so the keys of block
+    j + 1 of 256 bytes are the 256-step map of block j's; the first block comes from lz00_stream's ladder."""
+    if count == 0:
+        return b""
+    M = 0xFFFFFFFF
+    first, keys = [], key
+    for _ in range(min(count, 256)):
+        keys = (1103515245 * keys + 12345) & M
+        first.append(keys)
+    a, c = 1, 0
+    for _ in range(256):
+        a, c = (1103515245 * a) & M, (1103515245 * c + 12345) & M
+    blocks = [np.array(first, dtype=np.uint64)]
+    for _ in range((count + 255) // 256 - 1):
+        blocks.append((blocks[-1] * np.uint64(a) + np.uint64(c)) & np.uint64(M))
+    k = np.concatenate(blocks)[:count]
+    t = (k >> np.uint64(16)) & np.uint64(0x7FFF)
+    return (((t << np.uint64(8)) - t) >> np.uint64(15)).astype(np.uint8).tobytes()
+
+
+def xor_bytes(a, b):
+    return (np.frombuffer(a, dtype=np.uint8) ^ np.frombuffer(b, dtype=np.uint8)).tobytes()
+
+
+def literal_lzss0_body(raw):
+    """An LZSS body of literals only: a 0xFF flag byte in front of every 8 bytes (flag bit 1 = literal).  Its length is any
+    value except 1 mod 9, and every byte of it reaches the output, so a wrong byte anywhere in it shows in the result."""
+    return b"".join(b"\xff" + raw[i:i + 8] for i in range(0, len(raw), 8))
+
+
+def lz00_file(body, raw_size, key):
+    """An LZ00 file (LZ00.cs:83-110) around an Lzss0 body: the 64-byte header, then the body under the keystream of `key`."""
+    le = lambda v: int(v).to_bytes(4, "little")
+    head = b"LZ00" + le(64 + len(body)) + bytes(8) + b"Temp.dat" + bytes(24) + le(raw_size) + le(key) + bytes(8)
+    return head + xor_bytes(body, lz00_stream_fast(key, len(body)))

@@ -7,11 +7,13 @@ with BatchCodec.decode_device, timed with CUDA events on the launching stream:
   (c) Level5: headerless LZ10 bodies behind the 4-byte Level5 word;
   (d) LZ77 ChunkLZ10 with 4 KiB chunks: 16 times as many (smaller) sub-streams, plus the call's one host read of the chunk
       count.  Files whose chunk ends do not fit u16 are refused by the encoder; only the files it accepts are kept;
-  (e) LZ00 (Lzss0 body under the keystream, a device copy of the source) against bare LZSS with the same properties.
+  (e) LZ00 (Lzss0 body under the keystream, lifted into per-stream scratch slots after one host read of their total) against
+      bare LZSS with the same properties.
 Every result is checked against the raw bytes.  The card's name, power limit and SM clock are read in the same process.
 Writes one JSON line to stdout and, with --out, to a file.
 
     python tools/wrapped_device_probe.py --out profiles/wrapped_device_probe.json
+    python tools/wrapped_device_probe.py --only e_lzss_lzss0,e_lz00     (some shapes only)
 """
 import argparse
 import json
@@ -30,6 +32,7 @@ def main():
     ap.add_argument("--files", type=int, default=16384)
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--only", default=None, help="comma-separated shape names (default: all)")
     args = ap.parse_args()
 
     import numpy as np
@@ -57,6 +60,8 @@ def main():
         ("e_lzss_lzss0", A.FMT_LZSS, A.make_opts(quality=8, lzss=lzss0)),
         ("e_lz00", A.FMT_LZ00, A.make_opts(quality=8, lz00_key=0x5EEDC0DE)),
     ]
+    if args.only:
+        shapes = [x for x in shapes if x[0] in args.only.split(",")]
     t = lambda a: torch.from_numpy(np.ascontiguousarray(a).astype(np.int64)).to(dev)
     for name, fmt, opts in shapes:
         comps, st = codec.encode_batch(fmt, raws, opts)
@@ -88,10 +93,11 @@ def main():
                      "decoded_gbps": round(m * size / (ms * 1e-3) / 1e9, 1)}
         del d_src, d_dst, comps
         torch.cuda.empty_cache()
-    a = res["a_lz10"]["decoded_gbps"]
     for k in ("b_gclz", "c_level5", "d_lz77_chunklz10_4k"):
-        res[k]["rate_vs_a"] = round(res[k]["decoded_gbps"] / a, 3)
-    res["e_lz00"]["rate_vs_bare_lzss"] = round(res["e_lz00"]["decoded_gbps"] / res["e_lzss_lzss0"]["decoded_gbps"], 3)
+        if k in res and "a_lz10" in res:
+            res[k]["rate_vs_a"] = round(res[k]["decoded_gbps"] / res["a_lz10"]["decoded_gbps"], 3)
+    if "e_lz00" in res and "e_lzss_lzss0" in res:
+        res["e_lz00"]["rate_vs_bare_lzss"] = round(res["e_lz00"]["decoded_gbps"] / res["e_lzss_lzss0"]["decoded_gbps"], 3)
     res["card_after"] = card()
     line = json.dumps(res)
     print(line)
