@@ -16,7 +16,7 @@ EXPORTS = [
     "aurora_lz_props_window", "aurora_lz_props_bits", "aurora_codec_opts_init", "aurora_decoded_size_batch",
     "aurora_is_match_batch", "aurora_scan_offsets", "aurora_decode_batch", "aurora_encode_bound", "aurora_encode_batch",
     "aurora_decode_batch_device", "aurora_encode_batch_device", "aurora_decoded_size_batch_device", "aurora_is_match_batch_device",
-    "aurora_scan_offsets_device", "aurora_kernel_launch_count",
+    "aurora_scan_offsets_device", "aurora_scan_decode_device", "aurora_kernel_launch_count",
 ]
 
 _LIB = None
@@ -76,6 +76,8 @@ def load():
     L.aurora_is_match_batch_device.argtypes = [vp, i32, i32, opts, sz, vp, vp, vp, vp, vp]
     L.aurora_scan_offsets_device.restype = i32
     L.aurora_scan_offsets_device.argtypes = [vp, i32, i32, opts, vp, u64, vp, vp]
+    L.aurora_scan_decode_device.restype = i32
+    L.aurora_scan_decode_device.argtypes = [vp, i32, i32, opts, vp, u64, u64, u64, sz, vp, vp, vp, vp, u64, vp, vp, vp, vp]
     L.aurora_kernel_launch_count.restype = u64
     L.aurora_kernel_launch_count.argtypes = [vp]
     _LIB = L

@@ -207,6 +207,55 @@ class BatchCodec:
                                                 d_match.data_ptr(), stream)
         self._check(rc, "aurora_scan_offsets_device")
 
+    def scan_decode_device(self, fmt, d_image, opts=None, max_size=1 << 26, begin=0, device=0, stream=None):
+        """The CLI's `-scan` on a device image: every stream the offset walk from `begin` finds (IsMatch at a position, decode
+        there with capacity `max_size`, resume after the consumed bytes of an OK stream, else one byte on), decoded on the
+        device.  -> (d_start, d_consumed, d_out_len, d_dst, d_dst_off) on the image's device: int64 descriptors in walk order
+        and the decoded bytes packed at 16-byte aligned offsets.  d_image must start 16-byte aligned.
+
+        Calls aurora_scan_decode_device until the walk reaches the end, with output pieces of at least max_size bytes, and
+        concatenates the pieces.  Each call reads back from the device, so this returns when the work on `stream` is done."""
+        import torch
+        opts = opts or _abi.make_opts()
+        dev = d_image.device
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+        if not stream:
+            # handle 0, torch's legacy default stream, means the library's own stream to the C ABI: finish the work that
+            # wrote the image first (each call returns after its own work, so its results are ready when it returns)
+            torch.cuda.current_stream(dev).synchronize()
+        ts = torch.cuda.ExternalStream(stream, device=dev)
+        length = d_image.numel()
+        entries = 1 << 16
+        piece = (max(int(max_size), 1 << 26) + 15) & ~15
+        found, nxt = C.c_uint64(0), C.c_uint64(0)
+        parts, dsts, base, pos = [], [], 0, begin
+        with torch.cuda.stream(ts):
+            while True:
+                d = [torch.empty(entries, dtype=torch.int64, device=dev) for _ in range(4)]   # start, consumed, out_len, dst_off
+                d_dst = torch.empty(piece, dtype=torch.uint8, device=dev)
+                rc = self._L.aurora_scan_decode_device(
+                    self._ctx, device, fmt, C.byref(opts), d_image.data_ptr(), length, pos, max_size, entries, d[0].data_ptr(),
+                    d[1].data_ptr(), d[2].data_ptr(), d_dst.data_ptr(), piece, d[3].data_ptr(), C.byref(found), C.byref(nxt),
+                    stream)
+                self._check(rc, "aurora_scan_decode_device")
+                k = found.value
+                if k:
+                    used = (int(d[3][k - 1]) + int(d[2][k - 1]) + 15) & ~15
+                    parts.append((d[0][:k], d[1][:k], d[2][:k], d[3][:k] + base))
+                    dsts.append(d_dst[:used])
+                    base += used
+                if nxt.value >= length:
+                    break
+                if k == 0:
+                    raise AuroraError(f"aurora_scan_decode_device: no progress at offset {nxt.value}")
+                pos = nxt.value
+            if not parts:
+                e = torch.empty(0, dtype=torch.int64, device=dev)
+                return e, e.clone(), e.clone(), torch.empty(0, dtype=torch.uint8, device=dev), e.clone()
+            cat = [torch.cat([p[i] for p in parts]) for i in range(4)]
+            return cat[0], cat[1], cat[2], torch.cat(dsts), cat[3]
+
     def decode_device_sized(self, fmt, d_src, d_off, d_len, opts=None, size_scan=True, max_size=1 << 30, device=0, stream=None):
         """Decode device streams whose decoded sizes the caller does not know.
         -> (d_dst, d_dst_off, d_cap, d_out_len, d_consumed, d_status), all on `stream` (None: torch's current stream).

@@ -96,6 +96,7 @@ struct DeviceCtx {
     DevBuf src, dst, desc, ticket, scratch, order;
     DevBuf size_scan;   // aurora_decoded_size_batch_device with a size scan: n zeroed offsets / capacities, then n consumed
     WrapScratch wrap;   // aurora_decode_batch_device of the wrapper formats
+    ScanScratch scan;   // aurora_scan_decode_device
     HostBuf hdesc;
     std::mutex mu;   // one batch at a time per device
 };
@@ -761,6 +762,7 @@ void aurora_shutdown(aurora_ctx* ctx) {
         d->order.release();
         d->size_scan.release();
         d->wrap.release();
+        d->scan.release();
         d->hdesc.release();
         for (cudaEvent_t e : d->ev_in) cudaEventDestroy(e);
         for (cudaEvent_t e : d->ev_k) cudaEventDestroy(e);
@@ -1096,6 +1098,52 @@ int aurora_scan_offsets_device(aurora_ctx* ctx, int device, int format, const au
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
     CU_TRY(ctx, launch_scan(d_image, len, d_match, format, st));
     ctx->launches++;
+    return AURORA_OK;
+}
+
+int aurora_scan_decode_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts, const uint8_t* d_image,
+                              uint64_t len, uint64_t begin, uint64_t max_size, size_t max_found, uint64_t* d_start, uint64_t* d_consumed,
+                              uint64_t* d_out_len, uint8_t* d_dst_base, uint64_t dst_bytes, uint64_t* d_dst_off, uint64_t* found,
+                              uint64_t* next, void* stream) {
+    if (!ctx || device < 0 || device >= int(ctx->devs.size()) || !found || !next) return AURORA_INVALID_ARGUMENT;
+    if (!scan_query_format(format)) {
+        ctx->set_error("aurora_scan_decode_device: this format has no offset scan (the formats aurora_scan_offsets takes)");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    if (begin > len || max_size == 0 || max_size > 0xFFFFFFFFull || len > 0xFFFFFFFF00ull) {
+        ctx->set_error("aurora_scan_decode_device: begin past len, or max_size outside 1 .. 0xFFFFFFFF, or len above 0xFFFFFFFF00");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    if (len == 0 || begin == len) {   // an empty walk reads nothing
+        *found = 0;
+        *next = len;
+        return AURORA_OK;
+    }
+    if (!d_image || !d_start || !d_consumed || !d_out_len || !d_dst_base || !d_dst_off) {
+        ctx->set_error("aurora_scan_decode_device: null argument");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    if ((reinterpret_cast<uintptr_t>(d_image) & 15) != 0) {
+        ctx->set_error("aurora_scan_decode_device: d_image must be 16-byte aligned");
+        return AURORA_INVALID_ARGUMENT;
+    }
+    DecodeParams P{};
+    if (fill_decode_params(P, format, opts) != AURORA_OK) {   // every decode reports NOT_SUPPORTED: the walk has no entry
+        *found = 0;
+        *next = len;
+        return AURORA_OK;
+    }
+    DeviceCtx* d = ctx->devs[device];
+    std::lock_guard<std::mutex> guard(d->mu);
+    CU_TRY(ctx, cudaSetDevice(d->dev));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+    CU_TRY(ctx, d->ticket.reserve(256));
+    uint64_t launched = 0;
+    const cudaError_t e = aurora::scan_decode_rounds(format, opts, d_image, len, begin, max_size, max_found, d_start, d_consumed, d_out_len,
+                                                     d_dst_base, dst_bytes, d_dst_off, found, next, d->scan,
+                                                     static_cast<unsigned int*>(d->ticket.p), d->sm_count, st, &launched);
+    ctx->launches += launched;
+    CU_TRY(ctx, e);
     return AURORA_OK;
 }
 

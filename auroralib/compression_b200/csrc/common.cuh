@@ -161,6 +161,29 @@ cudaError_t launch_is_match(const uint8_t* src_base, const uint64_t* src_off, co
 cudaError_t launch_decoded_size(const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len, uint64_t* size,
                                 int32_t* status, uint32_t n, int format, int byte_order, cudaStream_t st);
 cudaError_t launch_size_scan_status(int32_t* status, uint32_t n, cudaStream_t st);
+// the hits of the window [*d_base, *d_base + items) of an image (IsMatch to the image's end, is_match_one): the first `keep`
+// offsets relative to *d_base, ascending, into rel, the number of all of them into *d_count.  A cub::DeviceSelect::If (two
+// kernels); temp == nullptr only sets *temp_bytes.  ismatch.cu
+cudaError_t launch_window_hits(const uint8_t* image, uint64_t len, const uint64_t* d_base, uint32_t items, int format, uint32_t* rel,
+                               uint32_t keep, uint32_t* d_count, void* temp, size_t* temp_bytes, cudaStream_t st);
+#ifdef __CUDACC__
+// per-device scratch of aurora_scan_decode_device (scan_decode.cu): the walk state, the round's per-hit arrays, the select's
+// and the scan's temporary storage, and the slots the round's hits are decoded into
+struct ScanScratch {
+    DevBuf state, hits, temp, slots;
+    void release() {
+        state.release();
+        hits.release();
+        temp.release();
+        slots.release();
+    }
+};
+// the rounds of aurora_scan_decode_device on `st` (arguments checked by the caller); counts its kernel launches into *launches
+cudaError_t scan_decode_rounds(int format, const aurora_codec_opts* opts, const uint8_t* d_image, uint64_t len, uint64_t begin,
+                               uint64_t max_size, uint64_t max_found, uint64_t* d_start, uint64_t* d_consumed, uint64_t* d_out_len,
+                               uint8_t* d_dst_base, uint64_t dst_bytes, uint64_t* d_dst_off, uint64_t* found, uint64_t* next,
+                               ScanScratch& scr, unsigned int* ticket, int sm_count, cudaStream_t st, uint64_t* launches);
+#endif
 
 #ifdef __CUDACC__
 // ------------------------------------------------------------------------------------------------

@@ -8,6 +8,7 @@
 // the end) makes IsMatch false here, like the oracle.
 // core_decoded_size (size_peek.cuh) and decoded_size_one are __host__ __device__ too: aurora_decoded_size_batch runs them on the host,
 // aurora_decoded_size_batch_device in decoded_size_kernel, one thread per stream.
+// launch_window_hits (at the end) selects the hits of one window of aurora_scan_decode_device's walk with the same rule.
 #include "api_internal.hpp"
 #include "common.cuh"
 #include "size_peek.cuh"
@@ -266,6 +267,46 @@ cudaError_t launch_decoded_size(const uint8_t* src_base, const uint64_t* src_off
 cudaError_t launch_size_scan_status(int32_t* status, uint32_t n, cudaStream_t st) {
     size_scan_status_kernel<<<(n + 255) / 256, 256, 0, st>>>(status, n);
     return cudaGetLastError();
+}
+
+}  // namespace aurora
+
+// ---- the hits of one window of the offset walk (aurora_scan_decode_device, scan_decode.cu)
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
+#include <thrust/iterator/tabulate_output_iterator.h>
+
+namespace aurora {
+
+namespace {
+
+struct WindowHit {   // IsMatch of the stream at *base + i, to the end of the image (*base: the round's walk position)
+    const uint8_t* image;
+    uint64_t len;
+    const uint64_t* base;
+    int format;
+    __device__ bool operator()(uint32_t i) const {
+        const uint64_t q = *base + i;
+        return q < len && is_match_one(image + q, len - q, format) > 0;
+    }
+};
+
+struct KeepFirst {   // the select's output: only the first `keep` hits are stored, all of them are counted
+    uint32_t* out;
+    uint32_t keep;
+    template <typename I>
+    __device__ void operator()(I idx, uint32_t v) const {
+        if (uint64_t(idx) < keep) out[idx] = v;
+    }
+};
+
+}  // namespace
+
+cudaError_t launch_window_hits(const uint8_t* image, uint64_t len, const uint64_t* d_base, uint32_t items, int format, uint32_t* rel,
+                               uint32_t keep, uint32_t* d_count, void* temp, size_t* temp_bytes, cudaStream_t st) {
+    return cub::DeviceSelect::If(temp, *temp_bytes, thrust::counting_iterator<uint32_t>(0),
+                                 thrust::make_tabulate_output_iterator(KeepFirst{rel, keep}), d_count, int64_t(items),
+                                 WindowHit{image, len, d_base, format}, st);
 }
 
 }  // namespace aurora

@@ -234,8 +234,8 @@ int aurora_encode_batch(aurora_ctx* ctx, int format, const aurora_codec_opts* op
  * sub-stream (encode: core piece) descriptors and results, LZ77's chunk counts and their scan, and LZ00's keystream-free
  * bodies with their slot sizes and scan (decode).  A wrapped encode also uses the device's encoder scratch.
  * None of these calls synchronises with the host, reads a result on the host or copies the source to or from the host,
- * with three exceptions: aurora_decode_batch_device of LZ77 and of LZ00, and aurora_encode_batch_device of LZ77 with
- * opts.lz77_type 0xF7 (below).
+ * with four exceptions: aurora_decode_batch_device of LZ77 and of LZ00, aurora_encode_batch_device of LZ77 with
+ * opts.lz77_type 0xF7, and aurora_scan_decode_device, which reads back once per round (below).
  *
  * aurora_decode_batch_device of the wrapper formats: out_len, consumed, status and the decoded bytes in
  * [dst_off[i], dst_off[i] + min(out_len[i], dst_cap[i])) are those aurora_decode_batch gives for the same streams, options
@@ -315,6 +315,44 @@ int aurora_is_match_batch_device(aurora_ctx* ctx, int device, int format, const 
  * most 0xFFFFFFFF00.  The formats aurora_scan_offsets takes: the core formats except LZ4 block, Snappy block and BLZ. */
 int aurora_scan_offsets_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts,
                                const uint8_t* d_image, uint64_t len, uint8_t* d_match, void* stream);
+
+/*
+ * The CLI's `-scan` (ScanDecompressCommand.cs:23-39) on a device image: every stream the offset walk finds, decoded into device
+ * memory.  For a format f, options opts, the image I of len bytes, a start `begin` and a capacity max_size, the walk W(begin) is
+ *     i = begin
+ *     while i < len:
+ *         if aurora_scan_offsets(f, I)[i] and aurora_decode_batch(f, [I[i .. len)], cap = [max_size], opts) is AURORA_OK:
+ *             emit (start = i, consumed, out_len, the out_len decoded bytes);  i += max(consumed, 1)
+ *         else:
+ *             i += 1
+ * so a stream larger than max_size is not an entry (the decode reports DST_TOO_SMALL there and the walk steps by one byte).
+ * Entries k = 0 .. *found - 1 of W(begin) are written in walk order to d_start[k], d_consumed[k], d_out_len[k] and the bytes
+ * [d_dst_base + d_dst_off[k], + d_out_len[k]); d_dst_off[0] = 0 and d_dst_off[k + 1] = d_dst_off[k] + out_len[k] rounded up to
+ * 16.  The call stops before the first entry that would be the max_found + 1-th or whose bytes would pass dst_bytes; *next is
+ * that entry's start, or len when the walk reached the end, and W(*next) continues the walk exactly (no state between calls).
+ * Formats: those aurora_scan_offsets takes (the core formats except LZ4 block, Snappy block and BLZ); the others are
+ * AURORA_INVALID_ARGUMENT.  So are begin > len, max_size 0 or above 0xFFFFFFFF, len above 0xFFFFFFFF00, null pointers and a
+ * d_image that is not 16-byte aligned; d_image must be readable up to len rounded up to 16, as d_src_base of
+ * aurora_decode_batch_device.  len == 0 or begin == len: AURORA_OK, *found = 0, *next = len.  A rejected or empty call
+ * launches nothing; so does a call with LZSS properties the decoder does not take (every decode reports AURORA_NOT_SUPPORTED, so
+ * the walk has no entry: AURORA_OK, *found = 0, *next = len).  found and next are host pointers, the rest device memory on `device`.  Nothing is written outside the
+ * entries' bytes and descriptors, and the image is never modified.
+ * The walk runs in rounds from its position p.  Per round: the hits of a window [p, p + W) (a cub::DeviceSelect::If with the
+ * IsMatch rule, 2 kernels; W adapts between 128 KiB and 1 GiB, at most 65 536 hits are kept), ONE HOST READ (the walk
+ * position and the window's hit count), and when the window has hits: a capacity per hit (1 kernel; the byte-LZ formats first
+ * run the decode kernel's size-only parse, +1 kernel, and turn its lengths into capacities, +1), slots for them by an
+ * exclusive scan (2 kernels) cut at a budget of max(max_size, 256 MiB) decoded bytes (1), the decode kernel into the slots
+ * (1), one warp that follows the walk and writes the descriptors (1), and a copy of the entries' bytes to d_dst_base (1):
+ * 9 kernels per round (11 for the byte-LZ formats), 3 for a window without hits, plus a last window test that finds the
+ * walk's end.  So THIS CALL READS BACK and returns after its work on `stream` is done (like LZ77 and LZ00 above).  Per-device
+ * scratch: the walk state, the round's per-hit arrays (about 4 MiB), CUB's temporary storage, the slots (the budget), and the
+ * device's work counter; the stream-ordering rule above applies.
+ */
+int aurora_scan_decode_device(aurora_ctx* ctx, int device, int format, const aurora_codec_opts* opts,
+                              const uint8_t* d_image, uint64_t len, uint64_t begin, uint64_t max_size,
+                              size_t max_found, uint64_t* d_start, uint64_t* d_consumed, uint64_t* d_out_len,
+                              uint8_t* d_dst_base, uint64_t dst_bytes, uint64_t* d_dst_off,
+                              uint64_t* found, uint64_t* next, void* stream);
 
 /* Number of kernels this library has launched since aurora_init (all devices). */
 uint64_t aurora_kernel_launch_count(const aurora_ctx* ctx);
