@@ -146,7 +146,8 @@ int ceil_log2(long long x) {
 
 namespace aurora {
 
-cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
+// whether launch_encode runs the lane-per-position search (else the sequential replay)
+bool encode_par_chosen(const EncodeParams& p) {
     // Flag-byte formats (LZ10 / BLZ, LZ11 / LZ40 / LZ60, Yaz0 / Yaz1, LZSS, MIO0, Yay0, LZHudson, SMSR00): the window search with one lane per
     // position and shared-memory tables (encode_lz_par.cu).  Both encoders write the reference's bytes; which one runs is a
     // speed decision.  Measured on the C2 corpus (64 KiB streams, GB/s raw in, parallel / sequential replay): quality 8 LZ10
@@ -161,7 +162,24 @@ cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
     }();
     const int want = p.finder_choice ? p.finder_choice : forced;
     const bool par_default = p.max_chain <= 128 || p.max_length <= 32;
-    if (encode_lz_par_supported(p) && (want == 1 || (want == 0 && par_default))) return launch_encode_lz_par(p, warps / 48, st);
+    return encode_lz_par_supported(p) && (want == 1 || (want == 0 && par_default));
+}
+
+int encode_launch_warps(const EncodeParams& p, int sm_count) {
+    const bool par = encode_par_chosen(p);
+    const int per_block = par ? encode_lz_par_block_warps(p) : kEncWarpsPerBlock;
+    const long long most = par ? sm_count : encode_resident_warps(sm_count) / kEncWarpsPerBlock;
+    const long long needed = ((long long)p.n + per_block - 1) / per_block;
+    return int(std::max(1LL, std::min(most, needed))) * per_block;
+}
+
+// A position's link lives in chain slot position & (2^chain_bits - 1), so a table of 2^b slots with 2^b >= `longest` holds
+// every link of a stream in a slot of its own: the walk, and the bytes, are those of the full table.  (The result is at
+// least 12 whenever chain_bits is, so encode_lz_par_supported still picks the same finder.)
+int encode_chain_bits(int chain_bits, uint64_t longest) { return std::min(chain_bits, std::max(12, ceil_log2((long long)longest))); }
+
+cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st) {
+    if (encode_par_chosen(p)) return launch_encode_lz_par(p, warps / encode_lz_par_block_warps(p), st);
     if (is_flaglz(p.format) || p.format == AURORA_FMT_BLZ) return launch_encode_lz(p, warps, st);   // BLZ: LZ10's layout
     return launch_encode_bytelz(p, warps, st);
 }
@@ -593,7 +611,10 @@ int fill_encode_params(EncodeParams& p, int format, const aurora_codec_opts* o) 
         windows_bits = std::max(windows_bits, mwb);
         p.max_distance = std::max(p.max_distance, 1 << mwb);
     }
-    p.chain_bits = std::min(17 + isqrt2q(q), windows_bits);
+    // (at least 4 slots: finder_reset clears the chain table in 16-byte stores, and the small-match table behind it must stay
+    //  16-byte aligned.  A walk never reads a slot of a position more than 2^windows_bits back, so the wider table of LZSS with
+    //  windows_bits 1 holds the same links.)
+    p.chain_bits = std::max(2, std::min(17 + isqrt2q(q), windows_bits));
     p.min_length = lz.min_length;
     p.max_length = lz.max_length;
     p.min_distance = lz.min_distance;
@@ -625,7 +646,9 @@ int encode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
     const Layout D = plan_layout(dst_off, dst_cap, b, e);
     uint64_t max_len = 0;
     for (size_t i = b; i < e; i++) max_len = std::max(max_len, src_len[i]);
-    const int warps = encode_resident_warps(d->sm_count);
+    P.n = uint32_t(n);
+    P.chain_bits = encode_chain_bits(P.chain_bits, max_len);
+    const int warps = encode_launch_warps(P, d->sm_count);
     P.scratch_per_warp = encode_scratch_per_warp(format, P.hash_bits, P.chain_bits, max_len);
     CU_TRY(ctx, d->scratch.reserve(size_t(warps) * P.scratch_per_warp));
     CU_TRY(ctx, d->src.reserve(S.bytes + 16));
@@ -670,7 +693,6 @@ int encode_shard(aurora_ctx* ctx, DeviceCtx* d, int format, const aurora_codec_o
     P.out_len = dv + 4 * n;
     P.status = reinterpret_cast<int32_t*>(dv + 5 * n);
     P.ticket = static_cast<unsigned int*>(d->ticket.p);
-    P.n = uint32_t(n);
     CU_TRY(ctx, launch_encode(P, warps, st));
     ctx->launches++;
     if (format == AURORA_FMT_BLZ) {   // the codes are stored in the order the backwards decoder reads them
@@ -1273,7 +1295,10 @@ int aurora_encode_batch_device(aurora_ctx* ctx, int device, int format, const au
         const uint64_t* hl = static_cast<const uint64_t*>(d->hdesc.p);
         for (size_t i = 0; i < n; i++) max_len = std::max(max_len, hl[i]);
     }
-    const int warps = encode_resident_warps(d->sm_count);
+    // every window lies inside the src_total source bytes: that bounds the longest stream without reading the lengths back
+    P.n = uint32_t(n);
+    P.chain_bits = encode_chain_bits(P.chain_bits, max_len ? max_len : src_total);
+    const int warps = encode_launch_warps(P, d->sm_count);
     P.scratch_per_warp = encode_scratch_per_warp(format, P.hash_bits, P.chain_bits, max_len);
     CU_TRY(ctx, d->scratch.reserve(size_t(warps) * P.scratch_per_warp));
     CU_TRY(ctx, d->ticket.reserve(256));
@@ -1289,7 +1314,6 @@ int aurora_encode_batch_device(aurora_ctx* ctx, int device, int format, const au
     P.out_len = d_out_len;
     P.status = d_status;
     P.ticket = static_cast<unsigned int*>(d->ticket.p);
-    P.n = uint32_t(n);
     CU_TRY(ctx, launch_encode(P, warps, st));
     ctx->launches++;
     return AURORA_OK;

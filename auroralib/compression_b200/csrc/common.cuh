@@ -75,6 +75,8 @@ __host__ __device__ inline uint64_t core_encode_bound(int format, uint64_t raw_l
         case AURORA_FMT_SNAPPY_BLOCK: return raw_len + raw_len / 60 + 32 + 16 * (raw_len / 0x10000 + 1);
         // LZO: a far 3-byte match costs 3 bytes and splits the literal run around it (4 literals + 1 match = 7 bytes in, 8 out)
         case AURORA_FMT_LZO: return raw_len + raw_len / 6 + 64;
+        // LZSS with min_length 1: a two-byte token for each input byte, and a flag byte per 8 tokens
+        case AURORA_FMT_LZSS: return 2 * raw_len + raw_len / 8 + 64;
         default: return raw_len + raw_len / 8 + 64;
     }
 }
@@ -134,6 +136,11 @@ cudaError_t launch_decode(const DecodeParams& p, int sm_count, cudaStream_t st);
 // the same for the encoders: CompressionSettings + LzProperties -> finder parameters (AURORA_OK, or the batch's argument
 // error), and the encode kernel of p.format (the lane-per-position finder or the sequential replay)
 int fill_encode_params(EncodeParams& p, int format, const aurora_codec_opts* o);
+// The warps launch_encode starts for the p.n streams of a batch: one per stream, up to the resident warps of the encoder it
+// picks.  Each of them owns one slice of p.scratch, so the scratch reservation takes this count as well.
+int encode_launch_warps(const EncodeParams& p, int sm_count);
+// The sequential replay's chain table for streams of at most `longest` bytes (see api.cu)
+int encode_chain_bits(int chain_bits, uint64_t longest);
 cudaError_t launch_encode(const EncodeParams& p, int warps, cudaStream_t st);
 // kernel launchers (one translation unit per kernel family); all return cudaGetLastError()
 cudaError_t launch_decode_flaglz(const DecodeParams& p, int sm_count, cudaStream_t st);
@@ -142,10 +149,12 @@ cudaError_t launch_decode_blz(const DecodeParams& p, int sm_count, cudaStream_t 
 // in-place byte reversal of bytes [0, min(len[i], cap[i])) of every stream (BLZ encode; decode_blz.cu); cap may be null
 cudaError_t launch_reverse_bytes(uint8_t* base, const uint64_t* d_off, const uint64_t* d_len, const uint64_t* d_cap, uint32_t n,
                                  cudaStream_t st);
+constexpr int kEncWarpsPerBlock = 8;   // the sequential replay (encode_lz.cu, encode_bytelz.cu); `warps`: a multiple of it
 cudaError_t launch_encode_lz(const EncodeParams& p, int warps, cudaStream_t st);
 cudaError_t launch_encode_bytelz(const EncodeParams& p, int warps, cudaStream_t st);
 bool encode_lz_par_supported(const EncodeParams& p);   // encode_lz_par.cu: one lane per window position
-cudaError_t launch_encode_lz_par(const EncodeParams& p, int sm_count, cudaStream_t st);
+int encode_lz_par_block_warps(const EncodeParams& p);  // its warps per block (one block per SM)
+cudaError_t launch_encode_lz_par(const EncodeParams& p, int blocks, cudaStream_t st);
 size_t encode_scratch_per_warp(int format, int hash_bits, int chain_bits, uint64_t max_src_len);
 int encode_resident_warps(int sm_count);
 cudaError_t launch_size_order(const uint64_t* d_size, uint32_t n, uint32_t* d_hist64, uint32_t* d_order, cudaStream_t st);

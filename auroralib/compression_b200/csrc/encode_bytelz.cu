@@ -15,8 +15,6 @@ namespace aurora {
 
 namespace {
 
-constexpr int kEncWarpsPerBlock = 8;
-
 // bounded sequential output; lane 0 stores single bytes, runs are copied by the whole warp
 struct Out {
     uint8_t* out;
@@ -407,10 +405,7 @@ cudaError_t launch_encode_bytelz(const EncodeParams& p, int warps, cudaStream_t 
         if (e != cudaSuccess) return e;
         table_ready[dev & 63] = true;
     }
-    int blocks = (warps + kEncWarpsPerBlock - 1) / kEncWarpsPerBlock;
-    const int needed = int((p.n + kEncWarpsPerBlock - 1) / kEncWarpsPerBlock);
-    if (needed < blocks) blocks = needed > 0 ? needed : 1;
-    encode_bytelz_kernel<<<blocks, kEncWarpsPerBlock * 32, 0, st>>>(p);
+    encode_bytelz_kernel<<<warps / kEncWarpsPerBlock, kEncWarpsPerBlock * 32, 0, st>>>(p);
     return cudaGetLastError();
 }
 

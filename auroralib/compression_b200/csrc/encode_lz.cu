@@ -30,8 +30,6 @@ namespace aurora {
 
 namespace {
 
-constexpr int kEncWarpsPerBlock = 8;
-
 enum EncKind { E_LZ10 = 0, E_LZ11 = 1, E_YAZ0 = 2, E_LZSS = 3, E_MIO0 = 4, E_YAY0 = 5 };
 
 __device__ __forceinline__ void put_u32(Writer& w, uint32_t v, bool big) {
@@ -279,10 +277,7 @@ __global__ void __launch_bounds__(kEncWarpsPerBlock * 32) encode_lz_kernel(const
 
 template <int K>
 cudaError_t launch(const EncodeParams& p, int warps, cudaStream_t st) {
-    int blocks = (warps + kEncWarpsPerBlock - 1) / kEncWarpsPerBlock;
-    const int needed = int((p.n + kEncWarpsPerBlock - 1) / kEncWarpsPerBlock);
-    if (needed < blocks) blocks = needed > 0 ? needed : 1;
-    encode_lz_kernel<K><<<blocks, kEncWarpsPerBlock * 32, 0, st>>>(p);
+    encode_lz_kernel<K><<<warps / kEncWarpsPerBlock, kEncWarpsPerBlock * 32, 0, st>>>(p);
     return cudaGetLastError();
 }
 

@@ -828,7 +828,7 @@ __global__ void __launch_bounds__(kParWarps<M> * 32, 1) encode_lz_par_kernel(con
 }
 
 template <int K, bool M>
-cudaError_t launch_par_m(const EncodeParams& p, int sm_count, cudaStream_t st) {
+cudaError_t launch_par_m(const EncodeParams& p, int blocks, cudaStream_t st) {
     const size_t smem = size_t(kParWarps<M>) * kTablesPerWarp<M>;
     static bool configured[64] = {};
     int dev = 0;
@@ -838,17 +838,14 @@ cudaError_t launch_par_m(const EncodeParams& p, int sm_count, cudaStream_t st) {
         if (e != cudaSuccess) return e;
         configured[dev & 63] = true;
     }
-    int blocks = sm_count;
-    const int needed = int((p.n + kParWarps<M> - 1) / kParWarps<M>);
-    if (needed < blocks) blocks = needed > 0 ? needed : 1;
     encode_lz_par_kernel<K, M><<<blocks, kParWarps<M> * 32, smem, st>>>(p);
     return cudaGetLastError();
 }
 
 // the small-match table only exists at qualities >= 10 for formats whose shortest match is below 4 bytes (finder.cuh has_min)
 template <int K>
-cudaError_t launch_par(const EncodeParams& p, int sm_count, cudaStream_t st) {
-    return (p.use_min_table && p.min_length < 4) ? launch_par_m<K, true>(p, sm_count, st) : launch_par_m<K, false>(p, sm_count, st);
+cudaError_t launch_par(const EncodeParams& p, int blocks, cudaStream_t st) {
+    return (p.use_min_table && p.min_length < 4) ? launch_par_m<K, true>(p, blocks, st) : launch_par_m<K, false>(p, blocks, st);
 }
 
 }  // namespace
@@ -859,24 +856,30 @@ bool encode_lz_par_supported(const EncodeParams& p) {
                      p.format == AURORA_FMT_LZSS || p.format == AURORA_FMT_MIO0 || p.format == AURORA_FMT_YAY0 ||
                      p.format == AURORA_FMT_LZHUDSON || p.format == AURORA_FMT_SMSR00;
     const bool lz11 = p.format == AURORA_FMT_LZ11 || p.format == AURORA_FMT_LZ40 || p.format == AURORA_FMT_LZ60;   // any max_length
+    // (one-byte matches with the small-match table, LZSS with min_length 1 from quality 10 on, parse differently from the
+    //  reference here: the sequential replay writes its bytes)
     return (lz11 || (fmt && p.max_length <= kLook)) && p.hash_bits >= kBucketBits && p.hash_bits <= 24 && p.max_distance <= kWin && p.chain_bits >= 12 &&
-           p.min_length >= 1 && p.min_distance >= 1;
+           p.min_length >= 1 && p.min_distance >= 1 && !(p.use_min_table && p.min_length == 1);
 }
 
-cudaError_t launch_encode_lz_par(const EncodeParams& p, int sm_count, cudaStream_t st) {
+int encode_lz_par_block_warps(const EncodeParams& p) {
+    return (p.use_min_table && p.min_length < 4) ? kParWarps<true> : kParWarps<false>;
+}
+
+cudaError_t launch_encode_lz_par(const EncodeParams& p, int blocks, cudaStream_t st) {
     switch (p.format) {
         case AURORA_FMT_LZ10:
-        case AURORA_FMT_BLZ: return launch_par<P_LZ10>(p, sm_count, st);
+        case AURORA_FMT_BLZ: return launch_par<P_LZ10>(p, blocks, st);
         case AURORA_FMT_YAZ0:
-        case AURORA_FMT_YAZ1: return launch_par<P_YAZ0>(p, sm_count, st);
-        case AURORA_FMT_LZSS: return launch_par<P_LZSS>(p, sm_count, st);
-        case AURORA_FMT_MIO0: return launch_par<P_MIO0>(p, sm_count, st);
-        case AURORA_FMT_YAY0: return launch_par<P_YAY0>(p, sm_count, st);
+        case AURORA_FMT_YAZ1: return launch_par<P_YAZ0>(p, blocks, st);
+        case AURORA_FMT_LZSS: return launch_par<P_LZSS>(p, blocks, st);
+        case AURORA_FMT_MIO0: return launch_par<P_MIO0>(p, blocks, st);
+        case AURORA_FMT_YAY0: return launch_par<P_YAY0>(p, blocks, st);
         case AURORA_FMT_LZ11:
         case AURORA_FMT_LZ40:
-        case AURORA_FMT_LZ60: return launch_par<P_LZ11>(p, sm_count, st);
-        case AURORA_FMT_LZHUDSON: return launch_par<P_HUDSON>(p, sm_count, st);
-        case AURORA_FMT_SMSR00: return launch_par<P_SMSR>(p, sm_count, st);
+        case AURORA_FMT_LZ60: return launch_par<P_LZ11>(p, blocks, st);
+        case AURORA_FMT_LZHUDSON: return launch_par<P_HUDSON>(p, blocks, st);
+        case AURORA_FMT_SMSR00: return launch_par<P_SMSR>(p, blocks, st);
         default: return cudaErrorNotSupported;
     }
 }

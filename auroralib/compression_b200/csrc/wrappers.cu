@@ -1240,8 +1240,10 @@ int wrapped_encode_batch_device(int format, const aurora_codec_opts* opts, size_
         ++*launches;
     }
 
-    // the core encoder over every slot, as aurora_encode_batch_device runs it
-    const int warps = encode_resident_warps(sm_count);
+    // the core encoder over every slot, as aurora_encode_batch_device runs it (every slot lies inside the src_total bytes)
+    P.n = uint32_t(m);
+    P.chain_bits = encode_chain_bits(P.chain_bits, src_total);
+    const int warps = encode_launch_warps(P, sm_count);
     P.scratch_per_warp = encode_scratch_per_warp(e.core, P.hash_bits, P.chain_bits, 0);   // (no section staging: not MIO0 / Yay0)
     WRAP_ENC_TRY(enc_scratch.reserve(size_t(warps) * P.scratch_per_warp));
     WRAP_ENC_TRY(cudaMemsetAsync(ticket, 0, 64, st));
@@ -1256,7 +1258,6 @@ int wrapped_encode_batch_device(int format, const aurora_codec_opts* opts, size_
     P.out_len = A.out_len;
     P.status = A.status;
     P.ticket = ticket;
-    P.n = uint32_t(m);
     WRAP_ENC_TRY(launch_encode(P, warps, st));
     ++*launches;
     if (format == AURORA_FMT_LZ00) {   // the body the encoder just wrote goes under the keystream (bytes [16, out_len) of every piece)

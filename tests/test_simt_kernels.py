@@ -66,9 +66,14 @@ def _isqrt2q(q):
     return r
 
 
-def finder_params(fmt, quality, strategy=0, vram_mode=-1, lzss=None):
+def _ceil_log2(x):
+    return max(int(x) - 1, 0).bit_length()
+
+
+def finder_params(fmt, quality, strategy=0, vram_mode=-1, lzss=None, max_window_bits=0, longest=None):
     """CompressionSettings + LzProperties -> LzChainMatchFinder parameters (LzChainMatchFinder.cs:42-119), as api.cu
-    fill_encode_params derives them."""
+    fill_encode_params derives them; `longest` (the longest stream of the batch) sizes the sequential replay's chain table as
+    api.cu encode_chain_bits does."""
     if fmt == A.FMT_LZ10:
         lz = A.lz_props_window(0x1000, 18, 3, 0, 2 if vram_mode != 0 else 1)
     elif fmt == A.FMT_BLZ:
@@ -91,16 +96,22 @@ def finder_params(fmt, quality, strategy=0, vram_mode=-1, lzss=None):
         lz = lzss if lzss is not None else A.lz_props_bits(12, 4, 2)
     q = quality
     max_chain = q + 1 if q < 6 else 1 << (q - 5) if q >= 11 else (1 << (q >> 1)) | ((1 << (q >> 1)) >> (q & 1))
-    finder = [max_chain, 3 + q // 3, 15 + _isqrt2q(q), min(17 + _isqrt2q(q), max(1, lz.windows_bits)), lz.min_length, lz.max_length,
-              lz.min_distance, lz.max_distance, strategy & 1, 1 if q >= 10 else 0]
+    windows_bits, max_distance = max(1, lz.windows_bits), lz.max_distance
+    if max_window_bits:   # CompressionSettings.MaxWindowBits widens the window and the chain table
+        windows_bits, max_distance = max(windows_bits, max_window_bits), max(max_distance, 1 << max_window_bits)
+    chain_bits = max(2, min(17 + _isqrt2q(q), windows_bits))
+    if longest is not None:
+        chain_bits = min(chain_bits, max(12, _ceil_log2(longest)))
+    finder = [max_chain, 3 + q // 3, 15 + _isqrt2q(q), chain_bits, lz.min_length, lz.max_length,
+              lz.min_distance, max_distance, strategy & 1, 1 if q >= 10 else 0]
     return finder, [lz.windows_bits, lz.length_bits, lz.min_length, lz.max_distance, lz.windows_start]
 
 
 def simt_encode(lib, fmt, raws, quality, strategy=0, byte_order=A.ENDIAN_DEFAULT, vram_mode=-1, lzss=None, yaz0_alignment=0,
-                caps=None, skew=0, seq=False, lz4_block_size=0):
+                caps=None, skew=0, seq=False, lz4_block_size=0, max_window_bits=0):
     """One emulated warp encodes `raws`: the lane-per-position search, or (seq) the sequential replay of finder.cuh."""
     n = len(raws)
-    finder, lzp = finder_params(fmt, quality, strategy, vram_mode, lzss)
+    finder, lzp = finder_params(fmt, quality, strategy, vram_mode, lzss, max_window_bits, longest=max([len(r) for r in raws] + [0]))
     # sources back to back from an odd offset (any alignment is allowed), readable up to the next multiple of 16
     off, pos = [], skew
     for r in raws:
@@ -149,7 +160,7 @@ def simt_encode(lib, fmt, raws, quality, strategy=0, byte_order=A.ENDIAN_DEFAULT
 
 
 def _check(lib, oracle, fmt, raws, quality, **kw):
-    okw = {k: v for k, v in kw.items() if k not in ("skew", "seq")}
+    okw = {k: v for k, v in kw.items() if k not in ("skew", "seq", "caps")}
     ref, rst = oracle.encode_batch(fmt, raws, A.make_opts(quality=quality, **okw))
     if fmt == A.FMT_BLZ:
         # BLZ.cs:143-215: the kernel writes the token body of the REVERSED source (LZ10's layout, distance - 3); the host side

@@ -211,7 +211,8 @@ def _w_flag_single(fmt, program, rng, forms, lzss=None):
         elif fmt == A.FMT_LZSS:
             lz = lzss
             off = (lz.windows_start + pos - d) & (lz.max_distance - 1)
-            f.buf += ((off & 0xFF) | (off & 0xFF00) << lz.length_bits | (ln - lz.min_length) << 8).to_bytes(2, "little")
+            # (a u16 token: with windows_bits + length_bits > 16 the offset's top bits are dropped, as LZSS.cs writes them)
+            f.buf += (((off & 0xFF) | (off & 0xFF00) << lz.length_bits | (ln - lz.min_length) << 8) & 0xFFFF).to_bytes(2, "little")
         else:   # Yaz0 / Yaz1 / LZHudson
             if ln < 18:
                 f.buf += bytes([(ln - 2) << 4 | (d - 1) >> 8, (d - 1) & 0xFF])
@@ -618,7 +619,7 @@ def _flag_queue(b, rng):
         slots = set(int(x) for x in rng.choice(ITER_TOKENS, size=int(k), replace=False))
         for t in range(ITER_TOKENS):
             if t in slots:
-                b.match(b.rdist(), int(rng.integers(s.lo, min(s.hi, 18) + 1)))
+                b.match(b.rdist(), int(rng.integers(s.lo, max(s.lo, min(s.hi, 18)) + 1)))
             else:
                 b.lit(1)
     for delta in rng.permutation([-1, 0, 1]):
@@ -633,9 +634,9 @@ def _flag_queue(b, rng):
         for _ in range(int(rng.integers(2, 6))):
             b.match(d, int(rng.integers(s.lo, max(s.lo, hi - 1) + 1)))
             b.lit(1)
-        l1 = int(rng.integers(s.lo, min(s.hi, 40) + 1))
+        l1 = int(rng.integers(s.lo, max(s.lo, min(s.hi, 40)) + 1))
         b.match(b.rdist(), l1)
-        b.match(int(rng.integers(1, min(l1, s.dmax) + 1)), int(rng.integers(s.lo, min(s.hi, 40) + 1)))
+        b.match(int(rng.integers(1, min(l1, s.dmax) + 1)), int(rng.integers(s.lo, max(s.lo, min(s.hi, 40)) + 1)))
 
 
 def _lzo_forms(b, rng):
@@ -657,12 +658,13 @@ def _lzo_forms(b, rng):
             b.lit(int(rng.integers(4, 30)))
 
 
-def generate(fmt, rng, profile, size=None, oracle=None):
-    """One stream of `fmt` drawn from `profile` (mixed, short_periods, window, ring, queue, long, forms)."""
+def generate(fmt, rng, profile, size=None, oracle=None, lzss_props=None):
+    """One stream of `fmt` drawn from `profile` (mixed, short_periods, window, ring, queue, long, forms).  LZSS draws its
+    properties from LZSS_PROPS unless `lzss_props` names one set in the same notation."""
     lzp = None
     spec = SPEC.get(fmt)
     if fmt == A.FMT_LZSS:
-        lzp = LZSS_PROPS[int(rng.integers(0, len(LZSS_PROPS)))]
+        lzp = lzss_props if lzss_props is not None else LZSS_PROPS[int(rng.integers(0, len(LZSS_PROPS)))]
         spec = lzss_spec(lzp)
     b = Builder(rng, spec, fmt)
     size = size or int(rng.choice([300, 2000, 6000, 12000, 30000]))
@@ -697,7 +699,7 @@ def generate(fmt, rng, profile, size=None, oracle=None):
         if fmt != A.FMT_BLZ and rng.random() < 0.6:   # distances past the start of the output read the prehistory
             b.lit(int(rng.integers(1, 40)))
             for _ in range(int(rng.integers(1, 4))):
-                b.match(int(rng.integers(b.n + 1, spec.dmax + 1)), b.rlen(40))
+                b.match(int(rng.integers(min(b.n + 1, spec.dmax), spec.dmax + 1)), b.rlen(40))
                 b.lit(int(rng.integers(1, 10)))
         elif (fmt == A.FMT_BLZ or snappy) and rng.random() < 0.25:   # ... or are rejected
             b.lit(int(rng.integers(spec.dmin, 50)))
@@ -705,7 +707,7 @@ def generate(fmt, rng, profile, size=None, oracle=None):
             invalid = True
         b.lit(spec.dmax + int(rng.integers(0, 200)))
         for _ in range(int(rng.integers(5, 40))):
-            b.match(spec.dmax - int(rng.choice([0, 0, 1, 2])), b.rlen(60))
+            b.match(max(spec.dmax - int(rng.choice([0, 0, 1, 2])), spec.dmin), b.rlen(60))
             b.lit(int(rng.integers(0, 6)))
     elif profile == "ring":
         start(20, 100)
